@@ -2,6 +2,7 @@
 """bench.py -- env-steps/s of the batched gym-cellular step on N B200s (one process per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4|cfg2|cfg3|cfg5] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -24,12 +25,17 @@ Workloads (BASELINE.json configs; per-GPU batch fixed => weak scaling):
   cfg5            mixed: per GPU 4M stochastic polarisation + 4M grid world envs (64M at 8 GPUs)
 The default line also carries cfg2/cfg3/cfg5 results under "workloads" on 1 GPU, and cfg5 (the multi-GPU
 config of BASELINE.json) at every N > 1, where the line also holds a shard check run on the hardware.
+
+--dump-outputs DIR writes what the timed device path computed in its last step (see dump_outputs); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  The script writes
+nothing into the tree it runs from.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -52,6 +58,7 @@ WORKLOADS = {
                         ("gridworld", 0.5, dict(max_episode_steps=128))], l2_resident=False),
 }
 RING = 8            # pre-generated action buffers per sub-batch
+DUMP_ENVS = 1 << 16  # --dump-outputs: envs per sub-batch in the written sample (every env of a smaller one)
 
 
 def bytes_per_env_step(kind, n_cells):
@@ -262,6 +269,26 @@ def time_device_path(batches, steps, warmup, dist, device, sampler_index, reduce
     return ms, launches, clk.summary(), 1e6 * t_host / max(launches, 1)
 
 
+def dump_outputs(batches, out_dir):
+    """What the last step handed its caller -- observation, reward, terminated, truncated and the infos unsafe,
+    count, time_step and tabular_state -- for a fixed, seeded sample of each sub-batch's envs, as float64 arrays
+    out_dir/<kind>_<name>.npy (at most 13 MB per sub-batch); <kind>_env_ids.npy holds the sampled env indices."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for b in batches:
+        env, n = b["env"], b["n"]
+        ids = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ENVS), replace=False))
+        sel = torch.from_numpy(ids).to(env.device)
+        infos = env._v_infos
+        out = {"env_ids": ids, "state": env.state[:, sel], "reward": env._v_reward[sel], "terminated": env._v_term[sel],
+               "truncated": env._v_trunc[sel], "unsafe": infos["unsafe"][sel], "count": infos["count"][sel],
+               "time_step": infos["time_step"][sel], "tabular_state": env.tabular_state()[sel]}
+        for name, a in out.items():
+            a = a.cpu().numpy() if torch.is_tensor(a) else a
+            np.save(os.path.join(out_dir, f"{b['kind']}_{name}.npy"), a.astype(np.float64))
+
+
 def sum_stats(batches):
     import torch
     return torch.stack([b["env"]._stats for b in batches]).sum(0)
@@ -417,7 +444,7 @@ def python_port_rate(workload):
     if part is None:
         return None
     try:
-        out = subprocess.run([sys.executable, "-m", "oracle.pyport", "--envs", "64", "--steps", "150", "--cells",
+        out = subprocess.run([sys.executable, "-B", "-m", "oracle.pyport", "--envs", "64", "--steps", "150", "--cells",
                               str(part["n_cells"]), "--levels", str(part["n_states"])], cwd=REPO, capture_output=True,
                              text=True, timeout=120).stdout.strip().splitlines()[-1]
         return json.loads(out)
@@ -632,8 +659,9 @@ def roofline_of(workload, batches, step_s, tag=None, resident_state=False):
             "l2_resident": resident}
 
 
-def bench_workload(workload, steps, warmup, dist, device, world, rank, e2e_steps, side=True):
-    """`side` = also time the CUDA-graph and fused-rollout variants (single process only)."""
+def bench_workload(workload, steps, warmup, dist, device, world, rank, e2e_steps, side=True, dump_dir=None):
+    """`side` = also time the CUDA-graph and fused-rollout variants (single process only).  `dump_dir`: where rank 0
+    writes the outputs of the timed path's last step (dump_outputs)."""
     import torch
     from gym_cellular_b200.distributed import StatsReducer
     batches = build_batches(workload, device, rank)
@@ -642,6 +670,8 @@ def bench_workload(workload, steps, warmup, dist, device, world, rank, e2e_steps
     # the per-iteration all-reduce of the statistics belongs to the multi-GPU path; one rank has nothing to reduce
     in_loop = reducer if dist is not None else None
     ms, launches, clocks, host_us = time_device_path(batches, steps, warmup, dist, device, device.index, in_loop)
+    if dump_dir is not None and rank == 0:          # before anything below steps these envs again
+        dump_outputs(batches, dump_dir)
     # Small shards: gc_step_many runs the bound steps of a call inside ONE kernel (state in registers between the steps,
     # every per-step output written at every step; include/gym_cellular_b200.h).  The same loop is then timed with one
     # launch per step as well (GC_B200_STEP_MANY_FUSED=0, read by the library at every call) and reported beside it.
@@ -812,11 +842,20 @@ def main():
     ap.add_argument("--no-side", action="store_true",
                     help="skip the CUDA-graph and fused-rollout side measurements (profiling runs: launch lists)")
     ap.add_argument("--host-chunk", type=int, default=None, help="envs per chunk of the host (e2e) path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the timed path's last step as DIR/<name>.npy (rank 0; a fixed sample "
+                         f"of {DUMP_ENVS} envs per sub-batch)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.host_chunk:
         global HOST_CHUNK_ENVS
         HOST_CHUNK_ENVS = args.host_chunk
+    # nothing is written into the tree, which may be read-only: no bytecode caches, and a CPU oracle that is
+    # missing or older than its source is compiled into a temporary directory
+    sys.dont_write_bytecode = True
+    from oracle import oracle as O
+    oracle_dir = tempfile.TemporaryDirectory(prefix="gc_bench_oracle_")
+    O.build_dir = oracle_dir.name
 
     if args.impl == "reference":
         run_reference_arm(args, args.workload)
@@ -847,17 +886,16 @@ def main():
 
     e2e_steps = max(3, min(args.steps, 10))
     main_res = bench_workload(args.workload, args.steps, args.warmup, dist, device, world, rank, e2e_steps,
-                              side=not args.no_side)
-    # side workloads: the launch-bound configs 2 and 3 on one GPU (with enough steps that a short driver run is
-    # not a pipeline-fill measurement), the mixed multi-GPU config 5 at every N
+                              side=not args.no_side, dump_dir=args.dump_outputs)
+    # side workloads, over the same --steps: the launch-bound configs 2 and 3 on one GPU, the mixed multi-GPU
+    # config 5 at every N (a run of a few steps times the launch-bound ones mostly filling the pipeline)
     extra = {}
-    side_steps = max(args.steps, 2000)
     if not args.no_extra:
         for w in (("cfg2", "cfg3", "cfg5") if world == 1 else ("cfg5",)):
             if w != args.workload:
-                r = bench_workload(w, side_steps, args.warmup, dist, device, world, rank, e2e_steps, side=not args.no_side)
+                r = bench_workload(w, args.steps, args.warmup, dist, device, world, rank, e2e_steps, side=not args.no_side)
                 extra[w] = {"description": WORKLOADS[w]["desc"], "value": r["value"], "ms_per_step": r["ms_per_step"],
-                            "steps": side_steps, "host_us_per_launch": r["host_us_per_launch"],
+                            "steps": args.steps, "host_us_per_launch": r["host_us_per_launch"],
                             "roofline_frac": r["roofline"]["frac"], "achieved_gbs": r["roofline"]["achieved"],
                             "traffic": r["roofline"]["traffic"],
                             "dram_bytes_over_algorithmic": r["roofline"]["dram_bytes_over_algorithmic"],

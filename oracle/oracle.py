@@ -32,12 +32,22 @@ class _Config(C.Structure):
                 ("reward_table", C.POINTER(C.c_double))]
 
 
-def build(force=False):
-    """Compile oracle/gc_oracle.c with gcc (Makefile in this directory)."""
-    src = os.path.join(_HERE, "gc_oracle.c")
-    if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "libgc_oracle.so"])
-    return _LIB_PATH
+# Where lib() compiles the oracle when the library in this directory is missing or older than its source;
+# None = this directory.  bench.py points it at a temporary directory: it must run from a read-only tree.
+build_dir = None
+
+
+def _stale(path):
+    return not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(os.path.join(_HERE, "gc_oracle.c"))
+
+
+def build(force=False, out_dir=None):
+    """Compile oracle/gc_oracle.c with gcc (Makefile in this directory) into `out_dir` (default: this
+    directory); returns the library's path."""
+    path = _LIB_PATH if out_dir is None else os.path.join(out_dir, "libgc_oracle.so")
+    if force or _stale(path):
+        subprocess.check_call(["make", "-s", "-C", _HERE, "OUT=" + path])
+    return path
 
 
 _lib = None
@@ -46,8 +56,8 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_LIB_PATH)
+        path = build(out_dir=build_dir if _stale(_LIB_PATH) else None)
+        L = C.CDLL(path)
         vp = C.c_void_p
         L.gco_step.restype = C.c_int64
         L.gco_step.argtypes = [C.POINTER(_Config), C.c_int64, C.c_int64] + [vp] * 11 + [C.c_int64, vp]

@@ -49,3 +49,35 @@ def test_native_arm_line():
     assert e["h2d_bytes_per_step"] == 4 * 65536 and e["d2h_bytes_per_step"] == 13 * 65536 and 0 < e["value"] < d["value"]
     assert d["clocks"]["sm_max_mhz"] and not {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"} & set(d["clocks"]["reasons"])
     assert d["cpu_baseline"]["kind"] == "port" and d["config"]["workload"] == "cfg2"
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """--dump-outputs writes what the timed path computed in its last step, as float arrays: on cfg2 (65,536 envs,
+    all of them in the sample) it equals the oracle stepped through the warmup and timed steps of the bench's
+    seeded action ring."""
+    import numpy as np
+    import torch
+    import bench
+    from oracle import oracle as O
+    warmup, steps = 5, 30
+    d = _run("--steps", str(steps), "--warmup", str(warmup), "--workload", "cfg2", "--no-extra", "--no-cpu-baseline",
+             "--no-side", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == steps and d["warmup"] == warmup
+    out = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert set(out) == {"cellular_" + k for k in ("env_ids", "state", "reward", "terminated", "truncated", "unsafe",
+                                                   "count", "time_step", "tabular_state")}
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    b, = bench.build_batches("cfg2", torch.device("cuda", 0), 0)
+    n, ring = b["n"], [a[:, :b["n"]].cpu().numpy() for a in b["ring"]]
+    b["env"].close()
+    assert (out["cellular_env_ids"] == np.arange(n)).all()
+    ora = O.OracleEnv(n_envs=n, seed=0)
+    for i in range(warmup + steps):
+        ora.step(ring[i % len(ring)])
+    assert (out["cellular_state"] == ora.state).all() and (out["cellular_tabular_state"] == ora.index).all()
+    assert (out["cellular_time_step"] == warmup + steps).all() and (out["cellular_time_step"] == ora.t).all()
+    assert (out["cellular_unsafe"] == ora.unsafe).all() and (out["cellular_count"] == ora.count).all()
+    assert not out["cellular_terminated"].any() and not out["cellular_truncated"].any()
+    np.testing.assert_allclose(out["cellular_reward"], ora.reward, rtol=1e-6, atol=1e-7)
