@@ -829,6 +829,34 @@ int gc_step_host(gc_env *env, const int8_t *h_actions, int8_t *h_state, float *h
     return GC_OK;
 }
 
+namespace {
+
+// RolloutIO of a whole-shard gc_rollout / gc_collect launch (the record and epsilon fields stay zero)
+RolloutIO make_rollout_io(const gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, int8_t *state,
+                          int32_t *t, uint32_t *index, int64_t *stats)
+{
+    RolloutIO io;
+    std::memset(&io, 0, sizeof(io));
+    io.state = state; io.t = t; io.index = index; io.policy = policy;
+    io.stats = reinterpret_cast<unsigned long long *>(stats);
+    io.status = env->d_status;
+    io.n = env->cfg.n_envs; io.ld = env->cfg.ld; io.env_id_offset = env->cfg.env_id_offset;
+    const uint32_t lo = static_cast<uint32_t>(env->cfg.seed), hi = static_cast<uint32_t>(env->cfg.seed >> 32);
+    for (int r = 0; r < 10; ++r) {
+        io.round_key[2 * r] = lo + static_cast<uint32_t>(r) * 0x9E3779B9u;
+        io.round_key[2 * r + 1] = hi + static_cast<uint32_t>(r) * 0xBB67AE85u;
+    }
+    io.step_ctr = env->d_step; io.done_ctr = env->d_done;
+    io.episodic = (env->cfg.flags & GC_F_RNG_EPISODIC) ? 1 : 0;
+    io.max_episode_steps = env->cfg.max_episode_steps;
+    io.n_steps = n_steps; io.policy_kind = policy_kind;
+    return io;
+}
+
+bool misaligned(const void *p) { return p && (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
+
+}  // namespace
+
 int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, int8_t *state,
                int32_t *t, uint32_t *index, float *ret, int32_t *n_unsafe, int64_t *stats, void *stream)
 {
@@ -842,20 +870,8 @@ int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     if (env->cfg.kind == GC_KIND_CELLULAR && !env->fast_ok)
         return fail(GC_ERR_INVALID, "gc_rollout supports the cellular family with n_states, n_actions <= 4 only");
     GC_ON_DEVICE(env->cfg.device);
-    RolloutIO io;
-    io.state = state; io.t = t; io.index = index; io.ret = ret; io.n_unsafe = n_unsafe; io.policy = policy;
-    io.stats = reinterpret_cast<unsigned long long *>(stats);
-    io.status = env->d_status;
-    io.n = env->cfg.n_envs; io.ld = env->cfg.ld; io.env_id_offset = env->cfg.env_id_offset;
-    const uint32_t lo = static_cast<uint32_t>(env->cfg.seed), hi = static_cast<uint32_t>(env->cfg.seed >> 32);
-    for (int r = 0; r < 10; ++r) {
-        io.round_key[2 * r] = lo + static_cast<uint32_t>(r) * 0x9E3779B9u;
-        io.round_key[2 * r + 1] = hi + static_cast<uint32_t>(r) * 0xBB67AE85u;
-    }
-    io.step_ctr = env->d_step; io.done_ctr = env->d_done;
-    io.episodic = (env->cfg.flags & GC_F_RNG_EPISODIC) ? 1 : 0;
-    io.max_episode_steps = env->cfg.max_episode_steps;
-    io.n_steps = n_steps; io.policy_kind = policy_kind;
+    RolloutIO io = make_rollout_io(env, n_steps, policy_kind, policy, state, t, index, stats);
+    io.ret = ret; io.n_unsafe = n_unsafe;
     cudaError_t e;
     if (env->cfg.kind == GC_KIND_CELLULAR)
         e = gc_launch_cell_rollout(env->tab, io, env->d_pair_lut, (env->cfg.flags & GC_F_NOISE) != 0, env->n_sm,
@@ -863,6 +879,49 @@ int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     else
         e = gc_launch_grid_rollout(env->grid, io, env->n_sm, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return fail(GC_ERR_CUDA, "rollout kernel launch failed: %s", cudaGetErrorString(e));
+    env->launches += 1;
+    env->global_step += n_steps;
+    return GC_OK;
+}
+
+
+int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+               int8_t *state, int32_t *t, uint32_t *index, const gc_record *record, int64_t *stats, void *stream)
+{
+    GC_NVTX("gc_collect");
+    if (int rc = check_env(env)) return rc;
+    if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
+    if (!state || !t || !index || !record) return fail(GC_ERR_INVALID, "a required pointer is NULL");
+    if (n_steps < 1) return fail(GC_ERR_INVALID, "n_steps must be >= 1");
+    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE) return fail(GC_ERR_INVALID, "unknown policy kind");
+    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
+    if (!(epsilon >= 0.0 && epsilon <= 1.0)) return fail(GC_ERR_INVALID, "epsilon must lie in [0, 1] (got %g)", epsilon);
+    if (policy_kind == GC_POLICY_RANDOM && epsilon != 0.0)
+        return fail(GC_ERR_INVALID, "epsilon applies to GC_POLICY_TABLE only (GC_POLICY_RANDOM needs epsilon 0)");
+    if (record->struct_size != sizeof(gc_record))
+        return fail(GC_ERR_INVALID, "record->struct_size %u != sizeof(gc_record) %zu", record->struct_size, sizeof(gc_record));
+    if (misaligned(record->obs) || misaligned(record->action) || misaligned(record->reward) || misaligned(record->flags) ||
+        misaligned(record->next_obs))
+        return fail(GC_ERR_INVALID, "record pointers must be 16-byte aligned");
+    if (env->cfg.kind == GC_KIND_CELLULAR && !env->fast_ok)
+        return fail(GC_ERR_INVALID, "gc_collect supports the cellular family with n_states, n_actions <= 4 only");
+    GC_ON_DEVICE(env->cfg.device);
+    RolloutIO io = make_rollout_io(env, n_steps, policy_kind, policy, state, t, index, stats);
+    io.rec_obs = record->obs; io.rec_action = record->action; io.rec_reward = record->reward;
+    io.rec_flags = record->flags; io.rec_next_obs = record->next_obs;
+    unsigned long long joint = 1;
+    for (int c = 0; c < env->cfg.n_cells; ++c) joint *= static_cast<unsigned long long>(env->cfg.n_actions);
+    io.joint_actions = joint;
+    const unsigned long long thr = threshold_of(epsilon);
+    io.explore_thr_nz = thr != 0 ? 1u : 0u;
+    io.explore_thr_m1 = static_cast<uint32_t>(thr - 1);
+    cudaError_t e;
+    if (env->cfg.kind == GC_KIND_CELLULAR)
+        e = gc_launch_cell_collect(env->tab, io, env->d_pair_lut, (env->cfg.flags & GC_F_NOISE) != 0, env->n_sm,
+                                   static_cast<cudaStream_t>(stream));
+    else
+        e = gc_launch_grid_collect(env->grid, io, env->n_sm, static_cast<cudaStream_t>(stream));
+    if (e != cudaSuccess) return fail(GC_ERR_CUDA, "collect kernel launch failed: %s", cudaGetErrorString(e));
     env->launches += 1;
     env->global_step += n_steps;
     return GC_OK;

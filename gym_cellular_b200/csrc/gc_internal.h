@@ -94,6 +94,13 @@ struct RolloutIO {
     const uint32_t *step_ctr;
     uint32_t *done_ctr;
     int32_t episodic, max_episode_steps, n_steps, policy_kind;
+    // gc_collect (the RECORD kernels; appended so that the fields above keep their offsets): the transition
+    // record, step-major [n_steps][ld], each pointer NULL = not recorded
+    uint32_t *rec_obs, *rec_action, *rec_next_obs;
+    float    *rec_reward;
+    uint8_t  *rec_flags;
+    unsigned long long joint_actions;        // A^C (<= 2^32): an explored cellular action is floor(word * A^C / 2^32)
+    uint32_t explore_thr_m1, explore_thr_nz; // the table policy explores iff thr_nz && word <= thr_m1 (P = eps)
 };
 
 // Constant tables of the cellular family, passed by value as a __grid_constant__ parameter and
@@ -185,6 +192,10 @@ cudaError_t gc_launch_unpack(int64_t n, int64_t ld, int n_cells, const uint32_t 
 cudaError_t gc_launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise,
                                    int n_sm, cudaStream_t stream);
 cudaError_t gc_launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t stream);
+// the same kernels writing the transition record, table policy epsilon-greedy (gc_collect)
+cudaError_t gc_launch_cell_collect(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise,
+                                   int n_sm, cudaStream_t stream);
+cudaError_t gc_launch_grid_collect(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t stream);
 cudaError_t gc_launch_grid_step(const GridParams &gp, const StepIO &io, int rng_mode, int n_sm,
                                 cudaStream_t stream);
 cudaError_t gc_launch_reset(int n_cells, const int8_t *init, uint32_t init_index, const uint8_t *mask,

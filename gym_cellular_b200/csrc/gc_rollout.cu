@@ -17,11 +17,21 @@
 //   cellular: action = floor(word * 2^-32 * A);  grid world (c = 0): jurisdiction = bit 31, position =
 //   bits 29-30, the other jurisdiction names no position (the reference sampler's distribution,
 //   grid_world.py:191-195).  T is the counter the step's noise uses (episode step or global step).
+//
+// Experience collection (gc_collect): the RECORD instantiations also write every transition (obs, executed
+// action, reward, flags, next_obs) into step-major [n_steps][ld] arrays and take the table policy
+// epsilon-greedily (restated in tests/_collect_oracle.py).  For env g at global step G:
+//   explore iff word (g % 4) of philox(key, ((g/4)_lo, (g/4)_hi, G, 0x50000000)) < ceil(eps * 2^32);
+//   explore action = word (g % 4) of philox(key, ((g/4)_lo, (g/4)_hi, G, 0x50000001)): cellular joint action
+//   floor(word * A^C / 2^32), grid world the random policy's rule.
+// G is the global step even for episodic envs: exploration belongs to the agent, and keying it by the episode
+// step would make every episode explore at the same steps with the same actions.
 #include "gc_device.cuh"
 
 namespace {
 
 constexpr uint32_t kActionStream = 0x40000000u;
+constexpr uint32_t kExploreStream = 0x50000000u;     // + 0: explore test, + 1: explore action
 
 __device__ __forceinline__ bool same4(const int (&t)[kEPT]) { return t[0] == t[1] && t[1] == t[2] && t[2] == t[3]; }
 
@@ -41,8 +51,30 @@ __device__ __forceinline__ void action_words(const RolloutIO &io, uint32_t grp_l
     }
 }
 
+// grid world, the reference sampler's distribution: (a_0, a_1) = (4, pos) or (pos, 4) as a_0 + 5 a_1
+__device__ __forceinline__ uint32_t random_grid_action(uint32_t w)
+{
+    const uint32_t pos = (w >> 29) & 3u;
+    return (w >> 31) ? (4u + 5u * pos) : (pos + 20u);
+}
+
+// epsilon-greedy (RECORD kernels): bit e of the result is set when env e of the thread explores at global step G;
+// w then holds the explore-action words (drawn only when one of the 4 envs explores)
+__device__ __forceinline__ uint32_t explore_words(const RolloutIO &io, uint32_t grp_lo, uint32_t grp_hi, uint32_t G,
+                                                  uint32_t (&w)[kEPT])
+{
+    if (!io.explore_thr_nz) return 0u;
+    uint32_t x[4];
+    philox4x32_10(grp_lo, grp_hi, G, kExploreStream, io.round_key, x);
+    uint32_t m = 0;
+#pragma unroll
+    for (int e = 0; e < kEPT; ++e) m |= (x[e] <= io.explore_thr_m1 ? 1u : 0u) << e;
+    if (m) philox4x32_10(grp_lo, grp_hi, G, kExploreStream + 1u, io.round_key, w);
+    return m;
+}
+
 // ---------------------------------------------------------------------------------------------
-template <int C, bool NOISE>
+template <int C, bool NOISE, bool RECORD>
 __global__ void __launch_bounds__(kThreads, 2)
 cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constant__ RolloutIO io,
                     const uint2 *__restrict__ lut)
@@ -80,19 +112,20 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
         uint32_t nuns[kEPT] = {0, 0, 0, 0};
         uint32_t idx[kEPT];
 
-        auto fold_index = [&]() {                      // tabular index of the 4 envs from the state words
+        auto fold_words = [&](const uint32_t (&w)[C], uint32_t (&out)[kEPT]) {   // tabular index of the 4 envs
 #pragma unroll
-            for (int e = 0; e < kEPT; ++e) idx[e] = 0;
+            for (int e = 0; e < kEPT; ++e) out[e] = 0;
 #pragma unroll
             for (int g = 0; g < (C + 3) / 4; ++g) {
                 uint32_t q = 0;
 #pragma unroll
                 for (int i = 0; i < 4; ++i)
-                    if (4 * g + i < C) q += sw[4 * g + i] * tab.place4[i];
+                    if (4 * g + i < C) q += w[4 * g + i] * tab.place4[i];
 #pragma unroll
-                for (int e = 0; e < kEPT; ++e) idx[e] += byte_of(q, e) * tab.place[4 * g];
+                for (int e = 0; e < kEPT; ++e) out[e] += byte_of(q, e) * tab.place[4 * g];
             }
         };
+        auto fold_index = [&]() { fold_words(sw, idx); };
 
 #pragma unroll 1
         for (int k = 0; k < io.n_steps; ++k) {
@@ -107,6 +140,13 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                 uint32_t p[kEPT];
 #pragma unroll
                 for (int e = 0; e < kEPT; ++e) p[e] = static_cast<uint32_t>(__ldg(io.policy + idx[e]));
+                if constexpr (RECORD) {
+                    uint32_t xw[kEPT];
+                    const uint32_t xm = explore_words(io, grp_lo, grp_hi, step0 + static_cast<uint32_t>(k), xw);
+#pragma unroll
+                    for (int e = 0; e < kEPT; ++e)
+                        if ((xm >> e) & 1u) p[e] = static_cast<uint32_t>((static_cast<unsigned long long>(xw[e]) * io.joint_actions) >> 32);
+                }
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
                     aw[c] = 0;
@@ -119,6 +159,28 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                     uint32_t w[kEPT];
                     action_words(io, grp_lo, grp_hi, T, shared, c, w);
                     aw[c] = __umulhi(w[0], A) | (__umulhi(w[1], A) << 8) | (__umulhi(w[2], A) << 16) | (__umulhi(w[3], A) << 24);
+                }
+            }
+            const int64_t kofs = static_cast<int64_t>(k) * ld;        // record row of this step (K * ld may pass 2^31)
+            if constexpr (RECORD) {
+                if (io.rec_obs) {
+                    if (io.policy_kind != GC_POLICY_TABLE) fold_index();
+                    st_stream_v4(io.rec_obs + kofs + e0, make_int4(idx[0], idx[1], idx[2], idx[3]));
+                }
+                if (io.rec_action) {                                   // sum_c a_c A^c of the executed digits
+                    const uint32_t A2 = A * A, pl4[4] = {1u, A, A2, A2 * A};
+                    uint32_t ai[kEPT] = {0, 0, 0, 0}, plg = 1u;
+#pragma unroll
+                    for (int g = 0; g < (C + 3) / 4; ++g) {
+                        uint32_t q = 0;                                // digits <= 3, A <= 4: bytes do not carry
+#pragma unroll
+                        for (int i = 0; i < 4; ++i)
+                            if (4 * g + i < C) q += aw[4 * g + i] * pl4[i];
+#pragma unroll
+                        for (int e = 0; e < kEPT; ++e) ai[e] += byte_of(q, e) * plg;
+                        plg *= A2 * A2;
+                    }
+                    st_stream_v4(io.rec_action + kofs + e0, make_int4(ai[0], ai[1], ai[2], ai[3]));
                 }
             }
             // ---- transition, reward, side effects (pair table, as in gc_cell_fast.cu) ----------------
@@ -200,6 +262,19 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
             st_unsafe = add_bytes(unsafe_w & vb, st_unsafe);
             st_count = add_bytes(count_w & vb, st_count);
             st_trunc = add_bytes(trunc_w & vb, st_trunc);
+            if constexpr (RECORD) {
+                if (io.rec_reward)
+                    st_stream_v4(io.rec_reward + kofs + e0, make_int4(__float_as_int(rlog[0]), __float_as_int(rlog[1]),
+                                                                      __float_as_int(rlog[2]), __float_as_int(rlog[3])));
+                if (io.rec_flags)
+                    st_stream_u32(io.rec_flags + kofs + e0,
+                                  unsafe_w * GC_FLAG_UNSAFE | trunc_w * GC_FLAG_TRUNCATED | (count_w << GC_FLAG_COUNT_SHIFT));
+                if (io.rec_next_obs) {                                 // successor before the auto-reset
+                    uint32_t nx[kEPT];
+                    fold_words(rows, nx);
+                    st_stream_v4(io.rec_next_obs + kofs + e0, make_int4(nx[0], nx[1], nx[2], nx[3]));
+                }
+            }
 #pragma unroll
             for (int c = 0; c < C; ++c)
                 sw[c] = (rows[c] & keep) | ((0x01010101u * static_cast<uint8_t>(tab.init[c])) & ~keep);
@@ -209,9 +284,11 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
         for (int c = 0; c < C; ++c) st_stream_u32(io.state + c * ld + e0, sw[c]);
         st_stream_v4(io.t + e0, make_int4(t[0], t[1], t[2], t[3]));
         st_stream_v4(io.index + e0, make_int4(idx[0], idx[1], idx[2], idx[3]));
-        st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
-                                            __float_as_int(ret[2]), __float_as_int(ret[3])));
-        st_stream_v4(io.n_unsafe + e0, make_int4(nuns[0], nuns[1], nuns[2], nuns[3]));
+        if constexpr (!RECORD) {
+            st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
+                                                __float_as_int(ret[2]), __float_as_int(ret[3])));
+            st_stream_v4(io.n_unsafe + e0, make_int4(nuns[0], nuns[1], nuns[2], nuns[3]));
+        }
     }
     if (io.stats) {
         const ThreadStats ts = {st_steps, st_unsafe, st_count, st_trunc, st_reward};
@@ -221,6 +298,7 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
 }
 
 // ---------------------------------------------------------------------------------------------
+template <bool RECORD>
 __global__ void __launch_bounds__(kThreads, 4)
 grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant__ RolloutIO io)
 {
@@ -264,14 +342,25 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                     act[e] = static_cast<uint32_t>(__ldg(io.policy + (tab < 400u ? tab : 0u)));
                     if (act[e] > 24u) act[e] = 24u;
                 }
+                if constexpr (RECORD) {
+                    uint32_t xw[kEPT];
+                    const uint32_t xm = explore_words(io, grp_lo, grp_hi, step0 + static_cast<uint32_t>(k), xw);
+#pragma unroll
+                    for (int e = 0; e < kEPT; ++e)
+                        if ((xm >> e) & 1u) act[e] = random_grid_action(xw[e]);
+                }
             } else {
                 uint32_t w[kEPT];
                 action_words(io, grp_lo, grp_hi, T, shared, 0u, w);
 #pragma unroll
-                for (int e = 0; e < kEPT; ++e) {
-                    const uint32_t pos = (w[e] >> 29) & 3u;
-                    act[e] = (w[e] >> 31) ? (4u + 5u * pos) : (pos + 20u);     // (a_0, a_1) = (4, pos) or (pos, 4)
-                }
+                for (int e = 0; e < kEPT; ++e) act[e] = random_grid_action(w[e]);
+            }
+            const int64_t kofs = static_cast<int64_t>(k) * ld;        // record row of this step (K * ld may pass 2^31)
+            if constexpr (RECORD) {
+                if (io.rec_obs)
+                    st_stream_v4(io.rec_obs + kofs + e0, make_int4(c0[0] + 20u * c1[0], c0[1] + 20u * c1[1],
+                                                                   c0[2] + 20u * c1[2], c0[3] + 20u * c1[3]));
+                if (io.rec_action) st_stream_v4(io.rec_action + kofs + e0, make_int4(act[0], act[1], act[2], act[3]));
             }
             uint32_t trig[kEPT];
             if (shared) {
@@ -285,6 +374,7 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                 }
             }
             uint32_t count_w = 0, trunc_w = 0, rew_w = 0;
+            uint32_t nx[kEPT];
 #pragma unroll
             for (int e = 0; e < kEPT; ++e) {
                 const uint32_t ix = (c0[e] + 20u * c1[e]) * 25u + act[e];
@@ -302,6 +392,7 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                 const uint32_t rew = (ent >> 16) & 3u;
                 ret[e] += static_cast<float>(rew);
                 c0[e] = ent & 0xFFu; c1[e] = (ent >> 8) & 0xFFu;
+                nx[e] = c0[e] + 20u * c1[e];                              // successor before the auto-reset
                 t[e] += 1;
                 uint32_t tr = 0;
                 if (io.max_episode_steps > 0 && t[e] >= io.max_episode_steps) { tr = 1; t[e] = 0; c0[e] = 15u; c1[e] = 18u; }
@@ -312,14 +403,26 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
             st_count = add_bytes(count_w & vb, st_count);
             st_trunc = add_bytes(trunc_w & vb, st_trunc);
             st_reward = add_bytes(rew_w & vb, st_reward);
+            if constexpr (RECORD) {
+                if (io.rec_reward)
+                    st_stream_v4(io.rec_reward + kofs + e0, make_int4(__float_as_int(static_cast<float>(byte_of(rew_w, 0))),
+                                                                      __float_as_int(static_cast<float>(byte_of(rew_w, 1))),
+                                                                      __float_as_int(static_cast<float>(byte_of(rew_w, 2))),
+                                                                      __float_as_int(static_cast<float>(byte_of(rew_w, 3)))));
+                if (io.rec_flags)                                      // never 'unsafe'
+                    st_stream_u32(io.rec_flags + kofs + e0, trunc_w * GC_FLAG_TRUNCATED | (count_w << GC_FLAG_COUNT_SHIFT));
+                if (io.rec_next_obs) st_stream_v4(io.rec_next_obs + kofs + e0, make_int4(nx[0], nx[1], nx[2], nx[3]));
+            }
         }
         st_stream_u32(io.state + e0, c0[0] | (c0[1] << 8) | (c0[2] << 16) | (c0[3] << 24));
         st_stream_u32(io.state + ld + e0, c1[0] | (c1[1] << 8) | (c1[2] << 16) | (c1[3] << 24));
         st_stream_v4(io.t + e0, make_int4(t[0], t[1], t[2], t[3]));
         st_stream_v4(io.index + e0, make_int4(c0[0] + 20u * c1[0], c0[1] + 20u * c1[1], c0[2] + 20u * c1[2], c0[3] + 20u * c1[3]));
-        st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
-                                            __float_as_int(ret[2]), __float_as_int(ret[3])));
-        st_stream_v4(io.n_unsafe + e0, make_int4(0, 0, 0, 0));                       // never 'unsafe'
+        if constexpr (!RECORD) {
+            st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
+                                                __float_as_int(ret[2]), __float_as_int(ret[3])));
+            st_stream_v4(io.n_unsafe + e0, make_int4(0, 0, 0, 0));                   // never 'unsafe'
+        }
     }
     if (bad_bits & (1u << 22)) atomicOr(io.status, 1ull);
     if (io.stats) {
@@ -341,14 +444,36 @@ inline int rollout_grid(int64_t n, int threads, int n_sm, int blocks_per_sm_256)
     return static_cast<int>(need < cap ? (need < 1 ? 1 : need) : cap);
 }
 
-template <int C>
+template <int C, bool RECORD>
 cudaError_t launch_rollout_c(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm, cudaStream_t st)
 {
     const int threads = rollout_threads(io.n, n_sm), grid = rollout_grid(io.n, threads, n_sm, 2);
     if (noise)
-        cell_rollout_kernel<C, true><<<grid, threads, 0, st>>>(tab, io, lut);
+        cell_rollout_kernel<C, true, RECORD><<<grid, threads, 0, st>>>(tab, io, lut);
     else
-        cell_rollout_kernel<C, false><<<grid, threads, 0, st>>>(tab, io, lut);
+        cell_rollout_kernel<C, false, RECORD><<<grid, threads, 0, st>>>(tab, io, lut);
+    return cudaGetLastError();
+}
+
+template <bool RECORD>
+cudaError_t launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
+                                cudaStream_t st)
+{
+    switch (tab.n_cells) {
+#define GC_CASE(C) case C: return launch_rollout_c<C, RECORD>(tab, io, lut, noise, n_sm, st);
+        GC_CASE(1) GC_CASE(2) GC_CASE(3) GC_CASE(4) GC_CASE(5) GC_CASE(6) GC_CASE(7) GC_CASE(8)
+        GC_CASE(9) GC_CASE(10) GC_CASE(11) GC_CASE(12) GC_CASE(13) GC_CASE(14) GC_CASE(15) GC_CASE(16)
+#undef GC_CASE
+    default: return cudaErrorInvalidValue;
+    }
+}
+
+template <bool RECORD>
+cudaError_t launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
+{
+    // the 40 KB table is staged per block: keep 256-thread blocks unless the batch is really small
+    const int threads = (io.n + kEPT - 1) / kEPT < static_cast<int64_t>(n_sm) * kThreads / 2 ? 64 : kThreads;
+    grid_rollout_kernel<RECORD><<<rollout_grid(io.n, threads, n_sm, 4), threads, 0, st>>>(gp, io);
     return cudaGetLastError();
 }
 
@@ -357,19 +482,21 @@ cudaError_t launch_rollout_c(const CellTables &tab, const RolloutIO &io, const u
 cudaError_t gc_launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
                                    cudaStream_t st)
 {
-    switch (tab.n_cells) {
-#define GC_CASE(C) case C: return launch_rollout_c<C>(tab, io, lut, noise, n_sm, st);
-        GC_CASE(1) GC_CASE(2) GC_CASE(3) GC_CASE(4) GC_CASE(5) GC_CASE(6) GC_CASE(7) GC_CASE(8)
-        GC_CASE(9) GC_CASE(10) GC_CASE(11) GC_CASE(12) GC_CASE(13) GC_CASE(14) GC_CASE(15) GC_CASE(16)
-#undef GC_CASE
-    default: return cudaErrorInvalidValue;
-    }
+    return launch_cell_rollout<false>(tab, io, lut, noise, n_sm, st);
+}
+
+cudaError_t gc_launch_cell_collect(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
+                                   cudaStream_t st)
+{
+    return launch_cell_rollout<true>(tab, io, lut, noise, n_sm, st);
 }
 
 cudaError_t gc_launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
 {
-    // the 40 KB table is staged per block: keep 256-thread blocks unless the batch is really small
-    const int threads = (io.n + kEPT - 1) / kEPT < static_cast<int64_t>(n_sm) * kThreads / 2 ? 64 : kThreads;
-    grid_rollout_kernel<<<rollout_grid(io.n, threads, n_sm, 4), threads, 0, st>>>(gp, io);
-    return cudaGetLastError();
+    return launch_grid_rollout<false>(gp, io, n_sm, st);
+}
+
+cudaError_t gc_launch_grid_collect(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
+{
+    return launch_grid_rollout<true>(gp, io, n_sm, st);
 }

@@ -294,6 +294,18 @@ class PackedCellularVectorEnv(CellularVectorEnv):
             self._index.copy_(self._ro_index)
         return self._ro_ret[:n], self._ro_unsafe[:n]
 
+    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False):
+        """Experience collection (see `CellularVectorEnv.collect`): the recording kernel takes the int8 layout,
+        so the packed state is unpacked for it and packed again afterwards, as in `rollout()`."""
+        if getattr(self, "_ro_index", None) is None:
+            self._ro_index = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
+        cells = self.unpack(self._state).contiguous()            # int8 [n_cells, ld]
+        tr = self._collect(n_steps, policy, epsilon, next_obs, cells, self._ro_index)
+        self._state.copy_(self.pack(cells))
+        if self._index is not self._state:
+            self._index.copy_(self._ro_index)
+        return tr
+
     # ---- views ---------------------------------------------------------------------------------------
     def _lazy_truncated(self):
         return (self._flags[:self.num_envs] & _lib.FLAG_TRUNCATED).ne(0)

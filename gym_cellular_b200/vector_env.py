@@ -17,6 +17,7 @@ Two ways to drive it:
 There is no CPU implementation behind this class: without the CUDA library or a CUDA device it raises.
 """
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -31,6 +32,26 @@ _FAMILIES = {
     "Cells3ResetVDeadlock-v0": ("cellular", 3, 3, 3, True),
     "GridWorld-v0": ("gridworld", 2, 20, 5, True),
 }
+
+
+class Transitions(namedtuple("Transitions", "obs action reward flags next_obs")):
+    """Experience of `collect(K)`: [K, num_envs] device tensors, row k = step k.
+    obs / action / next_obs are int32 tensors carrying the uint32 tabular indices (as `tabular_state(torch.int32)`);
+    next_obs is the successor before the time-limit auto-reset (None unless requested); flags is the packed
+    layout's flag byte (bit 0 unsafe, bit 1 truncated, bits 2-6 count), decoded by `unsafe`, `truncated`, `count`."""
+    __slots__ = ()
+
+    @property
+    def unsafe(self):
+        return (self.flags & _lib.FLAG_UNSAFE).ne(0)
+
+    @property
+    def truncated(self):
+        return (self.flags & _lib.FLAG_TRUNCATED).ne(0)
+
+    @property
+    def count(self):
+        return self.flags >> _lib.FLAG_COUNT_SHIFT
 
 
 def _round_up(n, m):
@@ -517,6 +538,47 @@ class CellularVectorEnv(gym.vector.VectorEnv):
                                         _ptr(self._index), _ptr(self._ro_ret), _ptr(self._ro_unsafe), _ptr(self._stats),
                                         self._stream()))
         return self._ro_ret[:n], self._ro_unsafe[:n]
+
+    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False):
+        """Experience collection: `n_steps` steps per env inside one kernel, as `rollout()`, recording every
+        transition.  policy=None: uniformly random actions (epsilon must be 0); a table as for `rollout()`: the
+        epsilon-greedy policy that takes policy[obs] and, with probability `epsilon`, a uniformly random joint
+        action instead (grid world: the reference sampler's).  Exploration is keyed by global env id and global
+        step, so it differs between episodes even when the env's noise replays (`rng_episodic`).
+        Returns `Transitions(obs, action, reward, flags, next_obs)` of [n_steps, num_envs] views; state,
+        time_step, tabular_state() and stats() advance exactly as `rollout()` advances them.  The views alias
+        buffers cached per n_steps: the next `collect` with the same n_steps overwrites them, as a step
+        overwrites its outputs."""
+        return self._collect(n_steps, policy, epsilon, next_obs, self._state, self._index)
+
+    def _policy_table(self, policy):
+        if policy is None:
+            return _lib.POLICY_RANDOM, None
+        ptab = torch.as_tensor(policy, device=self.device).to(torch.int32).contiguous()
+        if ptab.numel() != self.n_states ** self.n_cells:
+            raise ValueError("policy must have one entry per tabular state")
+        return _lib.POLICY_TABLE, ptab
+
+    def _collect(self, n_steps, policy, epsilon, next_obs, state, index):
+        n_steps = int(n_steps)
+        kind, ptab = self._policy_table(policy)
+        bufs = self.__dict__.setdefault("_record_bufs", {})
+        buf = bufs.get(n_steps)
+        if buf is None:
+            rows = max(n_steps, 1)              # n_steps < 1 is rejected by the library, with its message
+            z = lambda dtype: torch.zeros(rows, self.ld, dtype=dtype, device=self.device)     # noqa: E731
+            buf = bufs[n_steps] = {"obs": z(torch.int32), "action": z(torch.int32), "reward": z(torch.float32),
+                                   "flags": z(torch.uint8), "next_obs": None}
+        if next_obs and buf["next_obs"] is None:
+            buf["next_obs"] = torch.zeros_like(buf["obs"])
+        nx = buf["next_obs"] if next_obs else None
+        rec = _lib.GcRecord(C.sizeof(_lib.GcRecord), buf["obs"].data_ptr(), buf["action"].data_ptr(),
+                            buf["reward"].data_ptr(), buf["flags"].data_ptr(), None if nx is None else nx.data_ptr())
+        _lib.check(self._lib.gc_collect(self._h, n_steps, kind, _ptr(ptab), float(epsilon), _ptr(state), _ptr(self._t),
+                                        _ptr(index), C.byref(rec), _ptr(self._stats), self._stream()))
+        n = self.num_envs
+        return Transitions(buf["obs"][:, :n], buf["action"][:, :n], buf["reward"][:, :n], buf["flags"][:, :n],
+                           None if nx is None else nx[:, :n])
 
     def capture_steps(self, action_ring):
         """Captures one step per tensor of `action_ring` (int8 [n_cells, ld] device tensors, kept alive

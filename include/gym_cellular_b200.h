@@ -284,6 +284,30 @@ int gc_unpack_cells(int device, int64_t n, int64_t ld, int32_t n_cells, const ui
 int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, int8_t *state,
                int32_t *t, uint32_t *index, float *ret, int32_t *n_unsafe, int64_t *stats, void *stream);
 
+/* Transition record of gc_collect: step-major arrays [n_steps][ld] (element (k, e) at k*ld + e, the handle's ld),
+ * device memory owned by the caller, base pointers 16-byte aligned.  Every pointer may be NULL (not recorded). */
+typedef struct {
+    uint32_t  struct_size;
+    uint32_t *obs;       /* tabular index of the state step k starts from (what gc_step wrote to `index` before it) */
+    uint32_t *action;    /* tabular action index of the action EXECUTED at step k                                 */
+    float    *reward;    /* reward of step k, the bits gc_step writes                                             */
+    uint8_t  *flags;     /* GC_FLAG_UNSAFE | GC_FLAG_TRUNCATED | count << GC_FLAG_COUNT_SHIFT                      */
+    uint32_t *next_obs;  /* tabular index of the successor BEFORE the time-limit auto-reset (== obs[k+1] unless truncated) */
+} gc_record;
+
+/* Experience collection: the fused rollout above (same envs, same kernel, same advance of state, t, index, global
+ * step, statistics and launch count) that also writes every transition into `record`.  Policies:
+ *   GC_POLICY_RANDOM  as in gc_rollout; epsilon must be 0
+ *   GC_POLICY_TABLE   epsilon-greedy, epsilon in [0, 1]: env g at global step G explores iff word (g % 4) of
+ *                     philox(key, ((g/4)_lo, (g/4)_hi, G, 0x50000000)) < ceil(epsilon * 2^32); the explored action is
+ *                     word (g % 4) of philox(key, ((g/4)_lo, (g/4)_hi, G, 0x50000001)) mapped to the joint action
+ *                     floor(word * A^C / 2^32) (cellular) or by the random policy's rule (grid world); otherwise
+ *                     action = policy[obs].  G is the global step even under GC_F_RNG_EPISODIC (exploration is the
+ *                     agent's, not the environment's).  epsilon = 0 draws nothing: gc_rollout's actions exactly.
+ * No per-env return / unsafe count: the record holds the per-step values.  One kernel launch. */
+int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+               int8_t *state, int32_t *t, uint32_t *index, const gc_record *record, int64_t *stats, void *stream);
+
 /* Reads and clears the handle's device status word (synchronises `stream`).  Returns GC_OK or
  * GC_ERR_ACTION if some env received a grid-world action without any go-to position since the
  * last poll (the reference raises KeyError('position'), grid_world.py:143). */
