@@ -291,6 +291,11 @@ int gc_create(const gc_config *cfg, gc_env **out)
                     (long long)((int64_t(1) << 31) / cfg->n_cells));
     if (cfg->env_id_offset < 0 || cfg->env_id_offset % 4 != 0)
         return fail(GC_ERR_INVALID, "env_id_offset must be a non-negative multiple of 4");
+    // probabilities, not thresholds: NaN or a value outside [0, 1] is a caller's mistake, never "never" or "always"
+    if (!(cfg->noise_prob >= 0.0 && cfg->noise_prob <= 1.0))
+        return fail(GC_ERR_INVALID, "noise_prob must lie in [0, 1] (got %g)", cfg->noise_prob);
+    if (!(cfg->dispersal_prob >= 0.0 && cfg->dispersal_prob <= 1.0))
+        return fail(GC_ERR_INVALID, "dispersal_prob must lie in [0, 1] (got %g)", cfg->dispersal_prob);
     if (cfg->kind == GC_KIND_CELLULAR) {
         if (cfg->n_cells < 1 || cfg->n_cells > GC_MAX_CELLS)
             return fail(GC_ERR_INVALID, "n_cells must be in 1..%d", GC_MAX_CELLS);

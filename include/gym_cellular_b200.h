@@ -100,8 +100,8 @@ typedef struct {
                                     (the kernels index with 32-bit element offsets)               */
     int64_t  env_id_offset;      /* global id of env 0 (multiple of 4): RNG streams are keyed by global env id */
     uint64_t seed;               /* Philox key                                                    */
-    double   noise_prob;         /* cellular noise threshold (0.1, cells3resetVdeadlock.py:36)    */
-    double   dispersal_prob;     /* grid-world seed dispersal (0.01, grid_world.py:161)           */
+    double   noise_prob;         /* cellular noise threshold (0.1, cells3resetVdeadlock.py:36), in [0, 1] */
+    double   dispersal_prob;     /* grid-world seed dispersal (0.01, grid_world.py:161), in [0, 1]        */
 } gc_config;
 
 /* Tables of the cellular family (host pointers, copied into the handle).
