@@ -1,10 +1,12 @@
 // C ABI of libgymcellular_b200.so (include/gym_cellular_b200.h).  No C++ exceptions cross the
 // boundary: every entry point returns a gc_status and records a thread-local message.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <memory>
 #include <new>
 
@@ -394,9 +396,30 @@ int gc_set_tables(gc_env *env, const gc_cell_tables *t)
             if (mv < 0 || mv >= S || nz < 0 || nz >= S)
                 return fail(GC_ERR_INVALID, "move/noisy[%d][%d] outside [0, %d)", s, a, S);
             tab.sa[s * GC_LVL_PAD + a] = (uint32_t)mv | ((uint32_t)nz << 4) | ((uint32_t)dr << 8);
+            if (!std::isfinite(t->reward[s * A + a]) || (t->reward_noisy && !std::isfinite(t->reward_noisy[s * A + a])))
+                return fail(GC_ERR_INVALID, "reward/reward_noisy[%d][%d] is not finite", s, a);
             tab.reward[s * GC_LVL_PAD + a] = t->reward[s * A + a];
             tab.reward_noisy[s * GC_LVL_PAD + a] = (t->reward_noisy ? t->reward_noisy : t->reward)[s * A + a];
         }
+    {
+        // The reward statistic adds round(reward * 2^24) as a 32-bit integer per env-step, so every step's reward
+        // must stay below 128 in magnitude.  A step's cell sum lies in [C lo, C hi] for the smallest and largest
+        // table entry, and the float32 sum may pass that by half an ulp (< 2^-18 below 128) per addition.
+        double lo = t->reward[0], hi = t->reward[0];
+        for (int i = 0; i < S * A; ++i)
+            for (const float *r : {t->reward, t->reward_noisy})
+                if (r) { lo = std::min(lo, (double)r[i]); hi = std::max(hi, (double)r[i]); }
+        const double slack = C * std::ldexp(1.0, -18);
+        double bound = std::max(std::fabs(C * lo), std::fabs(C * hi)) + slack;
+        if (env->cfg.flags & GC_F_REWARD_LOG2)
+            bound = 1.0 + C * lo - slack > 0.0
+                        ? std::max(std::fabs(std::log2(1.0 + C * lo - slack)), std::fabs(std::log2(1.0 + C * hi + slack)))
+                        : HUGE_VAL;
+        if (!(bound < 128.0))
+            return fail(GC_ERR_INVALID, "rewards reach %g in magnitude per step (n_cells x the largest |reward|%s): the "
+                        "reward statistic holds |reward| < 128", bound,
+                        (env->cfg.flags & GC_F_REWARD_LOG2) ? ", under log2(1 + .)" : "");
+    }
     for (int j = 0; j < C; ++j)
         for (int s0 = 0; s0 < S; ++s0)
             for (int sp = 0; sp < S; ++sp) {

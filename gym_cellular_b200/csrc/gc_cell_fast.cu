@@ -313,7 +313,7 @@ cell_pair_kernel(const __grid_constant__ CellTables tab, const __grid_constant__
         const uint32_t unsafe_w = ((((present & rowmask) + 0x0F0F0F0Fu) | present) >> 4) & 0x01010101u;
 #pragma unroll
         for (int e = 0; e < kEPT; ++e)
-            if (e < rem) st_reward += __float2int_rn(rout[e] * 16777216.0f);     // |reward| < 128
+            if (e < rem) st_reward += __float2int_rn(rout[e] * 16777216.0f);     // |reward| < 128: gc_set_tables
         {
             const uint32_t vb = valid_bytes(rem);
             st_steps += rem;

@@ -216,7 +216,20 @@ def counted_levels(n_states):
 
 # ---------------------------------------------------------------------------------------------
 # The three debug MDPs (gym_cellular/envs/debug/*.py) as table sets of the same cellular kernel.
-# Each returns the dict `CellularVectorEnv(cell_tables=...)` takes.
+# Each returns the dict `CellularVectorEnv(cell_tables=...)` takes (gc_cell_tables of
+# include/gym_cellular_b200.h):
+#   n_cells, n_states, n_actions   shape C, S, A
+#   move [S][A]              next level without noise
+#   noisy [S][A], draws [S][A]   optional: next level when the draw fires, 1 where (level, action) draws;
+#                            a table set with `draws` is stochastic
+#   reward [S][A]            per-cell reward (lowered to float32); reward_noisy [S][A] optional, used when the
+#                            draw fired
+#   side_effects [C][S][S]   code of row-0 entry j for (s'_0, s'_p), p = 1 for j = 0, else p = j
+#   counted [S]              1 where a level counts towards side_effects_incidence
+#   initial_state [C]        optional: the reset state (default all zero)
+#   reset_row [C]            row 0 of the side-effects matrix reported by reset()
+#   noise_prob               optional: overrides the env's noise probability
+#   se_fill                  optional: the code of the side-effects rows >= 1 (the kernels report row 0 only)
 
 def debug_tables():
     """Debug-v0 (debug/debug.py:76-116, 183-188): 2 cells x 2 levels x 2 actions, next = level XOR

@@ -231,10 +231,12 @@ class CellularVectorEnv(gym.vector.VectorEnv):
     def _set_tables(self):
         S, A, Cn = self.n_states, self.n_actions, self.n_cells
         ct = self._cell_tables
-        reward_noisy, counted = None, tables.counted_levels(S)
+        reward_noisy, counted, init = None, tables.counted_levels(S), np.zeros(Cn)
         if ct is not None:
             move, noisy, draws, se = ct["move"], ct.get("noisy"), ct.get("draws"), ct["side_effects"]
             reward_noisy, counted = ct.get("reward_noisy"), ct["counted"]
+            if ct.get("initial_state") is not None:
+                init = ct["initial_state"]
         elif self.stochastic:
             move, noisy, draws = tables.noise_tables(S, A, self.deadlock)
             se = tables.side_effect_tables(Cn, S, self.difficulty)
@@ -247,11 +249,13 @@ class CellularVectorEnv(gym.vector.VectorEnv):
                 np.ascontiguousarray(self.reward_table, np.float32),
                 np.ascontiguousarray(se, np.int8),
                 np.ascontiguousarray(counted, np.uint8),
-                np.zeros(Cn, np.int8),
+                np.ascontiguousarray(init, np.int8),
                 None if reward_noisy is None else np.ascontiguousarray(reward_noisy, np.float32),
                 None if self.cell_radix is None else np.ascontiguousarray(self.cell_radix, np.int32)]
         if self.cell_radix is not None and len(self.cell_radix) != Cn:
             raise ValueError("cell_radix needs one entry per cell")
+        if len(keep[6]) != Cn:
+            raise ValueError("initial_state needs one entry per cell")
         t = _lib.GcCellTables(*[None if a is None else a.ctypes.data for a in keep])
         _lib.check(self._lib.gc_set_tables(self._h, C.byref(t)))
         self.side_effect_table = se
@@ -270,13 +274,26 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         `env.state = ...` on the reference; the tabular index is refreshed.  `validate` checks the level
         range (one host synchronisation)."""
         cells = torch.as_tensor(cells, device=self.device).to(torch.int8).reshape(self.n_cells, self.num_envs)
-        if validate and (bool((cells < 0).any()) or bool((cells >= self.n_states).any())):
-            raise ValueError(f"state levels must lie in [0, {self.n_states})")
+        if validate:
+            levels = self.n_states if self.cell_radix is None else \
+                torch.tensor(self.cell_radix, dtype=torch.int8, device=self.device)[:, None]
+            if bool((cells < 0).any()) or bool((cells >= levels).any()):
+                raise ValueError(f"state levels must lie in [0, {self.n_states if self.cell_radix is None else self.cell_radix})")
         self._state[:, :self.num_envs].copy_(cells)
         if t is not None:
             self._t[:self.num_envs].copy_(torch.as_tensor(t, device=self.device).to(torch.int32))
-        _lib.check(self._lib.gc_encode(self.device.index, self.num_envs, self.ld, self.n_cells, self.n_states,
-                                       _ptr(self._state), _ptr(self._index), self._stream()))
+        self._encode_state(self._state, self._index, self.num_envs, self.ld)
+
+    def _encode_state(self, cells, index, n, ld):
+        """Tabular index of int8 [n_cells, ld] device levels, with the place values the step kernels use: the
+        uniform radix n_states, or the per-cell `cell_radix` of a ragged state space."""
+        if self.cell_radix is None:
+            _lib.check(self._lib.gc_encode(self.device.index, n, ld, self.n_cells, self.n_states, _ptr(cells),
+                                           _ptr(index), self._stream()))
+        else:
+            radix = np.ascontiguousarray(self.cell_radix, np.int32)
+            _lib.check(self._lib.gc_encode_mixed(self.device.index, n, ld, self.n_cells, radix.ctypes.data, None,
+                                                 _ptr(cells), _ptr(index), self._stream()))
 
     def tabular_state(self, dtype=torch.int64):
         """Tabular index of the current observation (uint32 payload widened to `dtype`)."""
@@ -297,9 +314,13 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             pad = torch.zeros(cells.shape[0], ld, dtype=torch.int8, device=self.device)
             pad[:, :n] = cells
             cells = pad
-        radix = self.n_states if space == "state" else self.n_actions
         out = torch.empty(ld, dtype=torch.int32, device=self.device)
-        _lib.check(self._lib.gc_encode(self.device.index, n, ld, cells.shape[0], radix, _ptr(cells), _ptr(out), self._stream()))
+        if space == "state" and self.cell_radix is not None:
+            self._encode_state(cells, out, n, ld)
+        else:
+            radix = self.n_states if space == "state" else self.n_actions
+            _lib.check(self._lib.gc_encode(self.device.index, n, ld, cells.shape[0], radix, _ptr(cells), _ptr(out),
+                                           self._stream()))
         return out[:n].to(torch.int64) & 0xFFFFFFFF
 
     def detabularize(self, index, space="state"):
@@ -310,9 +331,15 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         ld = _round_up(n, 16)
         idx = torch.zeros(ld, dtype=torch.int32, device=self.device)
         idx[:n] = (index.to(torch.int64) & 0xFFFFFFFF).to(torch.int32) if index.dtype != torch.int32 else index
-        radix = self.n_states if space == "state" else self.n_actions
         out = torch.empty(self.n_cells, ld, dtype=torch.int8, device=self.device)
-        _lib.check(self._lib.gc_decode(self.device.index, n, ld, self.n_cells, radix, _ptr(idx), _ptr(out), self._stream()))
+        if space == "state" and self.cell_radix is not None:
+            radix = np.ascontiguousarray(self.cell_radix, np.int32)
+            _lib.check(self._lib.gc_decode_mixed(self.device.index, n, ld, self.n_cells, radix.ctypes.data, None,
+                                                 _ptr(idx), _ptr(out), self._stream()))
+        else:
+            radix = self.n_states if space == "state" else self.n_actions
+            _lib.check(self._lib.gc_decode(self.device.index, n, ld, self.n_cells, radix, _ptr(idx), _ptr(out),
+                                           self._stream()))
         return out[:, :n]
 
     def materialise(self, i):
@@ -358,8 +385,7 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             self._stats.copy_(sd["stats"])
         _lib.check(self._lib.gc_set_global_step(self._h, int(sd["global_step"])))
         # refresh the tabular index of the restored state
-        _lib.check(self._lib.gc_encode(self.device.index, self.num_envs, self.ld, self.n_cells, self.n_states,
-                                       _ptr(self._state), _ptr(self._index), self._stream()))
+        self._encode_state(self._state, self._index, self.num_envs, self.ld)
 
     @property
     def launch_count(self):
@@ -750,10 +776,12 @@ class _FinalInfo(dict):
     def __missing__(self, key):
         env = self._env
         if key == "tabular_state":
-            radix = 20 if env.kind == "gridworld" else env.n_states
             out = torch.empty(env.ld, dtype=torch.int32, device=env.device)
-            _lib.check(env._lib.gc_encode(env.device.index, env.num_envs, env.ld, env.n_cells, radix,
-                                          _ptr(env._final), _ptr(out), env._stream()))
+            if env.kind == "gridworld":
+                _lib.check(env._lib.gc_encode(env.device.index, env.num_envs, env.ld, env.n_cells, 20,
+                                              _ptr(env._final), _ptr(out), env._stream()))
+            else:
+                env._encode_state(env._final, out, env.num_envs, env.ld)
             return out[:env.num_envs].to(torch.int64) & 0xFFFFFFFF
         if key in ("unsafe", "count", "side_effects"):
             return env._v_infos[key]

@@ -83,7 +83,8 @@ typedef enum {
 #define GC_STAT_UNSAFE      1 /* steps whose side-effects row contains 'unsafe'                  */
 #define GC_STAT_COUNT       2 /* sum of polarised cells (cellular) / barren jurisdictions (grid) */
 #define GC_STAT_TRUNCATED   3 /* episodes ended by the time limit                                */
-#define GC_STAT_REWARD_Q24  4 /* sum of round(reward * 2^24): order-independent, exact across GPUs */
+#define GC_STAT_REWARD_Q24  4 /* sum of round(reward * 2^24): order-independent, exact across GPUs (each
+                                 term is a 32-bit integer: gc_set_tables keeps |reward| < 128) */
 
 typedef struct {
     uint32_t struct_size;        /* sizeof(gc_config), for ABI evolution                          */
@@ -108,9 +109,13 @@ typedef struct {
  *   move   [S][A] int8   next level without noise          (cells3states3actions3.py:133-154)
  *   noisy  [S][A] int8   next level when the draw fires    (cells3resetVdeadlock.py:37-41)
  *   draws  [S][A] uint8  1 if (level, action) consumes a draw (cells3resetVdeadlock.py:49-60)
- *   reward [S][A] float  per-cell reward of the OLD level  (cells3states3actions3.py:9-45)
+ *   reward [S][A] float  per-cell reward of the OLD level  (cells3states3actions3.py:9-45); finite
  *   reward_noisy [S][A] float  optional: per-cell reward when the draw fired, for rewards that depend on
- *          the NEXT level (debug/deep_exploration.py:11-16); NULL = same as `reward`
+ *          the NEXT level (debug/deep_exploration.py:11-16); NULL = same as `reward`; finite
+ *          Bound: every step's reward must stay below 128 in magnitude.  With lo / hi the smallest / largest
+ *          entry of reward and reward_noisy, gc_set_tables requires n_cells * max(|lo|, |hi|) < 128 (under
+ *          GC_F_REWARD_LOG2: 1 + n_cells * lo > 0 and |log2(1 + n_cells * lo)|, |log2(1 + n_cells * hi)| < 128),
+ *          with a margin of n_cells * 2^-18 for the float32 sum.
  *   side_effects [C][S][S] int8  code (0 silent, 1 safe, 2 unsafe) of row-0 entry j of the
  *          side-effects matrix as a function of (s'_0, s'_p), p = 1 for j = 0 and p = j otherwise
  *          (cells3states3actions3.py:157-212; only row 0 is ever written by the reference)

@@ -9,7 +9,8 @@ its exact boundary; `search` finds draws of a wanted shape.
                                     (half h = the low half of word h // 2 for even h, the high half for odd h)
   grid-world dispersal trigger:     philox(g // 4, T, 0)[g % 4]
   collect explore test:             philox(g // 4, G, 0x50000000)[g % 4]  (G = the global step)
-T is the episode step of the env under rng_episodic, else the global step.
+T is the episode step of the env under rng_episodic, else the global step.  The cellular draws take T as a scalar or as
+a per-env array [n] (episodic envs at different episode steps).
 """
 from types import SimpleNamespace
 
@@ -29,7 +30,7 @@ def _ids(first, n):
 
 
 def wide_tops(seed, n_cells, first, n, T):
-    """uint32 [n_cells, n]: top halves of the wide draws of envs first .. first + n - 1 at counter T."""
+    """uint32 [n_cells, n]: top halves of the wide draws of envs first .. first + n - 1 at counter T (scalar or [n])."""
     lo, hi = _ids(first, n)
     blocks = [np.stack(philox(lo, hi, T, b, seed)) for b in range((n_cells + 7) // 8)]
     return np.stack([(blocks[c // 8][(c % 8) // 2] >> np.uint32(16 * (c % 2))) & np.uint32(0xFFFF)
@@ -37,13 +38,14 @@ def wide_tops(seed, n_cells, first, n, T):
 
 
 def wide_lows(seed, cells, first, n, T):
-    """uint32 [len(cells), n]: low halves of the wide draws of the given cells."""
+    """uint32 [len(cells), n]: low halves of the wide draws of the given cells (T scalar or [n])."""
     lo, hi = _ids(first, n)
     return np.stack([philox(lo, hi, T, NOISE_LOW_STREAM + c, seed)[0] >> np.uint32(16) for c in cells])
 
 
 def cell_draws(seed, n_cells, first, n, T):
-    """uint32 [n_cells, n]: the 32-bit noise draw of every cell of envs first .. first + n - 1 at counter T."""
+    """uint32 [n_cells, n]: the 32-bit noise draw of every cell of envs first .. first + n - 1 at counter T (scalar or
+    [n])."""
     if n_cells <= NARROW_CELLS:
         lo, hi = _ids(first, n)
         return np.stack(philox(lo, hi, T, 0, seed))[:n_cells]
