@@ -6,7 +6,7 @@ Host code is Python; the hot path is hand-written CUDA for sm_100a behind a C AB
 from ._gym import gym  # noqa: F401  (real gymnasium, or the structural stand-in)
 from . import tables
 from .tables import right_polarizing, multiple_optima, nonlinear, nonlinear_right_polarizing
-from .vector_env import CellularVectorEnv, Transitions, make_vector_env
+from .vector_env import CellularVectorEnv, Counts, Transitions, make_vector_env
 from .packed_env import PackedCellularVectorEnv
 from .device_codec import encode_mixed, decode_mixed
 from .codec import (generalized_cellular2tabular, generalized_tabular2cellular, cellular2tabular,
@@ -17,7 +17,7 @@ from .envs import (Cells3States3Actions3Env, Cells2Rest3Env, Cells3ResetVDeadloc
 from . import registration  # noqa: F401  (registers the gym_cellular/<Name>-v0 ids)
 from .alias import install_alias
 
-__all__ = ["CellularVectorEnv", "PackedCellularVectorEnv", "Transitions", "make_vector_env", "tables", "right_polarizing", "multiple_optima",
+__all__ = ["CellularVectorEnv", "PackedCellularVectorEnv", "Transitions", "Counts", "make_vector_env", "tables", "right_polarizing", "multiple_optima",
            "nonlinear", "nonlinear_right_polarizing", "Cells3States3Actions3Env", "Cells2Rest3Env",
            "Cells3ResetVDeadlockEnv", "GridWorldEnv", "PriorKnowledge", "GridWorldPriorKnowledge",
            "generalized_cellular2tabular", "generalized_tabular2cellular", "cellular2tabular", "tabular2cellular",

@@ -20,7 +20,7 @@ POLICY_RANDOM, POLICY_TABLE = 0, 1
 
 EXPORTS = ["gc_abi_version", "gc_last_error", "gc_create", "gc_destroy", "gc_set_tables", "gc_set_final_obs",
            "gc_set_global_step", "gc_get_global_step", "gc_sync_global_step", "gc_launch_count", "gc_reset", "gc_step",
-           "gc_bind_step", "gc_step_bound", "gc_step_many", "gc_prepare_step_many", "gc_step_host", "gc_rollout", "gc_collect", "gc_poll_status", "gc_encode",
+           "gc_bind_step", "gc_step_bound", "gc_step_many", "gc_prepare_step_many", "gc_step_host", "gc_rollout", "gc_collect", "gc_collect_counts", "gc_poll_status", "gc_encode",
            "gc_decode", "gc_encode_mixed", "gc_decode_mixed", "gc_reset_packed", "gc_step_packed", "gc_bind_step_packed",
            "gc_step_host_packed", "gc_pack_cells", "gc_unpack_cells"]
 FLAG_UNSAFE, FLAG_TRUNCATED, FLAG_COUNT_SHIFT = 1, 2, 2
@@ -44,6 +44,12 @@ class GcRecord(C.Structure):
     """gc_record: step-major [n_steps][ld] device arrays of gc_collect (NULL = not recorded)."""
     _fields_ = [("struct_size", C.c_uint32), ("obs", C.c_void_p), ("action", C.c_void_p), ("reward", C.c_void_p),
                 ("flags", C.c_void_p), ("next_obs", C.c_void_p)]
+
+
+class GcCounts(C.Structure):
+    """gc_counts: int64 device count tables of gc_collect_counts (NULL = not counted)."""
+    _fields_ = [("struct_size", C.c_uint32), ("visits", C.c_void_p), ("next", C.c_void_p), ("reward_q24", C.c_void_p),
+                ("unsafe", C.c_void_p), ("cell_next", C.c_void_p)]
 
 
 class GcError(RuntimeError):
@@ -86,6 +92,7 @@ def load():
     L.gc_step_host.argtypes = [vp] * 21 + [i64]
     L.gc_rollout.argtypes = [vp, C.c_int32, C.c_int32] + [vp] * 8
     L.gc_collect.argtypes = [vp, C.c_int32, C.c_int32, vp, C.c_double, vp, vp, vp, C.POINTER(GcRecord), vp, vp]
+    L.gc_collect_counts.argtypes = [vp, C.c_int32, C.c_int32, vp, C.c_double, vp, vp, vp, C.POINTER(GcCounts), vp, vp]
     L.gc_poll_status.argtypes = [vp, vp]
     L.gc_encode.argtypes = [C.c_int, i64, i64, C.c_int32, C.c_int32, vp, vp, vp]
     L.gc_decode.argtypes = [C.c_int, i64, i64, C.c_int32, C.c_int32, vp, vp, vp]

@@ -883,6 +883,37 @@ RolloutIO make_rollout_io(const gc_env *env, int32_t n_steps, int32_t policy_kin
 
 bool misaligned(const void *p) { return p && (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
 
+// argument checks shared by gc_collect and gc_collect_counts, so that both reject the same calls (out = the record or
+// the count struct)
+int check_collect_args(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+                       const int8_t *state, const int32_t *t, const uint32_t *index, const void *out)
+{
+    if (int rc = check_env(env)) return rc;
+    if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
+    if (!state || !t || !index || !out) return fail(GC_ERR_INVALID, "a required pointer is NULL");
+    if (n_steps < 1) return fail(GC_ERR_INVALID, "n_steps must be >= 1");
+    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE) return fail(GC_ERR_INVALID, "unknown policy kind");
+    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
+    if (!(epsilon >= 0.0 && epsilon <= 1.0)) return fail(GC_ERR_INVALID, "epsilon must lie in [0, 1] (got %g)", epsilon);
+    if (policy_kind == GC_POLICY_RANDOM && epsilon != 0.0)
+        return fail(GC_ERR_INVALID, "epsilon applies to GC_POLICY_TABLE only (GC_POLICY_RANDOM needs epsilon 0)");
+    return GC_OK;
+}
+
+// RolloutIO of a gc_collect / gc_collect_counts launch: the rollout's, plus the epsilon-greedy fields
+RolloutIO make_collect_io(const gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+                          int8_t *state, int32_t *t, uint32_t *index, int64_t *stats)
+{
+    RolloutIO io = make_rollout_io(env, n_steps, policy_kind, policy, state, t, index, stats);
+    unsigned long long joint = 1;
+    for (int c = 0; c < env->cfg.n_cells; ++c) joint *= static_cast<unsigned long long>(env->cfg.n_actions);
+    io.joint_actions = joint;
+    const unsigned long long thr = threshold_of(epsilon);
+    io.explore_thr_nz = thr != 0 ? 1u : 0u;
+    io.explore_thr_m1 = static_cast<uint32_t>(thr - 1);
+    return io;
+}
+
 }  // namespace
 
 int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, int8_t *state,
@@ -917,15 +948,7 @@ int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
                int8_t *state, int32_t *t, uint32_t *index, const gc_record *record, int64_t *stats, void *stream)
 {
     GC_NVTX("gc_collect");
-    if (int rc = check_env(env)) return rc;
-    if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
-    if (!state || !t || !index || !record) return fail(GC_ERR_INVALID, "a required pointer is NULL");
-    if (n_steps < 1) return fail(GC_ERR_INVALID, "n_steps must be >= 1");
-    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE) return fail(GC_ERR_INVALID, "unknown policy kind");
-    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
-    if (!(epsilon >= 0.0 && epsilon <= 1.0)) return fail(GC_ERR_INVALID, "epsilon must lie in [0, 1] (got %g)", epsilon);
-    if (policy_kind == GC_POLICY_RANDOM && epsilon != 0.0)
-        return fail(GC_ERR_INVALID, "epsilon applies to GC_POLICY_TABLE only (GC_POLICY_RANDOM needs epsilon 0)");
+    if (int rc = check_collect_args(env, n_steps, policy_kind, policy, epsilon, state, t, index, record)) return rc;
     if (record->struct_size != sizeof(gc_record))
         return fail(GC_ERR_INVALID, "record->struct_size %u != sizeof(gc_record) %zu", record->struct_size, sizeof(gc_record));
     if (misaligned(record->obs) || misaligned(record->action) || misaligned(record->reward) || misaligned(record->flags) ||
@@ -934,15 +957,9 @@ int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     if (env->cfg.kind == GC_KIND_CELLULAR && !env->fast_ok)
         return fail(GC_ERR_INVALID, "gc_collect supports the cellular family with n_states, n_actions <= 4 only");
     GC_ON_DEVICE(env->cfg.device);
-    RolloutIO io = make_rollout_io(env, n_steps, policy_kind, policy, state, t, index, stats);
+    RolloutIO io = make_collect_io(env, n_steps, policy_kind, policy, epsilon, state, t, index, stats);
     io.rec_obs = record->obs; io.rec_action = record->action; io.rec_reward = record->reward;
     io.rec_flags = record->flags; io.rec_next_obs = record->next_obs;
-    unsigned long long joint = 1;
-    for (int c = 0; c < env->cfg.n_cells; ++c) joint *= static_cast<unsigned long long>(env->cfg.n_actions);
-    io.joint_actions = joint;
-    const unsigned long long thr = threshold_of(epsilon);
-    io.explore_thr_nz = thr != 0 ? 1u : 0u;
-    io.explore_thr_m1 = static_cast<uint32_t>(thr - 1);
     cudaError_t e;
     if (env->cfg.kind == GC_KIND_CELLULAR)
         e = gc_launch_cell_collect(env->tab, io, env->d_pair_lut, (env->cfg.flags & GC_F_NOISE) != 0, env->n_sm,
@@ -950,6 +967,62 @@ int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     else
         e = gc_launch_grid_collect(env->grid, io, env->n_sm, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return fail(GC_ERR_CUDA, "collect kernel launch failed: %s", cudaGetErrorString(e));
+    env->launches += 1;
+    env->global_step += n_steps;
+    return GC_OK;
+}
+
+int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+                      int8_t *state, int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream)
+{
+    GC_NVTX("gc_collect_counts");
+    if (int rc = check_collect_args(env, n_steps, policy_kind, policy, epsilon, state, t, index, counts)) return rc;
+    if (counts->struct_size != sizeof(gc_counts))
+        return fail(GC_ERR_INVALID, "counts->struct_size %u != sizeof(gc_counts) %zu", counts->struct_size, sizeof(gc_counts));
+    const void *ptrs[5] = {counts->visits, counts->next, counts->reward_q24, counts->unsafe, counts->cell_next};
+    bool any = false;
+    for (const void *p : ptrs) {
+        if (p && (reinterpret_cast<uintptr_t>(p) & 7u) != 0) return fail(GC_ERR_INVALID, "count pointers must be 8-byte aligned");
+        any = any || p;
+    }
+    if (!any) return fail(GC_ERR_INVALID, "every count pointer is NULL: nothing to count");
+    const bool cellular = env->cfg.kind == GC_KIND_CELLULAR;
+    if (!cellular && counts->cell_next) return fail(GC_ERR_INVALID, "cell_next counts the cellular family only, not grid world");
+    if (cellular && !env->fast_ok)
+        return fail(GC_ERR_INVALID, "gc_collect_counts supports the cellular family with n_states, n_actions <= 4 only");
+    // joint table sizes, saturated above the 2^31-entry limit (indices are 32-bit in the kernels)
+    constexpr unsigned long long kJointLimit = 1ull << 31;
+    auto sat_mul = [](unsigned long long a, unsigned long long b) { return a > kJointLimit || b > kJointLimit || a * b > kJointLimit ? kJointLimit + 1 : a * b; };
+    unsigned long long nS = 400, nA = 25;
+    if (cellular) {
+        nS = nA = 1;
+        for (int c = 0; c < env->cfg.n_cells; ++c) {
+            nS = sat_mul(nS, static_cast<unsigned long long>(env->cfg.n_states));
+            nA = sat_mul(nA, static_cast<unsigned long long>(env->cfg.n_actions));
+        }
+    }
+    const unsigned long long n_sa = sat_mul(nS, nA), n_sas = sat_mul(n_sa, nS);
+    if ((counts->visits || counts->reward_q24 || counts->unsafe) && n_sa > kJointLimit)
+        return fail(GC_ERR_INVALID, "the joint (state, action) tables would have more than 2^31 entries: count cell_next only");
+    if (counts->next && n_sas > kJointLimit)
+        return fail(GC_ERR_INVALID, "the joint 'next' table would have more than 2^31 entries");
+    GC_ON_DEVICE(env->cfg.device);
+    RolloutIO io = make_collect_io(env, n_steps, policy_kind, policy, epsilon, state, t, index, stats);
+    CountIO cnt;
+    cnt.visits = reinterpret_cast<unsigned long long *>(counts->visits);
+    cnt.next = reinterpret_cast<unsigned long long *>(counts->next);
+    cnt.reward_q24 = reinterpret_cast<unsigned long long *>(counts->reward_q24);
+    cnt.unsafe = reinterpret_cast<unsigned long long *>(counts->unsafe);
+    cnt.cell_next = reinterpret_cast<unsigned long long *>(counts->cell_next);
+    cnt.n_states = static_cast<uint32_t>(nS);          // used only when a joint table fits, i.e. nS, nA <= 2^31
+    cnt.n_actions = static_cast<uint32_t>(nA);
+    cudaError_t e;
+    if (cellular)
+        e = gc_launch_cell_count(env->tab, io, cnt, env->d_pair_lut, (env->cfg.flags & GC_F_NOISE) != 0, env->n_sm,
+                                 static_cast<cudaStream_t>(stream));
+    else
+        e = gc_launch_grid_count(env->grid, io, cnt, env->n_sm, static_cast<cudaStream_t>(stream));
+    if (e != cudaSuccess) return fail(GC_ERR_CUDA, "count kernel launch failed: %s", cudaGetErrorString(e));
     env->launches += 1;
     env->global_step += n_steps;
     return GC_OK;

@@ -103,6 +103,17 @@ struct RolloutIO {
     uint32_t explore_thr_m1, explore_thr_nz; // the table policy explores iff thr_nz && word <= thr_m1 (P = eps)
 };
 
+// gc_collect_counts (the COUNT rollout kernels): int64 counters the kernels add to, NULL = not counted.  A kernel
+// parameter of its own, after the others, so that RolloutIO and the other kernels' parameters keep their layout.
+struct CountIO {
+    unsigned long long *visits;        // [nS][nA]
+    unsigned long long *next;          // [nS][nA][nS]
+    unsigned long long *reward_q24;    // [nS][nA], two's complement
+    unsigned long long *unsafe;        // [nS][nA]
+    unsigned long long *cell_next;     // [C][S][A][S], cellular only
+    uint32_t n_states, n_actions;      // nS, nA of the joint tables
+};
+
 // Constant tables of the cellular family, passed by value as a __grid_constant__ parameter and
 // staged into shared memory once per block.
 struct CellTables {
@@ -196,6 +207,10 @@ cudaError_t gc_launch_grid_rollout(const GridParams &gp, const RolloutIO &io, in
 cudaError_t gc_launch_cell_collect(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise,
                                    int n_sm, cudaStream_t stream);
 cudaError_t gc_launch_grid_collect(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t stream);
+// the same kernels adding every transition to the counters of `cnt` (gc_collect_counts)
+cudaError_t gc_launch_cell_count(const CellTables &tab, const RolloutIO &io, const CountIO &cnt, const uint2 *lut,
+                                 bool noise, int n_sm, cudaStream_t stream);
+cudaError_t gc_launch_grid_count(const GridParams &gp, const RolloutIO &io, const CountIO &cnt, int n_sm, cudaStream_t stream);
 cudaError_t gc_launch_grid_step(const GridParams &gp, const StepIO &io, int rng_mode, int n_sm,
                                 cudaStream_t stream);
 cudaError_t gc_launch_reset(int n_cells, const int8_t *init, uint32_t init_index, const uint8_t *mask,

@@ -26,12 +26,26 @@
 //   floor(word * A^C / 2^32), grid world the random policy's rule.
 // G is the global step even for episodic envs: exploration belongs to the agent, and keying it by the episode
 // step would make every episode explore at the same steps with the same actions.
+//
+// Experience counts (gc_collect_counts): the COUNT instantiations take the same actions and draws as the RECORD
+// ones and add each transition to per-(state, action) counters instead of writing it out; no draw is added.
+//   joint tables: one warp-aggregated 64-bit global atomic per group of lanes on the same bin (__match_any_sync),
+//     since after a reset every env of a warp sits in the same state and, under a table policy, acts alike;
+//   per-cell N_c(s_c, a_c, s'_c): a 32-bit shared-memory histogram per block, [C][4][4][4], flushed at block exit.
+//     The add that takes a bin across 2^31 moves 2^31 to global memory, so no shared bin wraps as long as fewer than
+//     2^31 further adds land on it before that subtraction does (each add is at most 4, and the subtraction is the
+//     next instruction of the thread that crossed).
 #include "gc_device.cuh"
 
 namespace {
 
 constexpr uint32_t kActionStream = 0x40000000u;
 constexpr uint32_t kExploreStream = 0x50000000u;     // + 0: explore test, + 1: explore action
+
+// what a rollout kernel does with the transitions: nothing (gc_rollout), record them (gc_collect), count them
+// (gc_collect_counts).  RECORD and COUNT take the table policy epsilon-greedily.
+constexpr int kRollout = 0, kRecord = 1, kCount = 2;
+constexpr uint32_t kCellFlush = 1u << 31;           // per-cell shared bin: moved to global memory at 2^31
 
 __device__ __forceinline__ bool same4(const int (&t)[kEPT]) { return t[0] == t[1] && t[1] == t[2] && t[2] == t[3]; }
 
@@ -58,6 +72,13 @@ __device__ __forceinline__ uint32_t random_grid_action(uint32_t w)
     return (w >> 31) ? (4u + 5u * pos) : (pos + 20u);
 }
 
+// per-cell bin s * 16 + a * 4 + s' of cell c -> flat index of the caller's [C][S][A][S] table
+__device__ __forceinline__ uint32_t cell_bin(const CellTables &tab, uint32_t c, uint32_t bin)
+{
+    const uint32_t S = static_cast<uint32_t>(tab.n_states), A = static_cast<uint32_t>(tab.n_actions);
+    return ((c * S + (bin >> 4)) * A + ((bin >> 2) & 3u)) * S + (bin & 3u);
+}
+
 // epsilon-greedy (RECORD kernels): bit e of the result is set when env e of the thread explores at global step G;
 // w then holds the explore-action words (drawn only when one of the 4 envs explores)
 __device__ __forceinline__ uint32_t explore_words(const RolloutIO &io, uint32_t grp_lo, uint32_t grp_hi, uint32_t G,
@@ -73,12 +94,47 @@ __device__ __forceinline__ uint32_t explore_words(const RolloutIO &io, uint32_t 
     return m;
 }
 
+// lanes of this warp inside the env loop at this iteration (a prefix: lane l owns env e0 + 4 (l - lane))
+__device__ __forceinline__ unsigned live_lanes(int64_t e0, int64_t n)
+{
+    const int64_t left = n - (e0 - kEPT * static_cast<int64_t>(threadIdx.x & 31));
+    return left > 31 * kEPT ? 0xFFFFFFFFu : (1u << static_cast<uint32_t>((left + kEPT - 1) / kEPT)) - 1u;   // shift < 32
+}
+
+// one env per lane of the joint tables: bin sa = s * nA + a, successor nx, reward term q24 (round(r * 2^24)),
+// 'unsafe' uns.  Lanes on the same bin add as one group; valid = false lanes (past the batch) count nothing.
+__device__ __forceinline__ void count_joint(const CountIO &cnt, unsigned lanes, bool valid, uint32_t sa, uint32_t nx,
+                                            int32_t q24, uint32_t uns)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    const unsigned peers = __match_any_sync(lanes, valid ? sa : 0xFFFFFFFFu);
+    const bool leader = valid && static_cast<uint32_t>(__ffs(peers) - 1) == lane;
+    if (cnt.visits && leader) atomicAdd(cnt.visits + sa, static_cast<unsigned long long>(__popc(peers)));
+    if (cnt.unsafe) {
+        const unsigned u = __ballot_sync(lanes, uns != 0u) & peers;
+        if (leader && u) atomicAdd(cnt.unsafe + sa, static_cast<unsigned long long>(__popc(u)));
+    }
+    if (cnt.reward_q24) {                 // |q24| < 2^31: 16-bit halves, so that a group of 32 cannot overflow
+        const uint32_t lo = __reduce_add_sync(peers, static_cast<uint32_t>(q24) & 0xFFFFu);
+        const int hi = __reduce_add_sync(peers, q24 >> 16);
+        const long long sum = static_cast<long long>(hi) * 65536 + lo;
+        if (leader && sum) atomicAdd(cnt.reward_q24 + sa, static_cast<unsigned long long>(sum));
+    }
+    if (cnt.next) {
+        const uint32_t sas = sa * cnt.n_states + nx;
+        const unsigned p2 = __match_any_sync(lanes, valid ? sas : 0xFFFFFFFFu);
+        if (valid && static_cast<uint32_t>(__ffs(p2) - 1) == lane)
+            atomicAdd(cnt.next + sas, static_cast<unsigned long long>(__popc(p2)));
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
-template <int C, bool NOISE, bool RECORD>
+template <int C, bool NOISE, int MODE>
 __global__ void __launch_bounds__(kThreads, 2)
 cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constant__ RolloutIO io,
-                    const uint2 *__restrict__ lut)
+                    const uint2 *__restrict__ lut, const __grid_constant__ CountIO cnt)
 {
+    constexpr bool RECORD = MODE == kRecord, EXPLORE = MODE != kRollout;
     constexpr int N_PAIR = NOISE ? GC_PAIR_LUT_PAIRS : 256;
     constexpr int N_SINGLE = NOISE ? 32 : 16;
     constexpr int NPAIR = C / 2;
@@ -86,7 +142,10 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
     __shared__ uint2 s_pair[N_PAIR];
     __shared__ uint2 s_single[N_SINGLE];
     __shared__ unsigned long long s_stats[5];
+    __shared__ uint32_t s_cell[MODE == kCount ? C * 64 : 1];        // N_c(s, a, s') at c * 64 + s * 16 + a * 4 + s'
     const uint32_t step0 = io.step_ctr ? *reinterpret_cast<const volatile uint32_t *>(io.step_ctr) : 0u;
+    if constexpr (MODE == kCount)
+        for (int i = threadIdx.x; i < C * 64; i += blockDim.x) s_cell[i] = 0;
     for (int i = threadIdx.x; i < N_PAIR; i += blockDim.x) s_pair[i] = lut[i];
     if (threadIdx.x < N_SINGLE) s_single[threadIdx.x] = lut[GC_PAIR_LUT_PAIRS + threadIdx.x];
     if (threadIdx.x < 5) s_stats[threadIdx.x] = 0;
@@ -140,7 +199,7 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                 uint32_t p[kEPT];
 #pragma unroll
                 for (int e = 0; e < kEPT; ++e) p[e] = static_cast<uint32_t>(__ldg(io.policy + idx[e]));
-                if constexpr (RECORD) {
+                if constexpr (EXPLORE) {
                     uint32_t xw[kEPT];
                     const uint32_t xm = explore_words(io, grp_lo, grp_hi, step0 + static_cast<uint32_t>(k), xw);
 #pragma unroll
@@ -275,6 +334,51 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                     st_stream_v4(io.rec_next_obs + kofs + e0, make_int4(nx[0], nx[1], nx[2], nx[3]));
                 }
             }
+            if constexpr (MODE == kCount) {
+                if (cnt.cell_next) {
+#pragma unroll
+                    for (int c = 0; c < C; ++c) {
+                        const uint32_t b = (sw[c] << 4) | (aw[c] << 2) | rows[c];     // bytes s * 16 + a * 4 + s'
+                        auto add = [&](uint32_t bin, uint32_t v) {
+                            const uint32_t old = atomicAdd(&s_cell[c * 64 + bin], v);
+                            if (old < kCellFlush && old + v >= kCellFlush) {
+                                atomicSub(&s_cell[c * 64 + bin], kCellFlush);
+                                atomicAdd(cnt.cell_next + cell_bin(tab, c, bin), static_cast<unsigned long long>(kCellFlush));
+                            }
+                        };
+                        if (rem == kEPT && b == __byte_perm(b, 0, 0x0000)) {
+                            add(b & 0xFFu, 4u);
+                        } else {
+#pragma unroll
+                            for (int e = 0; e < kEPT; ++e)
+                                if (e < rem) add(byte_of(b, e), 1u);
+                        }
+                    }
+                }
+                if (cnt.visits || cnt.next || cnt.reward_q24 || cnt.unsafe) {
+                    if (io.policy_kind != GC_POLICY_TABLE) fold_index();
+                    // executed action sum_c a_c A^c, as recorded above (kept apart so that the RECORD kernels stay as
+                    // they were compiled before the COUNT mode existed)
+                    const uint32_t A2 = A * A, pl4[4] = {1u, A, A2, A2 * A};
+                    uint32_t ai[kEPT] = {0, 0, 0, 0}, nx[kEPT] = {0, 0, 0, 0}, plg = 1u;
+#pragma unroll
+                    for (int g = 0; g < (C + 3) / 4; ++g) {
+                        uint32_t q = 0;
+#pragma unroll
+                        for (int i = 0; i < 4; ++i)
+                            if (4 * g + i < C) q += aw[4 * g + i] * pl4[i];
+#pragma unroll
+                        for (int e = 0; e < kEPT; ++e) ai[e] += byte_of(q, e) * plg;
+                        plg *= A2 * A2;
+                    }
+                    if (cnt.next) fold_words(rows, nx);
+                    const unsigned lanes = live_lanes(e0, io.n);
+#pragma unroll
+                    for (int e = 0; e < kEPT; ++e)
+                        count_joint(cnt, lanes, e < rem, idx[e] * cnt.n_actions + ai[e], nx[e],
+                                    __float2int_rn(rlog[e] * 16777216.0f), byte_of(unsafe_w, e));
+                }
+            }
 #pragma unroll
             for (int c = 0; c < C; ++c)
                 sw[c] = (rows[c] & keep) | ((0x01010101u * static_cast<uint8_t>(tab.init[c])) & ~keep);
@@ -284,10 +388,17 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
         for (int c = 0; c < C; ++c) st_stream_u32(io.state + c * ld + e0, sw[c]);
         st_stream_v4(io.t + e0, make_int4(t[0], t[1], t[2], t[3]));
         st_stream_v4(io.index + e0, make_int4(idx[0], idx[1], idx[2], idx[3]));
-        if constexpr (!RECORD) {
+        if constexpr (MODE == kRollout) {
             st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
                                                 __float_as_int(ret[2]), __float_as_int(ret[3])));
             st_stream_v4(io.n_unsafe + e0, make_int4(nuns[0], nuns[1], nuns[2], nuns[3]));
+        }
+    }
+    if constexpr (MODE == kCount) {
+        if (cnt.cell_next) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < C * 64; i += blockDim.x)
+                if (s_cell[i]) atomicAdd(cnt.cell_next + cell_bin(tab, i >> 6, i & 63u), static_cast<unsigned long long>(s_cell[i]));
         }
     }
     if (io.stats) {
@@ -298,10 +409,13 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
 }
 
 // ---------------------------------------------------------------------------------------------
-template <bool RECORD>
-__global__ void __launch_bounds__(kThreads, 4)
-grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant__ RolloutIO io)
+// COUNT: the warp-aggregated adds need registers that 4 blocks per SM (64 per thread) do not leave
+template <int MODE>
+__global__ void __launch_bounds__(kThreads, MODE == kCount ? 2 : 4)
+grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant__ RolloutIO io,
+                    const __grid_constant__ CountIO cnt)
 {
+    constexpr bool RECORD = MODE == kRecord, EXPLORE = MODE != kRollout;
     __shared__ uint32_t s_lut[GC_GRID_LUT_ENTRIES];
     __shared__ unsigned long long s_stats[5];
     const uint32_t step0 = io.step_ctr ? *reinterpret_cast<const volatile uint32_t *>(io.step_ctr) : 0u;
@@ -342,7 +456,7 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                     act[e] = static_cast<uint32_t>(__ldg(io.policy + (tab < 400u ? tab : 0u)));
                     if (act[e] > 24u) act[e] = 24u;
                 }
-                if constexpr (RECORD) {
+                if constexpr (EXPLORE) {
                     uint32_t xw[kEPT];
                     const uint32_t xm = explore_words(io, grp_lo, grp_hi, step0 + static_cast<uint32_t>(k), xw);
 #pragma unroll
@@ -374,7 +488,9 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                 }
             }
             uint32_t count_w = 0, trunc_w = 0, rew_w = 0;
-            uint32_t nx[kEPT];
+            uint32_t nx[kEPT], ob[kEPT];
+#pragma unroll
+            for (int e = 0; e < kEPT; ++e) ob[e] = c0[e] + 20u * c1[e];
 #pragma unroll
             for (int e = 0; e < kEPT; ++e) {
                 const uint32_t ix = (c0[e] + 20u * c1[e]) * 25u + act[e];
@@ -413,12 +529,18 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                     st_stream_u32(io.rec_flags + kofs + e0, trunc_w * GC_FLAG_TRUNCATED | (count_w << GC_FLAG_COUNT_SHIFT));
                 if (io.rec_next_obs) st_stream_v4(io.rec_next_obs + kofs + e0, make_int4(nx[0], nx[1], nx[2], nx[3]));
             }
+            if constexpr (MODE == kCount) {                        // never 'unsafe'; reward term rew * 2^24
+                const unsigned lanes = live_lanes(e0, io.n);
+#pragma unroll
+                for (int e = 0; e < kEPT; ++e)
+                    count_joint(cnt, lanes, e < rem, ob[e] * 25u + act[e], nx[e], static_cast<int32_t>(byte_of(rew_w, e) << 24), 0u);
+            }
         }
         st_stream_u32(io.state + e0, c0[0] | (c0[1] << 8) | (c0[2] << 16) | (c0[3] << 24));
         st_stream_u32(io.state + ld + e0, c1[0] | (c1[1] << 8) | (c1[2] << 16) | (c1[3] << 24));
         st_stream_v4(io.t + e0, make_int4(t[0], t[1], t[2], t[3]));
         st_stream_v4(io.index + e0, make_int4(c0[0] + 20u * c1[0], c0[1] + 20u * c1[1], c0[2] + 20u * c1[2], c0[3] + 20u * c1[3]));
-        if constexpr (!RECORD) {
+        if constexpr (MODE == kRollout) {
             st_stream_v4(io.ret + e0, make_int4(__float_as_int(ret[0]), __float_as_int(ret[1]),
                                                 __float_as_int(ret[2]), __float_as_int(ret[3])));
             st_stream_v4(io.n_unsafe + e0, make_int4(0, 0, 0, 0));                   // never 'unsafe'
@@ -444,23 +566,24 @@ inline int rollout_grid(int64_t n, int threads, int n_sm, int blocks_per_sm_256)
     return static_cast<int>(need < cap ? (need < 1 ? 1 : need) : cap);
 }
 
-template <int C, bool RECORD>
-cudaError_t launch_rollout_c(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm, cudaStream_t st)
+template <int C, int MODE>
+cudaError_t launch_rollout_c(const CellTables &tab, const RolloutIO &io, const CountIO &cnt, const uint2 *lut, bool noise,
+                             int n_sm, cudaStream_t st)
 {
     const int threads = rollout_threads(io.n, n_sm), grid = rollout_grid(io.n, threads, n_sm, 2);
     if (noise)
-        cell_rollout_kernel<C, true, RECORD><<<grid, threads, 0, st>>>(tab, io, lut);
+        cell_rollout_kernel<C, true, MODE><<<grid, threads, 0, st>>>(tab, io, lut, cnt);
     else
-        cell_rollout_kernel<C, false, RECORD><<<grid, threads, 0, st>>>(tab, io, lut);
+        cell_rollout_kernel<C, false, MODE><<<grid, threads, 0, st>>>(tab, io, lut, cnt);
     return cudaGetLastError();
 }
 
-template <bool RECORD>
-cudaError_t launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
-                                cudaStream_t st)
+template <int MODE>
+cudaError_t launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const CountIO &cnt, const uint2 *lut, bool noise,
+                                int n_sm, cudaStream_t st)
 {
     switch (tab.n_cells) {
-#define GC_CASE(C) case C: return launch_rollout_c<C, RECORD>(tab, io, lut, noise, n_sm, st);
+#define GC_CASE(C) case C: return launch_rollout_c<C, MODE>(tab, io, cnt, lut, noise, n_sm, st);
         GC_CASE(1) GC_CASE(2) GC_CASE(3) GC_CASE(4) GC_CASE(5) GC_CASE(6) GC_CASE(7) GC_CASE(8)
         GC_CASE(9) GC_CASE(10) GC_CASE(11) GC_CASE(12) GC_CASE(13) GC_CASE(14) GC_CASE(15) GC_CASE(16)
 #undef GC_CASE
@@ -468,12 +591,12 @@ cudaError_t launch_cell_rollout(const CellTables &tab, const RolloutIO &io, cons
     }
 }
 
-template <bool RECORD>
-cudaError_t launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
+template <int MODE>
+cudaError_t launch_grid_rollout(const GridParams &gp, const RolloutIO &io, const CountIO &cnt, int n_sm, cudaStream_t st)
 {
     // the 40 KB table is staged per block: keep 256-thread blocks unless the batch is really small
     const int threads = (io.n + kEPT - 1) / kEPT < static_cast<int64_t>(n_sm) * kThreads / 2 ? 64 : kThreads;
-    grid_rollout_kernel<RECORD><<<rollout_grid(io.n, threads, n_sm, 4), threads, 0, st>>>(gp, io);
+    grid_rollout_kernel<MODE><<<rollout_grid(io.n, threads, n_sm, MODE == kCount ? 2 : 4), threads, 0, st>>>(gp, io, cnt);
     return cudaGetLastError();
 }
 
@@ -482,21 +605,32 @@ cudaError_t launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n
 cudaError_t gc_launch_cell_rollout(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
                                    cudaStream_t st)
 {
-    return launch_cell_rollout<false>(tab, io, lut, noise, n_sm, st);
+    return launch_cell_rollout<kRollout>(tab, io, CountIO{}, lut, noise, n_sm, st);
 }
 
 cudaError_t gc_launch_cell_collect(const CellTables &tab, const RolloutIO &io, const uint2 *lut, bool noise, int n_sm,
                                    cudaStream_t st)
 {
-    return launch_cell_rollout<true>(tab, io, lut, noise, n_sm, st);
+    return launch_cell_rollout<kRecord>(tab, io, CountIO{}, lut, noise, n_sm, st);
+}
+
+cudaError_t gc_launch_cell_count(const CellTables &tab, const RolloutIO &io, const CountIO &cnt, const uint2 *lut, bool noise,
+                                 int n_sm, cudaStream_t st)
+{
+    return launch_cell_rollout<kCount>(tab, io, cnt, lut, noise, n_sm, st);
 }
 
 cudaError_t gc_launch_grid_rollout(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
 {
-    return launch_grid_rollout<false>(gp, io, n_sm, st);
+    return launch_grid_rollout<kRollout>(gp, io, CountIO{}, n_sm, st);
 }
 
 cudaError_t gc_launch_grid_collect(const GridParams &gp, const RolloutIO &io, int n_sm, cudaStream_t st)
 {
-    return launch_grid_rollout<true>(gp, io, n_sm, st);
+    return launch_grid_rollout<kRecord>(gp, io, CountIO{}, n_sm, st);
+}
+
+cudaError_t gc_launch_grid_count(const GridParams &gp, const RolloutIO &io, const CountIO &cnt, int n_sm, cudaStream_t st)
+{
+    return launch_grid_rollout<kCount>(gp, io, cnt, n_sm, st);
 }

@@ -306,6 +306,18 @@ class PackedCellularVectorEnv(CellularVectorEnv):
             self._index.copy_(self._ro_index)
         return tr
 
+    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None):
+        """Experience counts (see `CellularVectorEnv.collect_counts`): the counting kernel takes the int8 layout, so the
+        packed state is unpacked for it and packed again afterwards, as in `collect()`."""
+        if getattr(self, "_ro_index", None) is None:
+            self._ro_index = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
+        cells = self.unpack(self._state).contiguous()            # int8 [n_cells, ld]
+        counts = self._collect_counts(n_steps, policy, epsilon, counts, cells, self._ro_index)
+        self._state.copy_(self.pack(cells))
+        if self._index is not self._state:
+            self._index.copy_(self._ro_index)
+        return counts
+
     # ---- views ---------------------------------------------------------------------------------------
     def _lazy_truncated(self):
         return (self._flags[:self.num_envs] & _lib.FLAG_TRUNCATED).ne(0)

@@ -54,6 +54,22 @@ class Transitions(namedtuple("Transitions", "obs action reward flags next_obs"))
         return self.flags >> _lib.FLAG_COUNT_SHIFT
 
 
+class Counts(namedtuple("Counts", "visits next reward_q24 unsafe cell_next")):
+    """Experience counts of `collect_counts`: int64 device tensors the kernel adds to (None = not counted).
+    s / a / s' are the tabular `obs`, executed `action` and `next_obs` of `collect` (nS = n_states ** n_cells,
+    nA = n_actions ** n_cells; grid world 400 and 25).
+      visits      [nS, nA]        N(s, a)
+      next        [nS, nA, nS]    N(s, a, s'), s' = successor before the time-limit auto-reset
+      reward_q24  [nS, nA]        sum of round(reward * 2**24), the term stats()['reward_sum'] is kept in
+      unsafe      [nS, nA]        steps that reported 'unsafe'
+      cell_next   [C, S, A, S]    per cell c: N_c(s_c, a_c, s'_c) (cellular family only)
+    P_hat(s' | s, a) = next / visits and R_hat(s, a) = reward_q24 * 2**-24 / visits."""
+    __slots__ = ()
+
+
+_JOINT_LIMIT = 2 ** 31              # entries of one joint count table (32-bit indices in the kernels)
+
+
 def _round_up(n, m):
     return (n + m - 1) // m * m
 
@@ -605,6 +621,57 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         n = self.num_envs
         return Transitions(buf["obs"][:, :n], buf["action"][:, :n], buf["reward"][:, :n], buf["flags"][:, :n],
                            None if nx is None else nx[:, :n])
+
+    def _joint_sizes(self):
+        if self.kind == "gridworld":
+            return 400, 25
+        return self.n_states ** self.n_cells, self.n_actions ** self.n_cells
+
+    def zero_counts(self, joint=True, transitions=True):
+        """Zeroed `Counts` tables for `collect_counts`.  joint=False leaves the four joint tables None (for envs too
+        large for them, such as 16 cells x 4 levels, only the per-cell `cell_next` is kept); transitions=False leaves
+        `next` None.  `cell_next` is None for grid world."""
+        nS, nA = self._joint_sizes()
+        if joint and (nS * nA > _JOINT_LIMIT or (transitions and nS * nA * nS > _JOINT_LIMIT)):
+            raise ValueError(f"the joint count tables of {nS} states x {nA} actions exceed 2**31 entries: use joint=False"
+                             + ("" if nS * nA > _JOINT_LIMIT else " or transitions=False"))
+        z = lambda *shape: torch.zeros(*shape, dtype=torch.int64, device=self.device)      # noqa: E731
+        S, A, Cn = self.n_states, self.n_actions, self.n_cells
+        return Counts(z(nS, nA) if joint else None, z(nS, nA, nS) if joint and transitions else None,
+                      z(nS, nA) if joint else None, z(nS, nA) if joint else None,
+                      z(Cn, S, A, S) if self.kind == "cellular" else None)
+
+    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None):
+        """Experience counts: `n_steps` steps per env inside one kernel, as `collect()` (same policies, same epsilon
+        rule, same draws), adding every transition to `counts` instead of recording it.  counts=None allocates
+        `zero_counts()`.  Returns `counts`; the counts equal the histogram of the record `collect()` would return, and
+        state, time_step, tabular_state() and stats() advance exactly as `collect()` advances them.  The counts are
+        integers, so they are exact, independent of the order of the adds and of how the envs are sharded."""
+        return self._collect_counts(n_steps, policy, epsilon, counts, self._state, self._index)
+
+    def _collect_counts(self, n_steps, policy, epsilon, counts, state, index):
+        kind, ptab = self._policy_table(policy)
+        if counts is None:
+            counts = self.zero_counts()
+        nS, nA = self._joint_sizes()
+        shapes = Counts((nS, nA), (nS, nA, nS), (nS, nA), (nS, nA),
+                        (self.n_cells, self.n_states, self.n_actions, self.n_states) if self.kind == "cellular" else None)
+        if not isinstance(counts, Counts) or all(t is None for t in counts):
+            raise ValueError("counts must be a Counts with at least one table (see zero_counts())")
+        for name, t, shape in zip(Counts._fields, counts, shapes):
+            if t is None:
+                continue
+            if shape is None:
+                raise ValueError(f"counts.{name} must be None for {self.kind}")
+            # the kernel adds at flat indices of these shapes: a smaller table would be written past its end
+            if tuple(t.shape) != shape:
+                raise ValueError(f"counts.{name} has shape {tuple(t.shape)}; this env's is {shape} (see zero_counts())")
+            if t.dtype != torch.int64 or t.device != self.device or not t.is_contiguous():
+                raise ValueError("count tables must be contiguous int64 tensors on the env's device")
+        cs = _lib.GcCounts(C.sizeof(_lib.GcCounts), *(None if t is None else t.data_ptr() for t in counts))
+        _lib.check(self._lib.gc_collect_counts(self._h, int(n_steps), kind, _ptr(ptab), float(epsilon), _ptr(state),
+                                               _ptr(self._t), _ptr(index), C.byref(cs), _ptr(self._stats), self._stream()))
+        return counts
 
     def capture_steps(self, action_ring):
         """Captures one step per tensor of `action_ring` (int8 [n_cells, ld] device tensors, kept alive

@@ -313,6 +313,27 @@ typedef struct {
 int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
                int8_t *state, int32_t *t, uint32_t *index, const gc_record *record, int64_t *stats, void *stream);
 
+/* Experience counts of gc_collect_counts: int64 device arrays owned by the caller, 8-byte aligned, each NULL = not
+ * counted (but not all of them).  s is the tabular index gc_collect records as `obs`, a the executed tabular action it
+ * records as `action`, s' its `next_obs`; nS = n_states^n_cells, nA = n_actions^n_cells (grid world: 400 and 25).  A
+ * joint table may have at most 2^31 entries; cell_next is cellular only (C = n_cells, S = n_states, A = n_actions). */
+typedef struct {
+    uint32_t struct_size;
+    int64_t *visits;      /* [nS][nA]       N(s, a)                                                      */
+    int64_t *next;        /* [nS][nA][nS]   N(s, a, s'), s' = successor BEFORE the time-limit auto-reset   */
+    int64_t *reward_q24;  /* [nS][nA]       sum of round(reward * 2^24), the term GC_STAT_REWARD_Q24 adds  */
+    int64_t *unsafe;      /* [nS][nA]       steps that reported 'unsafe'                                  */
+    int64_t *cell_next;   /* [C][S][A][S]   per cell c: N_c(s_c, a_c, s'_c); cellular only               */
+} gc_counts;
+
+/* Experience counts: gc_collect with the same arguments (same envs, policies, epsilon rule, Philox streams, and the
+ * same advance of state, t, index, global step, statistics and launch count) that ADDS every transition to `counts`
+ * instead of recording it, so that the counts equal the histogram of gc_collect's record.  Integer counts: exact,
+ * independent of the order of the adds and of the sharding of the envs.  Arguments are validated before any CUDA
+ * call.  One kernel launch. */
+int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+                      int8_t *state, int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream);
+
 /* Reads and clears the handle's device status word (synchronises `stream`).  Returns GC_OK or
  * GC_ERR_ACTION if some env received a grid-world action without any go-to position since the
  * last poll (the reference raises KeyError('position'), grid_world.py:143). */
