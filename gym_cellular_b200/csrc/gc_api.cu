@@ -530,6 +530,9 @@ int gc_set_global_step(gc_env *env, int64_t step)
     const uint32_t v = static_cast<uint32_t>(step);
     GC_ON_DEVICE(env->cfg.device);
     GC_CUDA(cudaMemcpy(env->d_step, &v, sizeof(v), cudaMemcpyHostToDevice));   // synchronous: rare, control path
+    // a copy from pageable memory may return before its DMA has landed: wait for it, so that a kernel queued next on
+    // a non-blocking stream reads the new value
+    GC_CUDA(cudaStreamSynchronize(cudaStreamLegacy));
     return GC_OK;
 }
 
@@ -620,6 +623,10 @@ int launch_bound(gc_env *env, int32_t slot, cudaStream_t st)
 {
     if (slot < 0 || slot >= GC_MAX_BINDINGS || !env->bound_set[slot])
         return fail(GC_ERR_INVALID, "no binding in slot %d", slot);
+    // a packed binding outlives the tables it was checked against: the packed LUT is rebuilt only for tables that
+    // admit the layout, so the slot is refused while the current ones do not
+    if (env->bound_set[slot] == 2)
+        if (int rc = check_packed(env)) return rc;
     if (int rc = env->bound_set[slot] == 2 ? launch_packed(env, env->bound_packed[slot], st)
                                            : launch_step(env, env->bound[slot], st))
         return rc;
@@ -761,9 +768,12 @@ int gc_prepare_step_many(gc_env *env, const int32_t *slots, int32_t n_slots)
 {
     if (!env || !slots || n_slots < 1) return fail(GC_ERR_INVALID, "gc_prepare_step_many: bad arguments");
     if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
-    for (int32_t i = 0; i < n_slots; ++i)
+    for (int32_t i = 0; i < n_slots; ++i) {
         if (slots[i] < 0 || slots[i] >= GC_MAX_BINDINGS || !env->bound_set[slots[i]])
             return fail(GC_ERR_INVALID, "no binding in slot %d", slots[i]);
+        if (env->bound_set[slots[i]] == 2)
+            if (int rc = check_packed(env)) return rc;
+    }
     GC_ON_DEVICE(env->cfg.device);
     if (n_slots <= GC_MAX_BINDINGS && many_fusable(env, slots, n_slots)) return GC_OK;     // one launch for all steps: no graph needed
     if (many_graphs_enabled(env) && n_slots >= 2) many_graph(env, slots, n_slots);   // best effort: plain launches otherwise
@@ -778,9 +788,13 @@ int gc_step_many(gc_env *env, const int32_t *slots, int32_t n_slots, int32_t n_s
     GC_ON_DEVICE(env->cfg.device);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     int32_t done = 0;
-    for (int32_t i = 0; i < n_slots; ++i)
+    // every slot is checked before the first step runs: a list the handle cannot step in full is refused whole
+    for (int32_t i = 0; i < n_slots; ++i) {
         if (slots[i] < 0 || slots[i] >= GC_MAX_BINDINGS || !env->bound_set[slots[i]])
             return fail(GC_ERR_INVALID, "no binding in slot %d", slots[i]);
+        if (env->bound_set[slots[i]] == 2)
+            if (int rc = check_packed(env)) return rc;
+    }
     // Small shards with one set of in-place buffers: all steps in one launch (many_fusable)
     if (n_steps >= 2 && n_slots <= GC_MAX_BINDINGS && many_fusable(env, slots, n_slots)) {
         for (; done < n_steps;) {

@@ -155,6 +155,7 @@ class PackedCellularVectorEnv(CellularVectorEnv):
         self._t.copy_(sd["t"])
         if self._stats is not None and sd["stats"] is not None:
             self._stats.copy_(sd["stats"])
+        torch.cuda.current_stream(self.device).synchronize()       # see CellularVectorEnv.load_state_dict
         _lib.check(self._lib.gc_set_global_step(self._h, int(sd["global_step"])))
         self._refresh_index()
 

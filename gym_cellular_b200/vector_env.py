@@ -399,6 +399,9 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         self._t.copy_(sd["t"])
         if self._stats is not None and sd["stats"] is not None:
             self._stats.copy_(sd["stats"])
+        # gc_set_global_step is ordered only after blocking streams: a step still queued on a non-blocking current
+        # stream would read the restored counter and then overwrite it with its own successor
+        torch.cuda.current_stream(self.device).synchronize()
         _lib.check(self._lib.gc_set_global_step(self._h, int(sd["global_step"])))
         # refresh the tabular index of the restored state
         self._encode_state(self._state, self._index, self.num_envs, self.ld)

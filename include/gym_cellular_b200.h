@@ -143,8 +143,11 @@ int gc_create(const gc_config *cfg, gc_env **out);
 int gc_destroy(gc_env *env);
 /* Cellular family only.  Validates everything first: a rejected call leaves the previous tables in force.  The
  * staged device tables are replaced with synchronous copies, so steps still in flight on a NON-BLOCKING stream must
- * be waited for by the caller before the tables are changed; bindings stay valid, cached gc_step_many graphs are
- * rebuilt on their next use. */
+ * be waited for by the caller before the tables are changed; cached gc_step_many graphs are rebuilt on their next
+ * use.  Int8 bindings stay valid and step by the new tables.  Packed bindings stay in their slots but step only
+ * while the tables admit the packed layout (as gc_bind_step_packed requires): under other tables gc_step_bound and
+ * gc_step_many / gc_prepare_step_many on a list holding one are refused with GC_ERR_INVALID before any step runs,
+ * and they step again once such tables are set. */
 int gc_set_tables(gc_env *env, const gc_cell_tables *tables);
 
 /* Final observation (gymnasium's SAME_STEP auto-reset convention; the reference never ends an episode,
@@ -157,7 +160,10 @@ int gc_set_final_obs(gc_env *env, int8_t *final_state);
 /* Global step counter used as the RNG counter when GC_F_RNG_EPISODIC is off.  It lives in device
  * memory: a gc_step over the whole shard reads it in the kernel and the kernel advances it, so a
  * gc_step captured into a CUDA graph keeps drawing fresh numbers on every replay.  The host keeps a
- * mirror (gc_get_global_step); after graph replays call gc_sync_global_step to refresh it. */
+ * mirror (gc_get_global_step); after graph replays call gc_sync_global_step to refresh it.
+ * gc_set_global_step is synchronous: it returns once the device word holds the new value, and it is ordered only
+ * after work on blocking streams.  A kernel still queued or running on a NON-BLOCKING stream reads the counter when
+ * it runs and writes it back when it ends, so the caller must wait for that stream first. */
 int gc_set_global_step(gc_env *env, int64_t step);
 int64_t gc_get_global_step(const gc_env *env);
 int gc_sync_global_step(gc_env *env, void *stream);
@@ -260,6 +266,8 @@ int gc_reset_packed(gc_env *env, const uint8_t *mask, uint32_t *state, int32_t *
 int gc_step_packed(gc_env *env, int64_t env_begin, int64_t env_count, const uint32_t *actions, uint32_t *state,
                    int32_t *t, float *reward, uint32_t *index, uint8_t *flags, uint32_t *final_state,
                    uint32_t *se_row, int64_t *stats, void *stream);
+/* Packed binding (gc_bind_step's slots): refused unless the current tables admit the packed layout; a bound slot is
+ * stepped only while they still do (gc_set_tables). */
 int gc_bind_step_packed(gc_env *env, int32_t slot, const uint32_t *actions, uint32_t *state, int32_t *t,
                         float *reward, uint32_t *index, uint8_t *flags, uint32_t *final_state, uint32_t *se_row,
                         int64_t *stats);
