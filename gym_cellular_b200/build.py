@@ -14,7 +14,7 @@ REPO = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.environ.get("GC_B200_LIB_DIR") or os.path.join(PKG, "lib")     # override: A/B builds of tuning runs
 LIB_PATH = os.path.join(LIB_DIR, "libgymcellular_b200.so")
-SOURCES = ["gc_kernels.cu", "gc_cell_fast.cu", "gc_cell_pair8.cu", "gc_cell_packed.cu", "gc_cell_tma.cu", "gc_grid.cu", "gc_rollout.cu", "gc_tables.cu", "gc_api.cu"]
+SOURCES = ["gc_kernels.cu", "gc_cell_fast.cu", "gc_cell_pair8.cu", "gc_cell_packed.cu", "gc_grid.cu", "gc_rollout.cu", "gc_tables.cu", "gc_api.cu"]
 HEADERS = [os.path.join(CSRC, "gc_internal.h"), os.path.join(CSRC, "gc_device.cuh"), os.path.join(REPO, "include", "gym_cellular_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I" + os.path.join(REPO, "include"), "-I" + CSRC]
@@ -44,7 +44,7 @@ def build(force=False, verbose=False):
         obj = os.path.join(LIB_DIR, src.replace(".cu", ".o"))
         objs.append(obj)
         if force or _stale(obj, [path] + HEADERS):
-            extra = os.environ.get("GC_NVCC_EXTRA", "").split()       # e.g. -DGC_PAIR_MINB_WIDE=1 (tuning runs)
+            extra = os.environ.get("GC_NVCC_EXTRA", "").split()       # e.g. -DGC_PACKED_MINB=3 (tuning runs)
             cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", path, "-o", obj]
             procs.append((cmd, subprocess.Popen(cmd)))
     for cmd, p in procs:

@@ -249,13 +249,7 @@ int launch_step(gc_env *env, const StepIO &io, cudaStream_t st)
         // noise with probability 0 never fires: the deterministic kernels then do the same job
         const bool draws = (env->cfg.flags & GC_F_NOISE) && env->tab.noise_thr_nz;
         const int mode = io.replay ? GC_RNG_REPLAY : (draws ? GC_RNG_PHILOX : GC_RNG_NONE);
-        // Experimental: wide deterministic envs staged tile by tile with TMA bulk copies (gc_cell_tma.cu).
-        // Measured slower than the register-staged kernel (profiles/r01_tuning_log.md), so it is opt-in:
-        // GC_B200_TMA=1 in the environment.
-        static const bool use_tma = [] { const char *v = std::getenv("GC_B200_TMA"); return v && v[0] == '1'; }();
-        if (env->fast_ok && use_tma && mode == GC_RNG_NONE && !io.se_row && !io.final_state && env->cfg.n_cells >= 8)
-            e = gc_launch_cell_tma_step(env->tab, io, env->d_pair_lut, env->n_sm, st);
-        else if (env->fast_ok)
+        if (env->fast_ok)
             e = gc_launch_cell_pair_step(env->tab, io, env->d_pair_lut, mode, env->n_sm, st);
         else if (env->pair8_ok && mode != GC_RNG_REPLAY)
             e = gc_launch_cell_pair8_step(env->tab, io, env->d_pair8_lut, mode, env->n_sm, st);

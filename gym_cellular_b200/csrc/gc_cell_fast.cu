@@ -21,41 +21,23 @@
 
 namespace {
 
-
-// resident blocks per SM the register budget is sized for: all 2C row words of a thread's 4 envs are
-// requested up front (memory-level parallelism), so wide envs trade occupancy for loads in flight
-#ifndef GC_PAIR_MINB
-#define GC_PAIR_MINB 4
-#endif
-// resident blocks per SM the register budget is sized for; the Philox variants of wide envs carry
-// 16 more registers (one random block per env) and get the budget of three blocks
-#ifndef GC_PAIR_MINB_NARROW
-#define GC_PAIR_MINB_NARROW GC_PAIR_MINB
-#endif
+// Resident blocks per SM the register budget is sized for: all 2C row words of a thread's 4 envs are
+// requested up front (memory-level parallelism), so wide envs trade occupancy for loads in flight.  The
+// Philox variants of wide envs carry 16 more registers (one random block per env) and get the budget of
+// three blocks.  (Five blocks of the narrow kernels, at 48 registers, measured 0.732 against 0.775 of the
+// roofline: profiles/r01_tuning_log.md.)
 constexpr int pair_min_blocks(int c, int rng)
 {
-#ifdef GC_PAIR_MINB_ALL
-    return GC_PAIR_MINB_ALL;
-#endif
     if (rng != GC_RNG_NONE && c > 4) return 3;
-    if (rng == GC_RNG_NONE && ((c >= 4 && c <= 8) || c == 10 || c == 11)) return GC_PAIR_MINB < 3 ? GC_PAIR_MINB : 3;
-    return c < 4 ? GC_PAIR_MINB_NARROW : GC_PAIR_MINB;
+    if (rng == GC_RNG_NONE && ((c >= 4 && c <= 8) || c == 10 || c == 11)) return 3;
+    return 4;
 }
 
-// Table replication (A/B switch, round 2): with GC_PAIR_REP_LOG2 = 4 the deterministic kernels of wide envs keep
-// 16 copies of the 256-entry pair table (entry i of replica r at word 16 i + r, lane l reads replica l % 16), so
-// that the 16 lanes of a half-warp never meet on a bank pair: profiles/r01_kernel_cfg4.md counted 70 % of the
-// shared-memory wavefronts of config 4 as conflicts.  See profiles/r02_tuning_log.md for the measurement.
-#ifndef GC_PAIR_REP_LOG2
-#define GC_PAIR_REP_LOG2 0
-#endif
-#ifndef GC_PAIR_REP_MIN_C
-#define GC_PAIR_REP_MIN_C 12
-#endif
-__host__ __device__ constexpr int pair_rep_log2(int c, int rng)
-{
-    return (rng == GC_RNG_NONE && c >= GC_PAIR_REP_MIN_C) ? GC_PAIR_REP_LOG2 : 0;
-}
+// The pair table is staged once per block, not replicated per lane.  Sixteen replicas (lane l reading replica
+// l % 16) would keep the lanes of a half-warp off each other's bank pairs -- profiles/r01_kernel_cfg4.md counted
+// 70 % of the shared-memory wavefronts of config 4 as conflicts -- but these kernels wait for HBM, and the
+// replicated table measured slower: 190.9 us per step plain, 191.5 with 8 replicas, 193.7-195.3 with 16
+// (profiles/r02_tuning_log.md).
 
 // Everything a thread carries across the cell groups of its four envs.  The low halves of the info
 // words (count byte, presence / flag byte) are accumulated two envs per register (16-bit lanes: envs
@@ -67,6 +49,13 @@ struct EnvAcc {
     uint32_t or01, or23;    // bit 12 of a lane: pair (cell 0, cell 1) is 'unsafe'; bits 8-11: levels present in cells j >= 2
     uint32_t idx[kEPT];     // tabular index
     uint32_t s0w, s1w;      // next level of cell 0 / cell 1 (before an auto-reset), byte lane e = env e
+
+    __device__ __forceinline__ void clear()
+    {
+#pragma unroll
+        for (int e = 0; e < kEPT; ++e) { r[e] = 0.f; idx[e] = 0; }
+        sum01 = sum23 = or01 = or23 = s0w = s1w = 0;
+    }
 };
 
 // One group of N <= 4 consecutive cells starting at cell c0 (c0 % 4 == 0) for the 4 envs of a thread.
@@ -120,7 +109,7 @@ __device__ __forceinline__ void do_cells(const CellTables &tab, const StepIO &io
             for (int e = 0; e < kEPT; ++e) {
                 uint32_t ix = byte_of(pidx, e);
                 if (RNG != GC_RNG_NONE) ix |= ((fb[e] >> i) & 3u) << 8;
-                const uint2 ent = s_pair[ix << pair_rep_log2(C, RNG)];     // s_pair points at this lane's replica
+                const uint2 ent = s_pair[ix];
                 if (FIRST && i == 0) acc.r[e] = __uint_as_float(ent.y); else acc.r[e] += __uint_as_float(ent.y);
                 inf[e] = ent.x;
             }
@@ -181,6 +170,74 @@ __device__ __forceinline__ void load_cells(const StepIO &io, int c0, uint32_t e0
     }
 }
 
+// What the step kernel and the many-step kernel do per 4-env word around the cell groups (do_cells): the time
+// limit and the wide-env draws before, the flags, statistics and stores after.
+
+// Episode steps after this step (0 where the time limit is reached), the truncated flags (byte lane e = env e)
+// and keep, the byte mask of the envs NOT reset.
+__device__ __forceinline__ void time_limit(const StepIO &io, const int (&tin)[kEPT], int (&tn)[kEPT], uint32_t &trunc_w,
+                                           uint32_t &keep)
+{
+#pragma unroll
+    for (int e = 0; e < kEPT; ++e) tn[e] = tin[e] + 1;
+    trunc_w = 0;
+    keep = 0xFFFFFFFFu;
+    if (io.max_episode_steps > 0) {
+#pragma unroll
+        for (int e = 0; e < kEPT; ++e)
+            if (tn[e] >= io.max_episode_steps) { tn[e] = 0; trunc_w |= 1u << (8 * e); keep &= ~(0xFFu << (8 * e)); }
+    }
+}
+
+// The fire bits of every cell of a wide env with Philox draws; zero otherwise (narrow envs draw in do_cells).
+template <int C, int RNG>
+__device__ __forceinline__ void wide_fire_bits(const CellTables &tab, const StepIO &io, uint32_t gid_lo, uint32_t gid_hi,
+                                               uint32_t step_counter, const int (&tin)[kEPT], uint32_t (&fire16)[kEPT])
+{
+#pragma unroll
+    for (int e = 0; e < kEPT; ++e) fire16[e] = 0;
+    if (RNG == GC_RNG_PHILOX && C > GC_NARROW_CELLS) {
+#pragma unroll
+        for (int e = 0; e < kEPT; ++e)
+            fire16[e] = fire_bits_wide<(C + 7) / 8>(tab, gid_lo | e, gid_hi, io.episodic ? static_cast<uint32_t>(tin[e]) : step_counter,
+                                                    io.round_key);
+    }
+}
+
+// Unsafe / count for the four envs at once (byte lanes): the count and the presence / flag bytes of the 16-bit
+// lanes, and the unsafe-levels mask of each env's s'_0 picked out of tab.unsafe_rows with one byte permute
+// (selector nibble e = s'_0 of env e); then the statistics and the per-env outputs other than the state rows.
+__device__ __forceinline__ void finish_word(const CellTables &tab, const StepIO &io, uint32_t e0, int rem, const EnvAcc &acc,
+                                            const int (&tn)[kEPT], uint32_t trunc_w, uint32_t &st_steps, uint32_t &st_unsafe,
+                                            uint32_t &st_count, uint32_t &st_trunc, long long &st_reward)
+{
+    float rout[kEPT];
+    log2_1p_x4(tab.reward_log2, acc.r, rout);
+    const uint32_t count_w = prmt(acc.sum01, acc.sum23, 0x6420) & 0x1F1F1F1Fu;
+    const uint32_t present = prmt(acc.or01, acc.or23, 0x7531);            // bits 0-3 levels present, bit 4 pair-(0,1) flag
+    const uint32_t nib = acc.s0w | (acc.s0w >> 4);                        // byte 0: s0_0 | s0_1 << 4, byte 2: s0_2 | s0_3 << 4
+    const uint32_t rowmask = prmt(tab.unsafe_rows, 0u, prmt(nib, 0u, 0x4420) & 0x3333u);
+    const uint32_t unsafe_w = ((((present & rowmask) + 0x0F0F0F0Fu) | present) >> 4) & 0x01010101u;
+#pragma unroll
+    for (int e = 0; e < kEPT; ++e)
+        if (e < rem) st_reward += __float2int_rn(rout[e] * 16777216.0f);     // |reward| < 128: gc_set_tables
+    {
+        const uint32_t vb = valid_bytes(rem);
+        st_steps += rem;
+        st_unsafe = add_bytes(unsafe_w & vb, st_unsafe);
+        st_count = add_bytes(count_w & vb, st_count);
+        st_trunc = add_bytes(trunc_w & vb, st_trunc);
+    }
+    st_stream_v4(io.t + e0, make_int4(tn[0], tn[1], tn[2], tn[3]));
+    st_stream_v4(io.reward + e0, make_int4(__float_as_int(rout[0]), __float_as_int(rout[1]),
+                                           __float_as_int(rout[2]), __float_as_int(rout[3])));
+    st_stream_v4(io.index + e0, make_int4(acc.idx[0], acc.idx[1], acc.idx[2], acc.idx[3]));
+    st_stream_u32(io.terminated + e0, 0u);
+    st_stream_u32(io.truncated + e0, trunc_w);
+    st_stream_u32(io.unsafe + e0, unsafe_w);
+    st_stream_u32(io.count + e0, count_w);
+}
+
 // The cells of an env are walked in groups of four (two table lookups per env and group) by a
 // software-pipelined loop: the rows of group g+1 are requested before group g is computed, so a
 // thread keeps 8-16 row words in flight with ~60 registers and four blocks stay resident per SM.
@@ -192,23 +249,18 @@ cell_pair_kernel(const __grid_constant__ CellTables tab, const __grid_constant__
     constexpr int NG = C / 4, R = C % 4;                        // full groups, cells in the tail group
     constexpr int N_PAIR = (RNG == GC_RNG_NONE) ? 256 : GC_PAIR_LUT_PAIRS;
     constexpr int N_SINGLE = (RNG == GC_RNG_NONE) ? 16 : 32;
-    constexpr int REP_LOG2 = pair_rep_log2(C, RNG), REP = 1 << REP_LOG2;
-    __shared__ uint2 s_pair_all[N_PAIR * REP];
-    const uint2 *const s_pair = s_pair_all + (threadIdx.x & (REP - 1));
+    __shared__ uint2 s_pair[N_PAIR];
     __shared__ uint2 s_single[N_SINGLE];
     __shared__ uint8_t s_se[WITH_SE ? C : 1][GC_TBL];
     __shared__ unsigned long long s_stats[5];
-
     __shared__ StepCounterShared s_ctr;
 
     const uint32_t stride = gridDim.x * kThreads * kEPT, e_end = static_cast<uint32_t>(io.end);
     // Narrow envs (C < 4: a thread reads only ~10 words per 4 envs) prefetch the inputs of their next
     // 4-env word before computing the current one, to keep enough bytes in flight per SM; the first
-    // word's inputs are requested before the tables are staged, so that the two latencies overlap.
-#ifndef GC_PAIR_PREFETCH_WIDE
-#define GC_PAIR_PREFETCH_WIDE 0
-#endif
-    constexpr bool PREFETCH = NG == 0 || GC_PAIR_PREFETCH_WIDE;
+    // word's inputs are requested before the tables are staged, so that the two latencies overlap.  Wide
+    // envs do not: their prefetched rows spill or cost a resident block (profiles/r01_tuning_log.md).
+    constexpr bool PREFETCH = NG == 0;
     constexpr int G0 = NG > 0 ? 4 : R;                       // cells in the first group
     uint32_t e0 = static_cast<uint32_t>(io.begin) + (blockIdx.x * kThreads + threadIdx.x) * kEPT;
     // the immutable tables are requested first (they may be read while the previous step kernel of the
@@ -228,9 +280,7 @@ cell_pair_kernel(const __grid_constant__ CellTables tab, const __grid_constant__
     }
     step_counter_read(io, &s_ctr);
 #pragma unroll
-    for (int k = 0; k < LUT_PER_THREAD; ++k)
-#pragma unroll
-        for (int r = 0; r < REP; ++r) s_pair_all[((threadIdx.x + k * kThreads) << REP_LOG2) + r] = lut_pair[k];
+    for (int k = 0; k < LUT_PER_THREAD; ++k) s_pair[threadIdx.x + k * kThreads] = lut_pair[k];
     if (threadIdx.x < N_SINGLE) s_single[threadIdx.x] = lut_single;
     if (WITH_SE)
         for (int i = threadIdx.x; i < C * GC_TBL; i += kThreads) s_se[i / GC_TBL][i % GC_TBL] = tab.se[i / GC_TBL][i % GC_TBL];
@@ -265,24 +315,12 @@ cell_pair_kernel(const __grid_constant__ CellTables tab, const __grid_constant__
         }
 
         const int tin[kEPT] = {t4.x, t4.y, t4.z, t4.w};
-        int tn[kEPT] = {t4.x + 1, t4.y + 1, t4.z + 1, t4.w + 1};
-        uint32_t trunc_w = 0, keep = 0xFFFFFFFFu;                 // keep: byte mask of envs NOT reset
-        if (io.max_episode_steps > 0) {
-#pragma unroll
-            for (int e = 0; e < kEPT; ++e)
-                if (tn[e] >= io.max_episode_steps) { tn[e] = 0; trunc_w |= 1u << (8 * e); keep &= ~(0xFFu << (8 * e)); }
-        }
-        uint32_t fire16[kEPT] = {0, 0, 0, 0};
-        if (RNG == GC_RNG_PHILOX && C > GC_NARROW_CELLS) {
-#pragma unroll
-            for (int e = 0; e < kEPT; ++e)
-                fire16[e] = fire_bits_wide<(C + 7) / 8>(tab, gid_lo | e, gid_hi, io.episodic ? static_cast<uint32_t>(tin[e]) : step_counter,
-                                                        io.round_key);
-        }
+        int tn[kEPT];
+        uint32_t trunc_w, keep, fire16[kEPT];
+        time_limit(io, tin, tn, trunc_w, keep);
+        wide_fire_bits<C, RNG>(tab, io, gid_lo, gid_hi, step_counter, tin, fire16);
         EnvAcc acc;
-#pragma unroll
-        for (int e = 0; e < kEPT; ++e) { acc.r[e] = 0.f; acc.idx[e] = 0; }
-        acc.sum01 = acc.sum23 = acc.or01 = acc.or23 = acc.s0w = acc.s1w = 0;
+        acc.clear();
         uint32_t nx[4];                   // next rows of a group: not needed here (every step reloads its state)
 
         if (NG == 0) {
@@ -301,34 +339,7 @@ cell_pair_kernel(const __grid_constant__ CellTables tab, const __grid_constant__
                 do_cells<R, C, RNG, WITH_SE, false>(tab, io, s_pair, s_single, s_se, 4 * NG, e0, rem, gid_lo, gid_hi, step_counter, tin, keep, sb, ab, fire16, acc, nx);
         }
 
-        // unsafe / count for the four envs at once (byte lanes): the count and the presence / flag bytes
-        // of the 16-bit lanes, and the unsafe-levels mask of each env's s'_0 picked out of
-        // tab.unsafe_rows with one byte permute (selector nibble e = s'_0 of env e)
-        float rout[kEPT];
-        log2_1p_x4(tab.reward_log2, acc.r, rout);
-        const uint32_t count_w = prmt(acc.sum01, acc.sum23, 0x6420) & 0x1F1F1F1Fu;
-        const uint32_t present = prmt(acc.or01, acc.or23, 0x7531);            // bits 0-3 levels present, bit 4 pair-(0,1) flag
-        const uint32_t nib = acc.s0w | (acc.s0w >> 4);                        // byte 0: s0_0 | s0_1 << 4, byte 2: s0_2 | s0_3 << 4
-        const uint32_t rowmask = prmt(tab.unsafe_rows, 0u, prmt(nib, 0u, 0x4420) & 0x3333u);
-        const uint32_t unsafe_w = ((((present & rowmask) + 0x0F0F0F0Fu) | present) >> 4) & 0x01010101u;
-#pragma unroll
-        for (int e = 0; e < kEPT; ++e)
-            if (e < rem) st_reward += __float2int_rn(rout[e] * 16777216.0f);     // |reward| < 128: gc_set_tables
-        {
-            const uint32_t vb = valid_bytes(rem);
-            st_steps += rem;
-            st_unsafe = add_bytes(unsafe_w & vb, st_unsafe);
-            st_count = add_bytes(count_w & vb, st_count);
-            st_trunc = add_bytes(trunc_w & vb, st_trunc);
-        }
-        st_stream_v4(io.t + e0, make_int4(tn[0], tn[1], tn[2], tn[3]));
-        st_stream_v4(io.reward + e0, make_int4(__float_as_int(rout[0]), __float_as_int(rout[1]),
-                                               __float_as_int(rout[2]), __float_as_int(rout[3])));
-        st_stream_v4(io.index + e0, make_int4(acc.idx[0], acc.idx[1], acc.idx[2], acc.idx[3]));
-        st_stream_u32(io.terminated + e0, 0u);
-        st_stream_u32(io.truncated + e0, trunc_w);
-        st_stream_u32(io.unsafe + e0, unsafe_w);
-        st_stream_u32(io.count + e0, count_w);
+        finish_word(tab, io, e0, rem, acc, tn, trunc_w, st_steps, st_unsafe, st_count, st_trunc, st_reward);
     }
     if (io.stats) {
         const ThreadStats ts = {st_steps, st_unsafe, st_count, st_trunc, st_reward};
@@ -354,11 +365,9 @@ cudaError_t launch_pair_cr(const CellTables &tab, const StepIO &io, const uint2 
 // (BASELINE config 2), so the steps are run back to back by the thread that owns the envs: state and episode step
 // stay in registers between two steps, the actions of step k + 1 are requested before step k is computed, and
 // EVERY per-step output (state, t, reward, index, flags, side-effect row, statistics) is written at every step
-// exactly as the n_steps separate launches write it -- same do_cells, same epilogue, same Philox counters
-// (global step of the launch + k) -- so the results are bit-identical to them (tests/test_gpu_many.py).
-#ifndef GC_MANY_SMALL_THREADS
-#define GC_MANY_SMALL_THREADS 64
-#endif
+// exactly as the n_steps separate launches write it -- same time_limit, wide_fire_bits, do_cells and finish_word as
+// cell_pair_kernel, same Philox counters (global step of the launch + k) -- so the results are bit-identical to them
+// (tests/test_gpu_many.py).
 template <int C, int RNG, bool WITH_SE, int THREADS>
 __global__ void __launch_bounds__(THREADS, 256 / THREADS * 2)
 cell_pair_many_kernel(const __grid_constant__ CellTables tab, const __grid_constant__ ManyIO mio, const uint2 *__restrict__ lut)
@@ -414,25 +423,13 @@ cell_pair_many_kernel(const __grid_constant__ CellTables tab, const __grid_const
                 for (int c = 0; c < C; ++c) an[c / 4][c % 4] = ld_stream_u32(nxt + (c * ld + e0));
             }
             const int tin[kEPT] = {t[0], t[1], t[2], t[3]};
-            int tn[kEPT] = {t[0] + 1, t[1] + 1, t[2] + 1, t[3] + 1};
-            uint32_t trunc_w = 0, keep = 0xFFFFFFFFu;
-            if (io.max_episode_steps > 0) {
-#pragma unroll
-                for (int e = 0; e < kEPT; ++e)
-                    if (tn[e] >= io.max_episode_steps) { tn[e] = 0; trunc_w |= 1u << (8 * e); keep &= ~(0xFFu << (8 * e)); }
-            }
+            int tn[kEPT];
+            uint32_t trunc_w, keep, fire16[kEPT];
+            time_limit(io, tin, tn, trunc_w, keep);
             const uint32_t step_counter = (RNG == GC_RNG_PHILOX) ? step0 + static_cast<uint32_t>(k) : 0u;
-            uint32_t fire16[kEPT] = {0, 0, 0, 0};
-            if (RNG == GC_RNG_PHILOX && C > GC_NARROW_CELLS) {
-#pragma unroll
-                for (int e = 0; e < kEPT; ++e)
-                    fire16[e] = fire_bits_wide<(C + 7) / 8>(tab, gid_lo | e, gid_hi, io.episodic ? static_cast<uint32_t>(tin[e]) : step_counter,
-                                                            io.round_key);
-            }
+            wide_fire_bits<C, RNG>(tab, io, gid_lo, gid_hi, step_counter, tin, fire16);
             EnvAcc acc;
-#pragma unroll
-            for (int e = 0; e < kEPT; ++e) { acc.r[e] = 0.f; acc.idx[e] = 0; }
-            acc.sum01 = acc.sum23 = acc.or01 = acc.or23 = acc.s0w = acc.s1w = 0;
+            acc.clear();
             uint32_t nx[G][4];
             if constexpr (NG == 0) {
                 do_cells<R, C, RNG, WITH_SE, true>(tab, io, s_pair, s_single, s_se, 0, e0, rem, gid_lo, gid_hi, step_counter, tin, keep, sw[0], aa[0], fire16, acc, nx[0]);
@@ -444,32 +441,7 @@ cell_pair_many_kernel(const __grid_constant__ CellTables tab, const __grid_const
                 if constexpr (R > 0)
                     do_cells<R, C, RNG, WITH_SE, false>(tab, io, s_pair, s_single, s_se, 4 * NG, e0, rem, gid_lo, gid_hi, step_counter, tin, keep, sw[NG], aa[NG], fire16, acc, nx[NG]);
             }
-            // (the epilogue of cell_pair_kernel, word for word)
-            float rout[kEPT];
-            log2_1p_x4(tab.reward_log2, acc.r, rout);
-            const uint32_t count_w = prmt(acc.sum01, acc.sum23, 0x6420) & 0x1F1F1F1Fu;
-            const uint32_t present = prmt(acc.or01, acc.or23, 0x7531);
-            const uint32_t nib = acc.s0w | (acc.s0w >> 4);
-            const uint32_t rowmask = prmt(tab.unsafe_rows, 0u, prmt(nib, 0u, 0x4420) & 0x3333u);
-            const uint32_t unsafe_w = ((((present & rowmask) + 0x0F0F0F0Fu) | present) >> 4) & 0x01010101u;
-#pragma unroll
-            for (int e = 0; e < kEPT; ++e)
-                if (e < rem) st_reward += __float2int_rn(rout[e] * 16777216.0f);
-            {
-                const uint32_t vb = valid_bytes(rem);
-                st_steps += rem;
-                st_unsafe = add_bytes(unsafe_w & vb, st_unsafe);
-                st_count = add_bytes(count_w & vb, st_count);
-                st_trunc = add_bytes(trunc_w & vb, st_trunc);
-            }
-            st_stream_v4(io.t + e0, make_int4(tn[0], tn[1], tn[2], tn[3]));
-            st_stream_v4(io.reward + e0, make_int4(__float_as_int(rout[0]), __float_as_int(rout[1]),
-                                                   __float_as_int(rout[2]), __float_as_int(rout[3])));
-            st_stream_v4(io.index + e0, make_int4(acc.idx[0], acc.idx[1], acc.idx[2], acc.idx[3]));
-            st_stream_u32(io.terminated + e0, 0u);
-            st_stream_u32(io.truncated + e0, trunc_w);
-            st_stream_u32(io.unsafe + e0, unsafe_w);
-            st_stream_u32(io.count + e0, count_w);
+            finish_word(tab, io, e0, rem, acc, tn, trunc_w, st_steps, st_unsafe, st_count, st_trunc, st_reward);
 #pragma unroll
             for (int c = 0; c < C; ++c) sw[c / 4][c % 4] = nx[c / 4][c % 4];
 #pragma unroll
@@ -480,11 +452,7 @@ cell_pair_many_kernel(const __grid_constant__ CellTables tab, const __grid_const
         const ThreadStats ts = {st_steps, st_unsafe, st_count, st_trunc, st_reward};
         block_flush_stats(ts, s_stats, io.stats);
     }
-    // the block that arrived last advances the device step counter by the steps of this launch
-    if (threadIdx.x == 0 && io.done_ctr != nullptr && s_ctr.arrived == gridDim.x - 1) {
-        *io.done_ctr = 0u;
-        *const_cast<uint32_t *>(io.step_ctr) = s_ctr.step + static_cast<uint32_t>(mio.n_steps);
-    }
+    step_counter_finish(io, &s_ctr, static_cast<uint32_t>(mio.n_steps));
 }
 
 template <int C, int RNG, bool WITH_SE, int THREADS>
@@ -495,18 +463,16 @@ cudaError_t launch_pair_many_t(const CellTables &tab, const ManyIO &mio, const u
                               grid_for<cell_pair_many_kernel<C, RNG, WITH_SE, THREADS>, THREADS>(n, n_sm), THREADS, 0, st, tab, mio, lut);
 }
 
-// Shards that do not fill every SM with 256-thread blocks (65,536 envs = 64 of them) are spread over more SMs with
-// 64-thread blocks: the steps of such a shard are bound by the dependent-instruction latency of its warps
-// (config 2, same box: 99-106 G env-steps/s with 256-thread blocks, 117-140 with 128, 132 with 64; packed 113-122 / 117-120 / 127-128).
+// shards that do not fill every SM with 256-thread blocks take smaller blocks (kManySmallThreads)
 template <int C, int RNG>
 cudaError_t launch_pair_many_cr(const CellTables &tab, const ManyIO &mio, const uint2 *lut, int n_sm, cudaStream_t st)
 {
     const int64_t n = mio.io.end - mio.io.begin;
     const bool small = (n + kThreads * kEPT - 1) / (kThreads * kEPT) < n_sm;
     if (mio.io.se_row)
-        return small ? launch_pair_many_t<C, RNG, true, GC_MANY_SMALL_THREADS>(tab, mio, lut, n_sm, st)
+        return small ? launch_pair_many_t<C, RNG, true, kManySmallThreads>(tab, mio, lut, n_sm, st)
                      : launch_pair_many_t<C, RNG, true, kThreads>(tab, mio, lut, n_sm, st);
-    return small ? launch_pair_many_t<C, RNG, false, GC_MANY_SMALL_THREADS>(tab, mio, lut, n_sm, st)
+    return small ? launch_pair_many_t<C, RNG, false, kManySmallThreads>(tab, mio, lut, n_sm, st)
                  : launch_pair_many_t<C, RNG, false, kThreads>(tab, mio, lut, n_sm, st);
 }
 

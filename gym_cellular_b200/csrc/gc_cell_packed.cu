@@ -274,9 +274,6 @@ cell_packed_kernel(const __grid_constant__ CellTables tab, const __grid_constant
 // k is computed, every per-step output is written at every step by the same packed_word as the step kernel (so
 // the results are bit-identical to n_steps launches), and the table is always replicated: its staging is paid
 // once per launch.
-#ifndef GC_MANY_SMALL_THREADS
-#define GC_MANY_SMALL_THREADS 64
-#endif
 template <int C, int RNG, bool EXTRA, int THREADS>
 __global__ void __launch_bounds__(THREADS, 256 / THREADS * 2)
 cell_packed_many_kernel(const __grid_constant__ CellTables tab, const __grid_constant__ PackedManyIO mio,
@@ -337,10 +334,7 @@ cell_packed_many_kernel(const __grid_constant__ CellTables tab, const __grid_con
         const ThreadStats ts = {st_steps, st_unsafe, st_count, st_trunc, st_reward};
         block_flush_stats(ts, s_stats, io.stats);
     }
-    if (threadIdx.x == 0 && io.done_ctr != nullptr && s_ctr.arrived == gridDim.x - 1) {
-        *io.done_ctr = 0u;
-        *const_cast<uint32_t *>(io.step_ctr) = s_ctr.step + static_cast<uint32_t>(mio.n_steps);
-    }
+    step_counter_finish(io, &s_ctr, static_cast<uint32_t>(mio.n_steps));
 }
 
 template <int C, int RNG, bool EXTRA, int THREADS>
@@ -359,13 +353,13 @@ cudaError_t launch_packed_many_t(const CellTables &tab, const PackedManyIO &mio,
     return launch_step_kernel(kernel, grid, THREADS, smem, st, tab, mio, lut, packed_rep_log2(RNG, true));
 }
 
-// shards that do not fill every SM with 256-thread blocks take smaller blocks (see cell_pair_many_kernel's launcher)
+// shards that do not fill every SM with 256-thread blocks take smaller blocks (kManySmallThreads)
 template <int C, int RNG, bool EXTRA>
 cudaError_t launch_packed_many_cre(const CellTables &tab, const PackedManyIO &mio, const uint2 *lut, int n_sm, cudaStream_t st)
 {
     const int64_t n = mio.io.end - mio.io.begin;
     const bool small = (n + kPackThreads * kEPT - 1) / (kPackThreads * kEPT) < n_sm;
-    return small ? launch_packed_many_t<C, RNG, EXTRA, GC_MANY_SMALL_THREADS>(tab, mio, lut, n_sm, st)
+    return small ? launch_packed_many_t<C, RNG, EXTRA, kManySmallThreads>(tab, mio, lut, n_sm, st)
                  : launch_packed_many_t<C, RNG, EXTRA, kPackThreads>(tab, mio, lut, n_sm, st);
 }
 

@@ -8,6 +8,11 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kEPT = 4;
+// Block size of the many-step kernels for shards that do not fill every SM with 256-thread blocks (65,536 envs =
+// 64 of them): such a shard is spread over more SMs, since its steps are bound by the dependent-instruction latency
+// of its warps (config 2, same box: 99-106 G env-steps/s with 256-thread blocks, 117-140 with 128, 132 with 64;
+// packed 113-122 / 117-120 / 127-128).
+constexpr int kManySmallThreads = 64;
 
 // ---------------------------------------------------------------------------------------------
 // Philox4x32-10, counter based: word w of env e at step t = philox(key=seed, ctr=(e_lo,e_hi,t,w/4))[w%4].
@@ -185,7 +190,7 @@ __device__ __forceinline__ void tick_step_counter(const IO &io) { tick_step_coun
 //   step_counter_read    before the block's first __syncthreads: thread 0 copies the counter to shared
 //                        memory (the store needs the loaded value, so the load has completed at the barrier)
 //   step_counter_arrive  after that barrier: thread 0 arrives; every thread gets the step from shared memory
-//   step_counter_finish  at kernel exit: the block that arrived last advances the counter.
+//   step_counter_finish  at kernel exit: the block that arrived last advances the counter by the launch's steps.
 // Every block has read the counter before it arrives, so when the last arrival is known nobody of this
 // launch reads the counter any more; the next launch starts after this one has completed.
 struct StepCounterShared { uint32_t step, arrived; };
@@ -204,11 +209,11 @@ __device__ __forceinline__ uint32_t step_counter_arrive(const IO &io, StepCounte
 }
 
 template <class IO>
-__device__ __forceinline__ void step_counter_finish(const IO &io, const StepCounterShared *s)
+__device__ __forceinline__ void step_counter_finish(const IO &io, const StepCounterShared *s, uint32_t n_steps = 1u)
 {
     if (threadIdx.x == 0 && io.done_ctr != nullptr && s->arrived == gridDim.x - 1) {
         *io.done_ctr = 0u;
-        *const_cast<uint32_t *>(io.step_ctr) = s->step + 1u;
+        *const_cast<uint32_t *>(io.step_ctr) = s->step + n_steps;
     }
 }
 

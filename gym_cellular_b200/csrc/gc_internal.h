@@ -179,9 +179,6 @@ cudaError_t gc_launch_cell_pair_step(const CellTables &tab, const StepIO &io, co
 cudaError_t gc_launch_grid_many(const GridParams &gp, const ManyIO &mio, int n_sm, cudaStream_t stream);
 cudaError_t gc_launch_cell_pair_many(const CellTables &tab, const ManyIO &mio, const uint2 *lut, int rng_mode, int n_sm,
                                      cudaStream_t stream);
-// TMA bulk-staged variant of the deterministic pair-table step for wide envs (gc_cell_tma.cu)
-cudaError_t gc_launch_cell_tma_step(const CellTables &tab, const StepIO &io, const uint2 *lut, int n_sm,
-                                    cudaStream_t stream);
 // 5..8 levels / actions (gc_cell_pair8.cu): 4096 pair entries [a_d][s_d][a_c][s_c] (3-bit digits, no noise)
 // followed by 128 single-cell entries [fire][a][s]
 #define GC_PAIR8_PAIRS 4096

@@ -22,7 +22,6 @@ import os
 import re
 import shutil
 import subprocess
-import sys
 import tempfile
 
 import numpy as np
@@ -287,70 +286,7 @@ def _run_plain(B, tabs, *, se, force, replay, seed, steps=3):
 
 
 # ---------------------------------------------------------------------------------------------
-# 2. TMA (opt-in, GC_B200_TMA=1, read once per process): every C = 8..16 in one subprocess
-
-_TMA_CHILD = """
-import json, sys, os
-sys.path.insert(0, os.getcwd())
-sys.path.insert(0, os.path.join(os.getcwd(), "tests"))
-import numpy as np, torch
-import gym_cellular_b200 as B
-from test_gpu_every_kernel import launches
-with launches() as L:
-    for path in sys.argv[1:]:
-        d = dict(np.load(path, allow_pickle=True))
-        tabs = d.pop("tabs").item()
-        env = B.CellularVectorEnv(num_envs=int(d["n"]), cell_tables=tabs, max_episode_steps=3, emit_side_effects=False,
-                                  rng_episodic=True)
-        env.set_state(torch.from_numpy(d["cells"]).cuda(), t=torch.from_numpy(d["t0"]).cuda())
-        out = {}
-        for k, a in enumerate(d["actions"]):
-            env.step_device(torch.from_numpy(a).cuda())
-            n = env.num_envs
-            for name, v in (("state", env.state), ("index", env.tabular_state(torch.int32)), ("t", env.time_step),
-                            ("reward", env._reward[:n]), ("unsafe", env._unsafe[:n]), ("count", env._count[:n]),
-                            ("truncated", env._truncated[:n])):
-                out[f"{name}{k}"] = v.cpu().numpy()
-        out["stats"] = env._stats.cpu().numpy()
-        np.savez(os.path.join(os.path.dirname(path), "out" + os.path.basename(path)[2:]), **out)
-print(json.dumps(sorted([k, list(v)] for k, v in L.names())))
-"""
-
-TMA_DECLARED = {("cell_tma_kernel", (C,)) for C in range(8, 17)}
-
-
-def test_tma_every_c(B, tmp_path):
-    from conftest import REPO
-    n, steps, cases = 100003, 3, {}
-    for C in range(8, 17):
-        S, A = STEP_SA[C]
-        tabs = make_tables(4242 + C, C, S, A, noise=False)
-        rng = np.random.default_rng(C)
-        cells = (rng.random((C, n)) * S).astype(np.int8)
-        t0 = rng.integers(0, 3, n).astype(np.int32)
-        acts = np.stack([(rng.random((C, n)) * A).astype(np.int8) for _ in range(steps)])
-        np.savez(tmp_path / f"in{C}.npz", tabs=np.array(tabs, dtype=object), n=n, cells=cells, t0=t0, actions=acts)
-        cases[C] = (tabs, cells, t0, acts)
-    r = subprocess.run([sys.executable, "-c", _TMA_CHILD] + [str(tmp_path / f"in{C}.npz") for C in cases],
-                       capture_output=True, text=True, cwd=REPO, env=dict(os.environ, GC_B200_TMA="1"))
-    assert r.returncode == 0, r.stderr[-1500:]
-    seen = {(k, tuple(v)) for k, v in json.loads(r.stdout.strip().splitlines()[-1])}
-    assert TMA_DECLARED <= seen, sorted(TMA_DECLARED - seen)
-    for C, (tabs, cells, t0, acts) in cases.items():
-        got = np.load(tmp_path / f"out{C}.npz")
-        ref = TR.TableEnv(f32_tables(tabs), n, rng_episodic=True, max_episode_steps=3)
-        ref.set_state(cells, t0)
-        for k, a in enumerate(acts):
-            ref.step(a)
-            for name in ("state", "t", "unsafe", "count", "truncated"):
-                assert (got[f"{name}{k}"] == getattr(ref, name)).all(), (C, name, k)
-            assert (got[f"index{k}"].view(np.uint32) == ref.index).all()
-            check_reward(got[f"reward{k}"], ref, "dyadic")
-        assert (got["stats"][:5] == ref.stats[:5]).all()
-
-
-# ---------------------------------------------------------------------------------------------
-# 3. step_many, fused: cell_pair_many_kernel<C, RNG, SE, THREADS> and cell_packed_many_kernel<C, RNG, EXTRA, THREADS>,
+# 2. step_many, fused: cell_pair_many_kernel<C, RNG, SE, THREADS> and cell_packed_many_kernel<C, RNG, EXTRA, THREADS>,
 #    C = 1..8, at 64-thread blocks (a batch that does not fill the SMs) and at 256-thread blocks with a wrapping
 #    grid-stride loop; against the reference and bit for bit against the separate launches
 
@@ -435,7 +371,7 @@ def test_step_many_every_kernel(B, monkeypatch, n_sm, C, big):
 
 
 # ---------------------------------------------------------------------------------------------
-# 4. rollout / record / count: cell_rollout_kernel<C, NOISE, MODE> for every C, with and without noise
+# 3. rollout / record / count: cell_rollout_kernel<C, NOISE, MODE> for every C, with and without noise
 
 ROLL_SA = {1: (4, 4), 2: (4, 3), 3: (3, 4), 4: (4, 2), 5: (2, 4), 6: (3, 3), 7: (3, 2), 8: (2, 3), 9: (3, 3),
            10: (4, 2), 11: (2, 4), 12: (4, 3), 13: (2, 2), 14: (3, 2), 15: (2, 3), 16: (2, 3)}
@@ -552,7 +488,7 @@ def test_rollout_modes_256_threads(B, n_sm, r):
 
 
 # ---------------------------------------------------------------------------------------------
-# 5. grid world: grid_step_kernel<RNG, LUT_GLOBAL>, grid_many_kernel, grid_rollout_kernel<MODE> at both block sizes
+# 4. grid world: grid_step_kernel<RNG, LUT_GLOBAL>, grid_many_kernel, grid_rollout_kernel<MODE> at both block sizes
 
 GRID_STEP_DECLARED = {("grid_step_kernel", (r, g)) for r in (1, 2) for g in (0, 1)}
 GRID_MANY_DECLARED = {("grid_many_kernel", ())}
@@ -661,7 +597,7 @@ def test_grid_rollout_modes(B, O, golden_gw, n_sm, big):
 
 
 # ---------------------------------------------------------------------------------------------
-# 6. the codec, reset, pack / unpack and step-counter kernels
+# 5. the codec, reset, pack / unpack and step-counter kernels
 
 AUX_DECLARED = {(k, ()) for k in ("encode_kernel", "decode_kernel", "encode_mixed_kernel", "decode_mixed_kernel",
                                   "reset_kernel", "reset_packed_kernel", "pack_kernel", "unpack_kernel", "tick_kernel")}
@@ -709,7 +645,7 @@ EXCLUDED = {}                   # (kernel, template values): reason
 
 
 def declared():
-    out = set(PAIR8_DECLARED | GENERIC_DECLARED | TMA_DECLARED | GRID_STEP_DECLARED | GRID_MANY_DECLARED |
+    out = set(PAIR8_DECLARED | GENERIC_DECLARED | GRID_STEP_DECLARED | GRID_MANY_DECLARED |
               GRID_ROLL_DECLARED | AUX_DECLARED)
     for C in range(1, 17):
         out |= step_declared(C) | roll_declared(C, False) | roll_declared(C, True)

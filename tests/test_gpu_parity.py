@@ -842,32 +842,6 @@ def test_second_device_leaves_current_device_alone(B, O):
     assert (np.stack(obs) == ora.state).all() and torch.cuda.current_device() == 0
 
 
-def test_tma_variant(B):
-    """The opt-in TMA bulk-staged kernel (GC_B200_TMA=1) is bit-identical to the default kernel."""
-    import subprocess
-    import sys
-    code = (
-        "import sys, os, zlib; sys.path.insert(0, os.getcwd())\n"
-        "import torch, gym_cellular_b200 as B\n"
-        "n = 100003\n"
-        "env = B.CellularVectorEnv(num_envs=n, n_cells=16, n_states=4, emit_side_effects=False, max_episode_steps=5, difficulty='hard')\n"
-        "g = torch.Generator(device='cuda').manual_seed(1)\n"
-        "h = 0\n"
-        "for _ in range(7):\n"
-        "    env.step_device(torch.randint(0, 4, (16, n), dtype=torch.int8, device='cuda', generator=g))\n"
-        "    for t in (env.state, env.tabular_state(), env._reward[:n], env._unsafe[:n], env._count[:n], env._truncated[:n], env.time_step):\n"
-        "        h = zlib.crc32(t.cpu().numpy().tobytes(), h)\n"
-        "print('crc', h, env.stats())\n")
-    from conftest import REPO
-    outs = []
-    for flag in ("0", "1"):
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=REPO,
-                           env=dict(__import__("os").environ, GC_B200_TMA=flag))
-        assert r.returncode == 0, r.stderr[-600:]
-        outs.append(r.stdout.strip().splitlines()[-1])
-    assert outs[0] == outs[1] and outs[0].startswith("crc")
-
-
 def test_example_plan_and_rollout(B):
     """examples/plan_and_rollout.py: value iteration on the exported model beats random play."""
     import importlib.util

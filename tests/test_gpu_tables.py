@@ -16,9 +16,6 @@ case checks its own power: draws fire at a fraction near p, `unsafe` takes both 
 non-zero initial state and `count` takes at least two values."""
 import ctypes as C
 import math
-import os
-import subprocess
-import sys
 import zlib
 
 import numpy as np
@@ -525,7 +522,7 @@ def test_rollout_and_collect_reject_other_tables(B, kind):
 
 
 # ---------------------------------------------------------------------------------------------
-# host path, TMA
+# host path
 
 @pytest.mark.parametrize("packed", [False, True], ids=["int8", "packed"])
 def test_host_path(B, packed):
@@ -558,59 +555,6 @@ def test_host_path(B, packed):
         q += TR.q24(rew)
     check_stats(env, ref, q, fam)
     power.check(fam)
-
-
-_TMA_CHILD = """
-import sys, os
-sys.path.insert(0, os.getcwd())
-import numpy as np, torch
-import gym_cellular_b200 as B
-d = dict(np.load(sys.argv[1], allow_pickle=True))
-tabs = d.pop("tabs").item()
-env = B.CellularVectorEnv(num_envs=int(d["n"]), cell_tables=tabs, max_episode_steps=3, emit_side_effects=False,
-                          rng_episodic=True)
-env.set_state(torch.from_numpy(d["cells"]).cuda(), t=torch.from_numpy(d["t0"]).cuda())
-out = {}
-for k, a in enumerate(d["actions"]):
-    env.step_device(torch.from_numpy(a).cuda())
-    n = env.num_envs
-    for name, v in (("state", env.state), ("index", env.tabular_state(torch.int32)), ("t", env.time_step),
-                    ("reward", env._reward[:n]), ("unsafe", env._unsafe[:n]), ("count", env._count[:n]),
-                    ("truncated", env._truncated[:n])):
-        out[f"{name}{k}"] = v.cpu().numpy()
-out["stats"] = env._stats.cpu().numpy()
-np.savez(sys.argv[2], **out)
-"""
-
-
-def test_tma_variant_against_reference(B, tmp_path):
-    """The opt-in TMA kernel (GC_B200_TMA=1: deterministic pair tables, 8 cells or more, no side-effect row) on one
-    16-cell random table set, in a subprocess because the switch is read once per process."""
-    n, C = 100003, 16
-    tabs = make_tables(4242, C, 4, 4, noise=False, fam="large")
-    assert derive_path(tabs) == "pair"
-    ref = TR.TableEnv(f32_tables(tabs), n, rng_episodic=True, max_episode_steps=3)
-    rng = np.random.default_rng(4)
-    cells = rng.integers(0, 4, (C, n)).astype(np.int8)
-    t0 = rng.integers(0, 3, n).astype(np.int32)
-    acts = np.stack([rng.integers(0, 4, (C, n)).astype(np.int8) for _ in range(4)])
-    np.savez(tmp_path / "in.npz", tabs=np.array(tabs, dtype=object), n=n, cells=cells, t0=t0, actions=acts)
-    from conftest import REPO
-    r = subprocess.run([sys.executable, "-c", _TMA_CHILD, str(tmp_path / "in.npz"), str(tmp_path / "out.npz")],
-                       capture_output=True, text=True, cwd=REPO, env=dict(os.environ, GC_B200_TMA="1"))
-    assert r.returncode == 0, r.stderr[-800:]
-    got = np.load(tmp_path / "out.npz")
-    ref.set_state(cells, t0)
-    power = Power(ref)
-    for k, a in enumerate(acts):
-        ref.step(a)
-        power.add(ref)
-        for name in ("state", "t", "unsafe", "count", "truncated"):
-            assert (got[f"{name}{k}"] == getattr(ref, name)).all(), (name, k)
-        assert (got[f"index{k}"].view(np.uint32) == ref.index).all()
-        check_reward(got[f"reward{k}"], ref, "large")
-    assert (got["stats"][:5] == ref.stats[:5]).all()
-    power.check("large")
 
 
 # ---------------------------------------------------------------------------------------------
