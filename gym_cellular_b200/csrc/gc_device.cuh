@@ -244,7 +244,9 @@ __device__ __forceinline__ float log2_1p(float r)
 }
 
 // The same for the four envs of a thread: one range test (two FMNMX trees) guards the polynomial path
-// of all four, so the common case carries no per-env branch.
+// of all four, so the common case carries no per-env branch.  A word with some sum outside [-1/2, 1] takes
+// log2_1p env by env, so that every env's reward is a function of its own sum (the one the generic kernel
+// computes), whatever the three other envs of its word hold.
 __device__ __forceinline__ void log2_1p_x4(int enabled, const float (&r)[4], float (&out)[4])
 {
     if (!enabled) {
@@ -258,7 +260,7 @@ __device__ __forceinline__ void log2_1p_x4(int enabled, const float (&r)[4], flo
         for (int e = 0; e < 4; ++e) out[e] = log2_1p_small(r[e]);
     } else {
 #pragma unroll
-        for (int e = 0; e < 4; ++e) out[e] = log1pf(r[e]) * 1.44269504088896341f;
+        for (int e = 0; e < 4; ++e) out[e] = log2_1p(r[e]);
     }
 }
 

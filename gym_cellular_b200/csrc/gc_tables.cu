@@ -56,6 +56,14 @@ void gc_build_grid_lut(uint32_t *lut)
 }
 
 // ---------------------------------------------------------------------------------------------
+// Reward entries of the cellular LUTs: the float32 sum of the cells' rewards in double, +0.0 where it is zero.
+// The kernels take the first entry of an env as its initial sum, so a -0.0 entry would give a -0.0 reward where
+// the paths that add from 0.0f (rollout, pair8, generic) give +0.0; with no -0.0 entry no float32 sum is -0.0.
+static float reward_entry(double r)
+{
+    return r == 0.0 ? 0.0f : (float)r;
+}
+
 // Cellular family, S, A <= 4: pair / single-cell entries (layout in gc_cell_fast.cu).
 void gc_build_pair_lut(const gc_cell_tables *t, int C, int S, int A, bool noise, uint2 *lut, uint32_t *unsafe_rows)
 {
@@ -78,14 +86,14 @@ void gc_build_pair_lut(const gc_cell_tables *t, int C, int S, int A, bool noise,
         const uint32_t uns01 = (C >= 2 && (se(0, nc, nd) == 2 || se(1, nc, nd) == 2)) ? 1u : 0u;
         lut[p].x = (cn(nc) + cn(nd)) | (((1u << nc) | (1u << nd)) << 8) | (uns01 << 12) |
                    ((uint32_t)nc << 16) | ((uint32_t)nd << 24);
-        const float f = (float)(rw(sc, ac, (p >> 8) & 1) + rw(sd, ad, (p >> 9) & 1));
+        const float f = reward_entry(rw(sc, ac, (p >> 8) & 1) + rw(sd, ad, (p >> 9) & 1));
         std::memcpy(&lut[p].y, &f, sizeof(f));
     }
     for (int p = 0; p < 32; ++p) {
         const int s = p & 3, a = (p >> 2) & 3, n = nxt(s, a, (p >> 4) & 1);
         const uint32_t uns0 = (C == 1 && se(0, n, n) == 2) ? 1u : 0u;
         lut[GC_PAIR_LUT_PAIRS + p].x = cn(n) | ((1u << n) << 8) | (uns0 << 12) | ((uint32_t)n << 16);
-        const float f = (float)rw(s, a, (p >> 4) & 1);
+        const float f = reward_entry(rw(s, a, (p >> 4) & 1));
         std::memcpy(&lut[GC_PAIR_LUT_PAIRS + p].y, &f, sizeof(f));
     }
     *unsafe_rows = 0;
@@ -136,14 +144,14 @@ void gc_build_packed_lut(const gc_cell_tables *t, int C, int S, int A, bool nois
         const int nc = nxt(sc, ac, fc), nd = nxt(sd, ad, fd);
         const uint32_t uns01 = (C >= 2 && (se(0, nc, nd) == 2 || se(1, nc, nd) == 2)) ? 1u : 0u;
         lut[p].x = (info(nc) + info(nd)) | (uns01 << 25) | ((uint32_t)(nc | (nd << 2)) << 28);
-        const float f = (float)(rw(sc, ac, fc) + rw(sd, ad, fd));
+        const float f = reward_entry(rw(sc, ac, fc) + rw(sd, ad, fd));
         std::memcpy(&lut[p].y, &f, sizeof(f));
     }
     for (int p = 0; p < 32; ++p) {
         const int s = p & 3, a = (p >> 2) & 3, n = nxt(s, a, (p >> 4) & 1);
         const uint32_t uns0 = (C == 1 && se(0, n, n) == 2) ? 1u : 0u;
         lut[GC_PAIR_LUT_PAIRS + p].x = info(n) | (uns0 << 25) | ((uint32_t)n << 28);
-        const float f = (float)rw(s, a, (p >> 4) & 1);
+        const float f = reward_entry(rw(s, a, (p >> 4) & 1));
         std::memcpy(&lut[GC_PAIR_LUT_PAIRS + p].y, &f, sizeof(f));
     }
 }
@@ -175,14 +183,14 @@ void gc_build_pair8_lut(const gc_cell_tables *t, int C, int S, int A, bool noise
         const int nc = nxt(sc, ac, 0), nd = nxt(sd, ad, 0);
         const uint32_t uns01 = (C >= 2 && (se(0, nc, nd) == 2 || se(1, nc, nd) == 2)) ? 1u : 0u;
         lut[p].x = (cn(nc) + cn(nd)) | (uns01 << 7) | (((1u << nc) | (1u << nd)) << 8) | ((uint32_t)nc << 16) | ((uint32_t)nd << 24);
-        const float f = (float)(rw(sc, ac, 0) + rw(sd, ad, 0));
+        const float f = reward_entry(rw(sc, ac, 0) + rw(sd, ad, 0));
         std::memcpy(&lut[p].y, &f, sizeof(f));
     }
     for (int p = 0; p < 128; ++p) {
         const int s = p & 7, a = (p >> 3) & 7, n = nxt(s, a, p >> 6);
         const uint32_t uns0 = (C == 1 && se(0, n, n) == 2) ? 1u : 0u;
         lut[GC_PAIR8_PAIRS + p].x = cn(n) | (uns0 << 7) | ((1u << n) << 8) | ((uint32_t)n << 16);
-        const float f = (float)rw(s, a, p >> 6);
+        const float f = reward_entry(rw(s, a, p >> 6));
         std::memcpy(&lut[GC_PAIR8_PAIRS + p].y, &f, sizeof(f));
     }
     *unsafe_rows8 = 0;

@@ -124,6 +124,7 @@ class TableEnv:
         self.final_state = ns.astype(np.int8)
         ns = np.where(trunc[None, :], self.init[:, None], ns)
         tn[trunc] = 0
+        self.last_s, self.last_a = s, a
         self.last_fire, self.last_draws = fire, self.draws[s, a] & self.noise
         self.state, self.t, self.index = ns.astype(np.int8), tn.astype(np.int32), self.encode(ns)
         self.reward_out, self.se_row = r, se_row.astype(np.int8)
