@@ -22,7 +22,8 @@ EXPORTS = ["gc_abi_version", "gc_last_error", "gc_create", "gc_destroy", "gc_set
            "gc_set_global_step", "gc_get_global_step", "gc_sync_global_step", "gc_launch_count", "gc_reset", "gc_step",
            "gc_bind_step", "gc_step_bound", "gc_step_many", "gc_prepare_step_many", "gc_step_host", "gc_rollout", "gc_collect", "gc_collect_counts", "gc_poll_status", "gc_encode",
            "gc_decode", "gc_encode_mixed", "gc_decode_mixed", "gc_reset_packed", "gc_step_packed", "gc_bind_step_packed",
-           "gc_step_host_packed", "gc_pack_cells", "gc_unpack_cells"]
+           "gc_step_host_packed", "gc_pack_cells", "gc_unpack_cells", "gc_compressible_supported", "gc_alloc_compressible",
+           "gc_free_compressible", "gc_is_compressible"]
 FLAG_UNSAFE, FLAG_TRUNCATED, FLAG_COUNT_SHIFT = 1, 2, 2
 
 
@@ -107,6 +108,12 @@ def load():
     L.gc_step_host_packed.argtypes = [vp] * 13 + [i64]
     L.gc_pack_cells.argtypes = [C.c_int, i64, i64, i32, vp, vp, vp]
     L.gc_unpack_cells.argtypes = [C.c_int, i64, i64, i32, vp, vp, vp]
+    L.gc_compressible_supported.argtypes = [C.c_int]
+    L.gc_alloc_compressible.argtypes = [C.c_size_t, C.c_int, vp]
+    L.gc_alloc_compressible.restype = vp
+    L.gc_free_compressible.argtypes = [vp, C.c_size_t, C.c_int, vp]
+    L.gc_free_compressible.restype = None
+    L.gc_is_compressible.argtypes = [vp]
     if L.gc_abi_version() != ABI_VERSION:
         raise ImportError(f"ABI version mismatch: library {L.gc_abi_version()} != binding {ABI_VERSION}")
     _lib = L

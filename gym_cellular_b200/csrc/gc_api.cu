@@ -6,10 +6,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <initializer_list>
 #include <memory>
 #include <new>
+#include <unordered_map>
 
+#include <cuda.h>
 #include <nvtx3/nvToolsExt.h>
 
 #include "gc_internal.h"
@@ -1231,6 +1234,183 @@ int gc_unpack_cells(int device, int64_t n, int64_t ld, int32_t n_cells, const ui
     cudaError_t e = gc_launch_unpack((n + 3) / 4 * 4, ld, n_cells, packed, cells, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return fail(GC_ERR_CUDA, "unpack kernel launch failed: %s", cudaGetErrorString(e));
     return GC_OK;
+}
+
+}  // extern "C"
+
+// ---- generic compressible device memory for the env-owned step buffers -------------------------------------------
+// L2 <-> DRAM transfers of low-entropy 128 B lines in such memory move fewer bytes; kernels see ordinary memory
+// (profiles/r05_compression.md).  The driver API is reached through the runtime's entry-point query, so the library
+// links against the runtime alone.
+namespace {
+
+struct VmmApi {
+    decltype(&cuMemCreate) create = nullptr;
+    decltype(&cuMemRelease) release = nullptr;
+    decltype(&cuMemAddressReserve) reserve = nullptr;
+    decltype(&cuMemAddressFree) address_free = nullptr;
+    decltype(&cuMemMap) map = nullptr;
+    decltype(&cuMemUnmap) unmap = nullptr;
+    decltype(&cuMemSetAccess) set_access = nullptr;
+    decltype(&cuMemGetAllocationGranularity) granularity = nullptr;
+    decltype(&cuMemGetAllocationPropertiesFromHandle) properties = nullptr;
+    decltype(&cuDeviceGet) device_get = nullptr;
+    decltype(&cuDeviceGetAttribute) attribute = nullptr;
+    bool ok = false;
+};
+
+template <class F>
+bool driver_entry(const char *name, F &fn)
+{
+    void *p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess || !p)
+        return false;
+    fn = reinterpret_cast<F>(p);
+    return true;
+}
+
+const VmmApi &vmm()
+{
+    static const VmmApi api = [] {
+        VmmApi a;
+        a.ok = driver_entry("cuMemCreate", a.create) && driver_entry("cuMemRelease", a.release) &&
+               driver_entry("cuMemAddressReserve", a.reserve) && driver_entry("cuMemAddressFree", a.address_free) &&
+               driver_entry("cuMemMap", a.map) && driver_entry("cuMemUnmap", a.unmap) &&
+               driver_entry("cuMemSetAccess", a.set_access) &&
+               driver_entry("cuMemGetAllocationGranularity", a.granularity) &&
+               driver_entry("cuMemGetAllocationPropertiesFromHandle", a.properties) &&
+               driver_entry("cuDeviceGet", a.device_get) && driver_entry("cuDeviceGetAttribute", a.attribute);
+        return a;
+    }();
+    return api;
+}
+
+struct Mapping {
+    CUmemGenericAllocationHandle handle;
+    size_t size;
+};
+std::mutex g_maps_mu;
+std::unordered_map<void *, Mapping> g_maps;     // compressible mappings; any other pointer came from cudaMallocAsync
+
+// GC_B200_COMPRESSIBLE=0 forces every allocation onto the cudaMallocAsync fallback
+bool compression_enabled()
+{
+    const char *v = std::getenv("GC_B200_COMPRESSIBLE");
+    return !(v && v[0] == '0');
+}
+
+// A compressible mapping of `size` bytes (rounded up to the granularity), or nullptr when the device or driver
+// does not grant one.
+void *map_compressible(size_t size, int device, size_t *mapped)
+{
+    const VmmApi &api = vmm();
+    if (!api.ok) return nullptr;
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t gran = 0;
+    if (api.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || gran == 0) return nullptr;
+    size = (size + gran - 1) / gran * gran;
+    CUmemGenericAllocationHandle h;
+    if (api.create(&h, size, &prop, 0) != CUDA_SUCCESS) return nullptr;
+    CUmemAllocationProp got = {};
+    CUdeviceptr ptr = 0;
+    bool ok = api.properties(&got, h) == CUDA_SUCCESS && got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC;
+    if (ok) ok = api.reserve(&ptr, size, gran, 0, 0) == CUDA_SUCCESS;
+    if (ok && api.map(ptr, size, 0, h, 0) != CUDA_SUCCESS) {
+        api.address_free(ptr, size);
+        ok = false;
+    }
+    if (ok) {
+        CUmemAccessDesc access = {};
+        access.location = prop.location;
+        access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+        if (api.set_access(ptr, size, &access, 1) != CUDA_SUCCESS) {
+            api.unmap(ptr, size);
+            api.address_free(ptr, size);
+            ok = false;
+        }
+    }
+    if (!ok) {
+        api.release(h);
+        return nullptr;
+    }
+    void *p = reinterpret_cast<void *>(ptr);
+    std::lock_guard<std::mutex> lock(g_maps_mu);
+    g_maps[p] = Mapping{h, size};
+    *mapped = size;
+    return p;
+}
+
+}  // namespace
+
+extern "C" {
+
+int gc_compressible_supported(int device)
+{
+    const VmmApi &api = vmm();
+    CUdevice dev;
+    int v = 0;
+    if (!compression_enabled() || !api.ok || api.device_get(&dev, device) != CUDA_SUCCESS ||
+        api.attribute(&v, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, dev) != CUDA_SUCCESS)
+        return 0;
+    return v ? 1 : 0;
+}
+
+void *gc_alloc_compressible(size_t size, int device, void *stream)
+{
+    if (size == 0) return nullptr;
+    DeviceGuard guard(device);
+    if (guard.error() != cudaSuccess) return nullptr;
+    size_t mapped = 0;
+    if (gc_compressible_supported(device))
+        if (void *p = map_compressible(size, device, &mapped)) return p;
+    void *p = nullptr;
+    if (cudaMallocAsync(&p, size, static_cast<cudaStream_t>(stream)) != cudaSuccess) {
+        cudaGetLastError();
+        return nullptr;
+    }
+    return p;
+}
+
+void gc_free_compressible(void *ptr, size_t size, int device, void *stream)
+{
+    (void)size;
+    if (!ptr) return;
+    DeviceGuard guard(device);
+    Mapping m{};
+    bool mapped = false;
+    {
+        std::lock_guard<std::mutex> lock(g_maps_mu);
+        auto it = g_maps.find(ptr);
+        if (it != g_maps.end()) {
+            m = it->second;
+            g_maps.erase(it);
+            mapped = true;
+        }
+    }
+    // the last owner may be gone while work on any stream still uses the memory, and unlike cudaFree, unmapping
+    // does not wait for it
+    cudaDeviceSynchronize();
+    if (!mapped) {
+        cudaFreeAsync(ptr, static_cast<cudaStream_t>(stream));
+        return;
+    }
+    const VmmApi &api = vmm();
+    CUdeviceptr p = reinterpret_cast<CUdeviceptr>(ptr);
+    api.unmap(p, m.size);
+    api.address_free(p, m.size);
+    api.release(m.handle);
+}
+
+int gc_is_compressible(const void *ptr)
+{
+    std::lock_guard<std::mutex> lock(g_maps_mu);
+    return g_maps.count(const_cast<void *>(ptr)) ? 1 : 0;
 }
 
 }  // extern "C"

@@ -65,18 +65,25 @@ class PackedCellularVectorEnv(CellularVectorEnv):
             raise ValueError("the packed layout needs n_states, n_actions <= 4 (2 bits per cell)")
         dev, ld = self.device, self.ld
         z = lambda *shape, dtype: torch.zeros(*shape, dtype=dtype, device=dev)
-        self._state = z(ld, dtype=torch.int32)            # uint32 payload: 2 bits per cell
+        step = self._step_buffer_zeros()
+        self._state = step(ld, dtype=torch.int32)         # uint32 payload: 2 bits per cell
         self._actions = z(ld, dtype=torch.int32)
-        self._t = z(ld, dtype=torch.int32)
-        self._reward = z(ld, dtype=torch.float32)
-        self._flags = z(ld, dtype=torch.uint8)
+        self._t = step(ld, dtype=torch.int32)
+        self._reward = step(ld, dtype=torch.float32)
+        self._flags = step(ld, dtype=torch.uint8)
         # four levels: the state word is the tabular index; otherwise the kernel writes it separately
-        self._index = self._state if self.n_states == 4 else z(ld, dtype=torch.int32)
+        self._index = self._state if self.n_states == 4 else step(ld, dtype=torch.int32)
         self._final = z(ld, dtype=torch.int32) if self.emit_final_obs else None
         self._se_row = z(ld, dtype=torch.int32) if self.emit_side_effects else None
         self._stats = z(_lib.N_STATS, dtype=torch.int64) if self._collect_stats else None
         self._false = z(ld, dtype=torch.bool)
         self._cells_scratch = None
+
+    def _step_buffers(self):
+        return (self._state, self._t, self._reward, self._flags, self._index)
+
+    def _step_bytes_per_env(self):
+        return 13 if self.n_states == 4 else 17
 
     def _index_ptr(self):
         return None if self._index is self._state else _ptr(self._index)

@@ -78,6 +78,29 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+_TYPESTR = {torch.int8: "|i1", torch.uint8: "|u1", torch.int32: "<i4", torch.float32: "<f4"}
+
+
+class _CompressibleBlock:
+    """One gc_alloc_compressible allocation, seen by torch through __cuda_array_interface__.  A tensor made from it
+    holds a reference to it, so the memory is freed (gc_free_compressible) when the last tensor and view is gone."""
+
+    def __init__(self, lib, shape, dtype, device):
+        self._lib, self._device = lib, device.index
+        self.nbytes = int(np.prod(shape)) * torch.empty(0, dtype=dtype).element_size()
+        stream = torch.cuda.current_stream(device).cuda_stream
+        self.ptr = lib.gc_alloc_compressible(self.nbytes, self._device, stream)
+        if not self.ptr:
+            raise torch.cuda.OutOfMemoryError(f"gc_alloc_compressible could not allocate {self.nbytes} bytes")
+        self.__cuda_array_interface__ = {"data": (self.ptr, False), "shape": tuple(shape), "typestr": _TYPESTR[dtype],
+                                         "version": 2, "strides": None}
+
+    def __del__(self):
+        if getattr(self, "ptr", None):
+            self._lib.gc_free_compressible(self.ptr, self.nbytes, self._device, None)     # synchronises the device
+            self.ptr = None
+
+
 class CellularVectorEnv(gym.vector.VectorEnv):
     """Batched polarisation / grid-world environment on one CUDA device.
 
@@ -96,6 +119,11 @@ class CellularVectorEnv(gym.vector.VectorEnv):
     emit_final_obs  also write the observation BEFORE a time-limit auto-reset: infos['final_obs'] (valid where
                     infos['_final_obs'], i.e. truncated) and infos['final_info'] -- gymnasium's SAME_STEP
                     convention; the reference itself never ends an episode (gym_cellular/__init__.py:7)
+    compressible_buffers   the env-owned step buffers (state, time step, reward, index, flags) in generic
+                    compressible memory, where L2 <-> DRAM transfers of low-entropy lines move fewer bytes
+                    (config 4 on a B200: 178 against 192 us per step, profiles/r05_compression.md); results are
+                    identical.  None = on where the device supports it and the step buffers exceed 1/16 of its
+                    L2.  `compressible` tells what was granted
     env_id_offset   global id of env 0: Philox streams are keyed by global id, so a batch sharded
                     over ranks reproduces the single-device results env by env
     """
@@ -109,7 +137,7 @@ class CellularVectorEnv(gym.vector.VectorEnv):
                  noise_prob=0.1, dispersal_prob=0.01, env_seed=0, rng_episodic=None,
                  max_episode_steps=None, device=None, env_id_offset=0, emit_side_effects=True,
                  collect_stats=True, host_chunk_envs=1 << 20, cell_tables=None, force_generic_kernel=False,
-                 emit_final_obs=False, cell_radix=None):
+                 emit_final_obs=False, cell_radix=None, compressible_buffers=None):
         self._lib = _lib.load()                      # raises ImportError when the .so is missing
         if not torch.cuda.is_available():
             raise RuntimeError("CellularVectorEnv needs a CUDA device: there is no CPU fallback")
@@ -186,6 +214,14 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             self._set_tables()
 
         self._collect_stats = bool(collect_stats)
+        if compressible_buffers is None:
+            # a small shard's step is bound by latency, not by DRAM bytes, and compressed lines cost latency: on by
+            # default above 1/16 of L2 (config 2, 1.2 MB of step buffers: 123-128 against 128-133 G env-steps/s
+            # compressed; config 3, 19 MB: 334-336 against 329-330 G)
+            l2 = torch.cuda.get_device_properties(self.device).L2_cache_size
+            compressible_buffers = (bool(self._lib.gc_compressible_supported(self.device.index))
+                                    and self.ld * self._step_bytes_per_env() > l2 // 16)
+        self._compressible_buffers = bool(compressible_buffers)
         self._alloc_device_buffers()
         self._host = None                                 # pinned mirrors, allocated on first host step
 
@@ -198,19 +234,46 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         self._build_views()
         self.reset()
 
+    def _step_buffer_zeros(self):
+        """zeros(*shape, dtype=...) for the env-owned step buffers: generic compressible memory when
+        `compressible_buffers` is on (gc_alloc_compressible, which falls back to ordinary device memory where the
+        device grants none), ordinary torch memory otherwise."""
+        dev = self.device
+        if not self._compressible_buffers:
+            return lambda *shape, dtype: torch.zeros(*shape, dtype=dtype, device=dev)
+
+        def zeros(*shape, dtype):
+            t = torch.as_tensor(_CompressibleBlock(self._lib, shape, dtype, dev), device=dev)
+            return t.zero_()
+        return zeros
+
+    @property
+    def compressible(self):
+        """True when every env-owned step buffer (state, time step, reward, index, flags) lives in generic
+        compressible memory: L2 <-> DRAM transfers of its low-entropy lines move fewer bytes."""
+        return all(self._lib.gc_is_compressible(_ptr(t)) for t in self._step_buffers())
+
+    def _step_buffers(self):
+        return (self._state, self._t, self._reward, self._index, self._terminated, self._truncated, self._unsafe,
+                self._count)
+
+    def _step_bytes_per_env(self):
+        return self.n_cells + 16
+
     def _alloc_device_buffers(self):
         """Device buffers (caller-owned as far as the library is concerned)."""
         dev, ld, Cn = self.device, self.ld, self.n_cells
         z = lambda *shape, dtype: torch.zeros(*shape, dtype=dtype, device=dev)
-        self._state = z(Cn, ld, dtype=torch.int8)
+        step = self._step_buffer_zeros()
+        self._state = step(Cn, ld, dtype=torch.int8)
         self._actions = z(Cn, ld, dtype=torch.int8)
-        self._t = z(ld, dtype=torch.int32)
-        self._reward = z(ld, dtype=torch.float32)
-        self._index = z(ld, dtype=torch.int32)           # uint32 payload (see tabular_state())
-        self._terminated = z(ld, dtype=torch.uint8)
-        self._truncated = z(ld, dtype=torch.uint8)
-        self._unsafe = z(ld, dtype=torch.uint8)
-        self._count = z(ld, dtype=torch.uint8)
+        self._t = step(ld, dtype=torch.int32)
+        self._reward = step(ld, dtype=torch.float32)
+        self._index = step(ld, dtype=torch.int32)        # uint32 payload (see tabular_state())
+        self._terminated = step(ld, dtype=torch.uint8)
+        self._truncated = step(ld, dtype=torch.uint8)
+        self._unsafe = step(ld, dtype=torch.uint8)
+        self._count = step(ld, dtype=torch.uint8)
         self._se_row = z(Cn, ld, dtype=torch.int8) if self.emit_side_effects else None
         self._stats = z(_lib.N_STATS, dtype=torch.int64) if self._collect_stats else None
         self._final = z(Cn, ld, dtype=torch.int8) if self.emit_final_obs else None

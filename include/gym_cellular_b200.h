@@ -43,6 +43,7 @@
 #ifndef GYM_CELLULAR_B200_H
 #define GYM_CELLULAR_B200_H
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -361,6 +362,20 @@ int gc_encode_mixed(int device, int64_t n, int64_t ld, int32_t n_cells, const in
                     const int8_t *cells, uint32_t *index, void *stream);
 int gc_decode_mixed(int device, int64_t n, int64_t ld, int32_t n_cells, const int32_t *radix, const int32_t *min,
                     const uint32_t *index, int8_t *cells, void *stream);
+
+/* Generic compressible device memory (cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC) for the env-owned step
+ * buffers: L2 <-> DRAM transfers of low-entropy 128 B lines move fewer bytes, and kernels see ordinary memory.  The gain
+ * depends on the data: zero and uniform lines compress, random state does not.
+ *   gc_compressible_supported: 1 when `device` grants such memory (0 also when GC_B200_COMPRESSIBLE=0).
+ *   gc_alloc_compressible / gc_free_compressible: the signatures of torch.cuda.memory.CUDAPluggableAllocator.  An
+ *     allocation is rounded up to the allocation granularity and mapped; when the device does not support it or the
+ *     driver does not grant a compressible allocation it comes from cudaMallocAsync on `stream` instead.  Alloc
+ *     returns NULL on failure.  Free synchronises the device first: the memory may still be in use on any stream.
+ *   gc_is_compressible: 1 when `ptr` is the base of a live compressible mapping of gc_alloc_compressible. */
+int gc_compressible_supported(int device);
+void *gc_alloc_compressible(size_t size, int device, void *stream);
+void gc_free_compressible(void *ptr, size_t size, int device, void *stream);
+int gc_is_compressible(const void *ptr);
 
 #ifdef __cplusplus
 }
