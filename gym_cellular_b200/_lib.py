@@ -16,14 +16,14 @@ F_NOISE, F_RNG_EPISODIC, F_REWARD_LOG2, F_GENERIC_KERNEL = 1, 4, 16, 32
 MAX_CELLS, MAX_LEVELS, N_STATS = 16, 8, 8
 STAT_STEPS, STAT_UNSAFE, STAT_COUNT, STAT_TRUNCATED, STAT_REWARD_Q24 = range(5)
 OK, ERR_INVALID, ERR_CUDA, ERR_STATE, ERR_ACTION = 0, -1, -2, -3, -4
-POLICY_RANDOM, POLICY_TABLE = 0, 1
+POLICY_RANDOM, POLICY_TABLE, POLICY_TABLE_STACK = 0, 1, 2
 
 EXPORTS = ["gc_abi_version", "gc_last_error", "gc_create", "gc_destroy", "gc_set_tables", "gc_set_final_obs",
            "gc_set_global_step", "gc_get_global_step", "gc_sync_global_step", "gc_launch_count", "gc_reset", "gc_step",
            "gc_bind_step", "gc_step_bound", "gc_step_many", "gc_prepare_step_many", "gc_step_host", "gc_rollout", "gc_collect", "gc_collect_counts", "gc_poll_status", "gc_encode",
            "gc_decode", "gc_encode_mixed", "gc_decode_mixed", "gc_reset_packed", "gc_step_packed", "gc_bind_step_packed",
            "gc_step_host_packed", "gc_pack_cells", "gc_unpack_cells", "gc_compressible_supported", "gc_alloc_compressible",
-           "gc_free_compressible", "gc_is_compressible"]
+           "gc_free_compressible", "gc_is_compressible", "gc_set_policy_stack"]
 FLAG_UNSAFE, FLAG_TRUNCATED, FLAG_COUNT_SHIFT = 1, 2, 2
 
 
@@ -114,6 +114,7 @@ def load():
     L.gc_free_compressible.argtypes = [vp, C.c_size_t, C.c_int, vp]
     L.gc_free_compressible.restype = None
     L.gc_is_compressible.argtypes = [vp]
+    L.gc_set_policy_stack.argtypes = [vp, vp, i32]
     if L.gc_abi_version() != ABI_VERSION:
         raise ImportError(f"ABI version mismatch: library {L.gc_abi_version()} != binding {ABI_VERSION}")
     _lib = L

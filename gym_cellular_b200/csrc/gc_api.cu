@@ -97,6 +97,8 @@ struct gc_env {
     uint2 *d_pair8_lut;           // 5..8 levels (gc_cell_pair8.cu): GC_PAIR8_ENTRIES entries
     bool pair8_ok;
     int8_t *final_state;          // gc_set_final_obs: optional extra output of every int8-layout step
+    const int32_t *policy_map;    // gc_set_policy_stack: table id of every env for GC_POLICY_TABLE_STACK, NULL = not set
+    int32_t n_policy_tables;
     bool fast_ok;
     StepIO bound[GC_MAX_BINDINGS];  // gc_bind_step slots
     PackedIO bound_packed[GC_MAX_BINDINGS];   // gc_bind_step_packed slots
@@ -520,6 +522,18 @@ int gc_set_final_obs(gc_env *env, int8_t *final_state)
     return GC_OK;
 }
 
+int gc_set_policy_stack(gc_env *env, const int32_t *table_of_env, int32_t n_tables)
+{
+    if (int rc = check_env(env)) return rc;
+    if (table_of_env) {
+        if (n_tables < 1) return fail(GC_ERR_INVALID, "n_tables must be >= 1 (got %d)", n_tables);
+        if ((reinterpret_cast<uintptr_t>(table_of_env) & 15u) != 0) return fail(GC_ERR_INVALID, "table_of_env must be 16-byte aligned");
+    }
+    env->policy_map = table_of_env;
+    env->n_policy_tables = table_of_env ? n_tables : 0;
+    return GC_OK;
+}
+
 int gc_set_global_step(gc_env *env, int64_t step)
 {
     if (int rc = check_env(env)) return rc;
@@ -889,7 +903,30 @@ RolloutIO make_rollout_io(const gc_env *env, int32_t n_steps, int32_t policy_kin
     io.episodic = (env->cfg.flags & GC_F_RNG_EPISODIC) ? 1 : 0;
     io.max_episode_steps = env->cfg.max_episode_steps;
     io.n_steps = n_steps; io.policy_kind = policy_kind;
+    if (policy_kind == GC_POLICY_TABLE_STACK) {
+        io.table_of_env = env->policy_map;
+        io.n_tables = static_cast<uint32_t>(env->n_policy_tables);
+        unsigned long long nS = 400;
+        if (env->cfg.kind == GC_KIND_CELLULAR) {
+            nS = 1;
+            for (int c = 0; c < env->cfg.n_cells; ++c) nS *= static_cast<unsigned long long>(env->cfg.n_states);
+        }
+        io.table_stride = nS;
+    }
     return io;
+}
+
+// the policy arguments of gc_rollout, gc_collect and gc_collect_counts
+int check_policy(const gc_env *env, int32_t policy_kind, const int32_t *policy)
+{
+    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE && policy_kind != GC_POLICY_TABLE_STACK)
+        return fail(GC_ERR_INVALID, "unknown policy kind");
+    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
+    if (policy_kind == GC_POLICY_TABLE_STACK && !policy)
+        return fail(GC_ERR_INVALID, "GC_POLICY_TABLE_STACK needs a stack of policy tables");
+    if (policy_kind == GC_POLICY_TABLE_STACK && !env->policy_map)
+        return fail(GC_ERR_STATE, "GC_POLICY_TABLE_STACK needs a table map: gc_set_policy_stack has not been called");
+    return GC_OK;
 }
 
 bool misaligned(const void *p) { return p && (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
@@ -903,8 +940,7 @@ int check_collect_args(gc_env *env, int32_t n_steps, int32_t policy_kind, const 
     if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
     if (!state || !t || !index || !out) return fail(GC_ERR_INVALID, "a required pointer is NULL");
     if (n_steps < 1) return fail(GC_ERR_INVALID, "n_steps must be >= 1");
-    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE) return fail(GC_ERR_INVALID, "unknown policy kind");
-    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
+    if (int rc = check_policy(env, policy_kind, policy)) return rc;
     if (!(epsilon >= 0.0 && epsilon <= 1.0)) return fail(GC_ERR_INVALID, "epsilon must lie in [0, 1] (got %g)", epsilon);
     if (policy_kind == GC_POLICY_RANDOM && epsilon != 0.0)
         return fail(GC_ERR_INVALID, "epsilon applies to GC_POLICY_TABLE only (GC_POLICY_RANDOM needs epsilon 0)");
@@ -935,8 +971,7 @@ int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     if (!env->tables_set) return fail(GC_ERR_STATE, "gc_set_tables has not been called");
     if (!state || !t || !index || !ret || !n_unsafe) return fail(GC_ERR_INVALID, "a required device pointer is NULL");
     if (n_steps < 1) return fail(GC_ERR_INVALID, "n_steps must be >= 1");
-    if (policy_kind != GC_POLICY_RANDOM && policy_kind != GC_POLICY_TABLE) return fail(GC_ERR_INVALID, "unknown policy kind");
-    if (policy_kind == GC_POLICY_TABLE && !policy) return fail(GC_ERR_INVALID, "GC_POLICY_TABLE needs a policy table");
+    if (int rc = check_policy(env, policy_kind, policy)) return rc;
     if (env->cfg.kind == GC_KIND_CELLULAR && !env->fast_ok)
         return fail(GC_ERR_INVALID, "gc_rollout supports the cellular family with n_states, n_actions <= 4 only");
     GC_ON_DEVICE(env->cfg.device);

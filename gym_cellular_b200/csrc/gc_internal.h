@@ -86,7 +86,7 @@ struct RolloutIO {
     uint32_t     *index;
     float        *ret;          // [ld] out: sum of the rewards of the n_steps steps
     int32_t      *n_unsafe;     // [ld] out: steps that reported 'unsafe'
-    const int32_t *policy;      // GC_POLICY_TABLE: tabular action index per tabular state, else NULL
+    const int32_t *policy;      // GC_POLICY_TABLE(_STACK): tabular action index per tabular state, else NULL
     unsigned long long *stats;
     unsigned long long *status;
     int64_t n, ld, env_id_offset;
@@ -101,6 +101,11 @@ struct RolloutIO {
     uint8_t  *rec_flags;
     unsigned long long joint_actions;        // A^C (<= 2^32): an explored cellular action is floor(word * A^C / 2^32)
     uint32_t explore_thr_m1, explore_thr_nz; // the table policy explores iff thr_nz && word <= thr_m1 (P = eps)
+    // GC_POLICY_TABLE_STACK (appended like the record fields): env e acts by table row table_of_env[e], clamped to
+    // [0, n_tables), of policy [n_tables][table_stride]
+    const int32_t *table_of_env;             // [ld], 16-byte aligned
+    unsigned long long table_stride;         // nS: n_states^n_cells (grid world 400)
+    uint32_t n_tables;
 };
 
 // gc_collect_counts (the COUNT rollout kernels): int64 counters the kernels add to, NULL = not counted.  A kernel

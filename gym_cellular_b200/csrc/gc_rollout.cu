@@ -94,6 +94,21 @@ __device__ __forceinline__ uint32_t explore_words(const RolloutIO &io, uint32_t 
     return m;
 }
 
+// GC_POLICY_TABLE_STACK: the table ids of the 4 envs of a thread, re-read at every step (an L1 hit) rather than held in
+// registers across the step loop
+__device__ __forceinline__ int4 stack_map(const RolloutIO &io, int64_t e0)
+{
+    return __ldg(reinterpret_cast<const int4 *>(io.table_of_env + e0));
+}
+
+// first entry of table `id` of the stack; an id outside [0, n_tables) is clamped, so only the rows [0, n_tables) are read
+// whatever the map holds.  64-bit offset: a table has up to 2^32 entries (16 cells x 4 levels)
+__device__ __forceinline__ const int32_t *stack_row(const RolloutIO &io, int32_t id)
+{
+    const uint32_t j = min(static_cast<uint32_t>(id), io.n_tables - 1u);
+    return io.policy + j * io.table_stride;
+}
+
 // lanes of this warp inside the env loop at this iteration (a prefix: lane l owns env e0 + 4 (l - lane))
 __device__ __forceinline__ unsigned live_lanes(int64_t e0, int64_t n)
 {
@@ -194,11 +209,8 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
             const bool shared = !io.episodic || same4(t);
             // ---- actions ------------------------------------------------------------------------
             uint32_t aw[C];
-            if (io.policy_kind == GC_POLICY_TABLE) {
-                fold_index();
-                uint32_t p[kEPT];
-#pragma unroll
-                for (int e = 0; e < kEPT; ++e) p[e] = static_cast<uint32_t>(__ldg(io.policy + idx[e]));
+            // the table action p[e] of each env -> epsilon-greedy -> per-cell digits aw
+            auto table_actions = [&](uint32_t (&p)[kEPT]) {
                 if constexpr (EXPLORE) {
                     uint32_t xw[kEPT];
                     const uint32_t xm = explore_words(io, grp_lo, grp_hi, step0 + static_cast<uint32_t>(k), xw);
@@ -212,6 +224,21 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
 #pragma unroll
                     for (int e = 0; e < kEPT; ++e) { aw[c] |= (p[e] % A) << (8 * e); p[e] /= A; }
                 }
+            };
+            if (io.policy_kind == GC_POLICY_TABLE) {
+                fold_index();
+                uint32_t p[kEPT];
+#pragma unroll
+                for (int e = 0; e < kEPT; ++e) p[e] = static_cast<uint32_t>(__ldg(io.policy + idx[e]));
+                table_actions(p);
+            } else if (io.policy_kind == GC_POLICY_TABLE_STACK) {
+                fold_index();
+                const int4 m = stack_map(io, e0);
+                uint32_t p[kEPT] = {static_cast<uint32_t>(__ldg(stack_row(io, m.x) + idx[0])),
+                                    static_cast<uint32_t>(__ldg(stack_row(io, m.y) + idx[1])),
+                                    static_cast<uint32_t>(__ldg(stack_row(io, m.z) + idx[2])),
+                                    static_cast<uint32_t>(__ldg(stack_row(io, m.w) + idx[3]))};
+                table_actions(p);
             } else {
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
@@ -223,7 +250,7 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
             const int64_t kofs = static_cast<int64_t>(k) * ld;        // record row of this step (K * ld may pass 2^31)
             if constexpr (RECORD) {
                 if (io.rec_obs) {
-                    if (io.policy_kind != GC_POLICY_TABLE) fold_index();
+                    if (io.policy_kind == GC_POLICY_RANDOM) fold_index();
                     st_stream_v4(io.rec_obs + kofs + e0, make_int4(idx[0], idx[1], idx[2], idx[3]));
                 }
                 if (io.rec_action) {                                   // sum_c a_c A^c of the executed digits
@@ -356,7 +383,7 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                     }
                 }
                 if (cnt.visits || cnt.next || cnt.reward_q24 || cnt.unsafe) {
-                    if (io.policy_kind != GC_POLICY_TABLE) fold_index();
+                    if (io.policy_kind == GC_POLICY_RANDOM) fold_index();
                     // executed action sum_c a_c A^c, as recorded above (kept apart so that the RECORD kernels stay as
                     // they were compiled before the COUNT mode existed)
                     const uint32_t A2 = A * A, pl4[4] = {1u, A, A2, A2 * A};
@@ -449,12 +476,23 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
             for (int e = 0; e < kEPT; ++e) T[e] = io.episodic ? static_cast<uint32_t>(t[e]) : step0 + static_cast<uint32_t>(k);
             const bool shared = !io.episodic || same4(t);
             uint32_t act[kEPT];                                   // a_0 + 5 a_1
-            if (io.policy_kind == GC_POLICY_TABLE) {
+            if (io.policy_kind != GC_POLICY_RANDOM) {                  // GC_POLICY_TABLE or GC_POLICY_TABLE_STACK
+                if (io.policy_kind == GC_POLICY_TABLE) {
 #pragma unroll
-                for (int e = 0; e < kEPT; ++e) {
-                    const uint32_t tab = c0[e] + 20u * c1[e];
-                    act[e] = static_cast<uint32_t>(__ldg(io.policy + (tab < 400u ? tab : 0u)));
-                    if (act[e] > 24u) act[e] = 24u;
+                    for (int e = 0; e < kEPT; ++e) {
+                        const uint32_t tab = c0[e] + 20u * c1[e];
+                        act[e] = static_cast<uint32_t>(__ldg(io.policy + (tab < 400u ? tab : 0u)));
+                        if (act[e] > 24u) act[e] = 24u;
+                    }
+                } else {
+                    const int4 m = stack_map(io, e0);
+                    const int32_t *row[kEPT] = {stack_row(io, m.x), stack_row(io, m.y), stack_row(io, m.z), stack_row(io, m.w)};
+#pragma unroll
+                    for (int e = 0; e < kEPT; ++e) {
+                        const uint32_t tab = c0[e] + 20u * c1[e];
+                        act[e] = static_cast<uint32_t>(__ldg(row[e] + (tab < 400u ? tab : 0u)));
+                        if (act[e] > 24u) act[e] = 24u;
+                    }
                 }
                 if constexpr (EXPLORE) {
                     uint32_t xw[kEPT];

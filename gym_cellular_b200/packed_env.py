@@ -278,7 +278,7 @@ class PackedCellularVectorEnv(CellularVectorEnv):
         launch.slot = slot
         return launch
 
-    def rollout(self, n_steps, policy=None):
+    def rollout(self, n_steps, policy=None, policy_of_env=None):
         """Fused K-step rollout (see `CellularVectorEnv.rollout`).  The rollout kernel keeps the per-cell levels in
         registers, so the packed state is unpacked for it and packed again afterwards (two extra launches per
         call, amortised over `n_steps` steps)."""
@@ -287,12 +287,7 @@ class PackedCellularVectorEnv(CellularVectorEnv):
             self._ro_ret = torch.zeros(self.ld, dtype=torch.float32, device=self.device)
             self._ro_unsafe = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
             self._ro_index = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
-        kind, ptab = _lib.POLICY_RANDOM, None
-        if policy is not None:
-            ptab = torch.as_tensor(policy, device=self.device).to(torch.int32).contiguous()
-            if ptab.numel() != self.n_states ** self.n_cells:
-                raise ValueError("policy must have one entry per tabular state")
-            kind = _lib.POLICY_TABLE
+        kind, ptab = self._policy_table(policy, policy_of_env)
         cells = self.unpack(self._state).contiguous()            # int8 [n_cells, ld]
         _lib.check(self._lib.gc_rollout(self._h, int(n_steps), kind, _ptr(ptab), _ptr(cells), _ptr(self._t),
                                         _ptr(self._ro_index), _ptr(self._ro_ret), _ptr(self._ro_unsafe), _ptr(self._stats),
@@ -302,25 +297,25 @@ class PackedCellularVectorEnv(CellularVectorEnv):
             self._index.copy_(self._ro_index)
         return self._ro_ret[:n], self._ro_unsafe[:n]
 
-    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False):
+    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False, policy_of_env=None):
         """Experience collection (see `CellularVectorEnv.collect`): the recording kernel takes the int8 layout,
         so the packed state is unpacked for it and packed again afterwards, as in `rollout()`."""
         if getattr(self, "_ro_index", None) is None:
             self._ro_index = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
         cells = self.unpack(self._state).contiguous()            # int8 [n_cells, ld]
-        tr = self._collect(n_steps, policy, epsilon, next_obs, cells, self._ro_index)
+        tr = self._collect(n_steps, policy, epsilon, next_obs, cells, self._ro_index, policy_of_env)
         self._state.copy_(self.pack(cells))
         if self._index is not self._state:
             self._index.copy_(self._ro_index)
         return tr
 
-    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None):
+    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None, policy_of_env=None):
         """Experience counts (see `CellularVectorEnv.collect_counts`): the counting kernel takes the int8 layout, so the
         packed state is unpacked for it and packed again afterwards, as in `collect()`."""
         if getattr(self, "_ro_index", None) is None:
             self._ro_index = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
         cells = self.unpack(self._state).contiguous()            # int8 [n_cells, ld]
-        counts = self._collect_counts(n_steps, policy, epsilon, counts, cells, self._ro_index)
+        counts = self._collect_counts(n_steps, policy, epsilon, counts, cells, self._ro_index, policy_of_env)
         self._state.copy_(self.pack(cells))
         if self._index is not self._state:
             self._index.copy_(self._ro_index)

@@ -17,6 +17,7 @@ Two ways to drive it:
 There is no CPU implementation behind this class: without the CUDA library or a CUDA device it raises.
 """
 import ctypes as C
+import weakref
 from collections import namedtuple
 
 import numpy as np
@@ -76,6 +77,32 @@ def _round_up(n, m):
 
 def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def _check_policy_stack(policy, policy_of_env, n_states_joint, num_envs, device):
+    """Shapes, dtypes and device of a policy stack: `policy` [P, nS] of int tabular actions (P >= 1), `policy_of_env`
+    an integer tensor [num_envs] on `device`.  Returns policy as a contiguous int32 tensor on `device`.  (The range of
+    the map is checked on the device by the caller.)"""
+    if policy is None:
+        raise ValueError("policy_of_env needs a stack of policy tables: the random policy has no table to pick from")
+    ptab = torch.as_tensor(policy, device=device)
+    if ptab.dtype.is_floating_point or ptab.dtype.is_complex or ptab.dtype == torch.bool:
+        raise ValueError(f"policy must hold integer tabular actions, not {ptab.dtype}")
+    if ptab.dim() != 2 or ptab.shape[0] < 1 or ptab.shape[1] != n_states_joint:
+        raise ValueError(f"with policy_of_env, policy must have shape [n_tables, {n_states_joint}] (n_tables >= 1); "
+                         f"got {tuple(ptab.shape)}")
+    if ptab.shape[0] >= 2 ** 31:
+        raise ValueError("a policy stack holds fewer than 2**31 tables")
+    m = policy_of_env
+    if not isinstance(m, torch.Tensor):
+        raise ValueError("policy_of_env must be a torch tensor on the env's device")
+    if m.dtype not in (torch.int32, torch.int64, torch.int16, torch.int8, torch.uint8):
+        raise ValueError(f"policy_of_env must be an integer tensor, not {m.dtype}")
+    if m.device != torch.device(device):
+        raise ValueError(f"policy_of_env lives on {m.device}, the env on {device}")
+    if tuple(m.shape) != (num_envs,):
+        raise ValueError(f"policy_of_env must have shape ({num_envs},); got {tuple(m.shape)}")
+    return ptab.to(torch.int32).contiguous()
 
 
 _TYPESTR = {torch.int8: "|i1", torch.uint8: "|u1", torch.int32: "<i4", torch.float32: "<f4"}
@@ -626,28 +653,27 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         arr = self._slot_array(slots)
         _lib.check(self._lib.gc_prepare_step_many(self._h, arr, len(arr)))
 
-    def rollout(self, n_steps, policy=None):
+    def rollout(self, n_steps, policy=None, policy_of_env=None):
         """Fused K-step rollout: `n_steps` steps per env inside one kernel, actions generated on the
         device -- uniformly at random (policy=None) or from a tabular policy (int tensor
         [n_states ** n_cells] of tabular action indices).  Returns (returns float32 [num_envs],
         unsafe_steps int32 [num_envs]); state, time_step, tabular_state() and stats() advance exactly as
-        if step() had been called n_steps times with those actions."""
+        if step() had been called n_steps times with those actions.
+        policy_of_env: a stack of policies in one launch -- `policy` is then [P, n_states ** n_cells] and env e acts
+        by table policy_of_env[e] (an integer tensor [num_envs] on the env's device, values in [0, P)), exactly as it
+        would under that table alone.  The map is checked (one host synchronisation) and copied when a new tensor,
+        or a new version of it, arrives; a repeated call with the same map adds neither."""
         n = self.num_envs
         if getattr(self, "_ro_ret", None) is None:
             self._ro_ret = torch.zeros(self.ld, dtype=torch.float32, device=self.device)
             self._ro_unsafe = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
-        kind, ptab = _lib.POLICY_RANDOM, None
-        if policy is not None:
-            ptab = torch.as_tensor(policy, device=self.device).to(torch.int32).contiguous()
-            if ptab.numel() != self.n_states ** self.n_cells:
-                raise ValueError("policy must have one entry per tabular state")
-            kind = _lib.POLICY_TABLE
+        kind, ptab = self._policy_table(policy, policy_of_env)
         _lib.check(self._lib.gc_rollout(self._h, int(n_steps), kind, _ptr(ptab), _ptr(self._state), _ptr(self._t),
                                         _ptr(self._index), _ptr(self._ro_ret), _ptr(self._ro_unsafe), _ptr(self._stats),
                                         self._stream()))
         return self._ro_ret[:n], self._ro_unsafe[:n]
 
-    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False):
+    def collect(self, n_steps, policy=None, epsilon=0.0, next_obs=False, policy_of_env=None):
         """Experience collection: `n_steps` steps per env inside one kernel, as `rollout()`, recording every
         transition.  policy=None: uniformly random actions (epsilon must be 0); a table as for `rollout()`: the
         epsilon-greedy policy that takes policy[obs] and, with probability `epsilon`, a uniformly random joint
@@ -656,10 +682,15 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         Returns `Transitions(obs, action, reward, flags, next_obs)` of [n_steps, num_envs] views; state,
         time_step, tabular_state() and stats() advance exactly as `rollout()` advances them.  The views alias
         buffers cached per n_steps: the next `collect` with the same n_steps overwrites them, as a step
-        overwrites its outputs."""
-        return self._collect(n_steps, policy, epsilon, next_obs, self._state, self._index)
+        overwrites its outputs.  policy_of_env: a stack of table policies, one per env, as for `rollout()`; an
+        exploring env takes the uniformly random joint action whatever its table."""
+        return self._collect(n_steps, policy, epsilon, next_obs, self._state, self._index, policy_of_env)
 
-    def _policy_table(self, policy):
+    def _policy_table(self, policy, policy_of_env=None):
+        if policy_of_env is not None:
+            ptab = _check_policy_stack(policy, policy_of_env, self._joint_sizes()[0], self.num_envs, self.device)
+            self._set_policy_map(policy_of_env, ptab.shape[0])
+            return _lib.POLICY_TABLE_STACK, ptab
         if policy is None:
             return _lib.POLICY_RANDOM, None
         ptab = torch.as_tensor(policy, device=self.device).to(torch.int32).contiguous()
@@ -667,9 +698,26 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             raise ValueError("policy must have one entry per tabular state")
         return _lib.POLICY_TABLE, ptab
 
-    def _collect(self, n_steps, policy, epsilon, next_obs, state, index):
+    def _set_policy_map(self, policy_of_env, n_tables):
+        """Hands the table map of a policy stack to the handle (gc_set_policy_stack): an [ld] int32 copy owned by the
+        env, so that the kernels' 4-env reads of the padding stay inside it.  A map tensor seen before, unchanged
+        (same object, same `_version`) and for the same number of tables, is neither checked nor copied again, so build
+        the map once and pass the same tensor: a map rebuilt on every call is checked on every call (one host
+        synchronisation).  The env holds only a weak reference to it."""
+        key = getattr(self, "_map_key", None)
+        if key is not None and key[0]() is policy_of_env and key[1] == policy_of_env._version and key[2] == n_tables:
+            return
+        if bool(((policy_of_env < 0) | (policy_of_env >= n_tables)).any()):
+            raise ValueError(f"policy_of_env holds table ids outside [0, {n_tables})")
+        if getattr(self, "_map", None) is None:
+            self._map = torch.zeros(self.ld, dtype=torch.int32, device=self.device)
+        self._map[:self.num_envs].copy_(policy_of_env)
+        _lib.check(self._lib.gc_set_policy_stack(self._h, _ptr(self._map), int(n_tables)))
+        self._map_key = (weakref.ref(policy_of_env), policy_of_env._version, n_tables)
+
+    def _collect(self, n_steps, policy, epsilon, next_obs, state, index, policy_of_env=None):
         n_steps = int(n_steps)
-        kind, ptab = self._policy_table(policy)
+        kind, ptab = self._policy_table(policy, policy_of_env)
         bufs = self.__dict__.setdefault("_record_bufs", {})
         buf = bufs.get(n_steps)
         if buf is None:
@@ -707,16 +755,17 @@ class CellularVectorEnv(gym.vector.VectorEnv):
                       z(nS, nA) if joint else None, z(nS, nA) if joint else None,
                       z(Cn, S, A, S) if self.kind == "cellular" else None)
 
-    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None):
+    def collect_counts(self, n_steps, policy=None, epsilon=0.0, counts=None, policy_of_env=None):
         """Experience counts: `n_steps` steps per env inside one kernel, as `collect()` (same policies, same epsilon
         rule, same draws), adding every transition to `counts` instead of recording it.  counts=None allocates
         `zero_counts()`.  Returns `counts`; the counts equal the histogram of the record `collect()` would return, and
         state, time_step, tabular_state() and stats() advance exactly as `collect()` advances them.  The counts are
-        integers, so they are exact, independent of the order of the adds and of how the envs are sharded."""
-        return self._collect_counts(n_steps, policy, epsilon, counts, self._state, self._index)
+        integers, so they are exact, independent of the order of the adds and of how the envs are sharded.
+        policy_of_env: a stack of table policies, one per env, as for `rollout()`; all envs add to the one `counts`."""
+        return self._collect_counts(n_steps, policy, epsilon, counts, self._state, self._index, policy_of_env)
 
-    def _collect_counts(self, n_steps, policy, epsilon, counts, state, index):
-        kind, ptab = self._policy_table(policy)
+    def _collect_counts(self, n_steps, policy, epsilon, counts, state, index, policy_of_env=None):
+        kind, ptab = self._policy_table(policy, policy_of_env)
         if counts is None:
             counts = self.zero_counts()
         nS, nA = self._joint_sizes()

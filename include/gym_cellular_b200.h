@@ -290,11 +290,21 @@ int gc_unpack_cells(int device, int64_t n, int64_t ld, int32_t n_cells, const ui
  *                     position; grid_world.py:191-195).  Philox, keyed like the step's noise.
  *   GC_POLICY_TABLE   action = policy[tabular state] (device int32 [n_states^n_cells], tabular action
  *                     index): `initial_policy` as a table (cells3states3actions3.py:293-295)
+ *   GC_POLICY_TABLE_STACK  a stack of tables, one per env: policy is device int32 [n_tables][nS] (nS =
+ *                     n_states^n_cells, grid world 400) and env e of the shard acts by table table_of_env[e] of the
+ *                     map set with gc_set_policy_stack, exactly as it would under GC_POLICY_TABLE with that table alone.
+ *                     A map id outside [0, n_tables) is clamped into it: only the rows [0, n_tables) are read.
  * The result is bit-identical to n_steps calls of gc_step with the same actions.  Cellular family:
  * fast path only (n_states, n_actions <= 4).  ret [ld] float: sum of the n_steps rewards;
  * n_unsafe [ld] int32: steps that reported 'unsafe'; state / t / index as in gc_step. */
 #define GC_POLICY_RANDOM 0
 #define GC_POLICY_TABLE  1
+#define GC_POLICY_TABLE_STACK 2
+/* The table map of GC_POLICY_TABLE_STACK for gc_rollout, gc_collect and gc_collect_counts: table_of_env is device int32
+ * [ld] owned by the caller (16-byte aligned), read by every following call of kind GC_POLICY_TABLE_STACK; n_tables >= 1
+ * is the number of tables of the stacks those calls pass.  NULL switches the stack off (n_tables is then ignored), and
+ * kind GC_POLICY_TABLE_STACK is refused with GC_ERR_STATE until a map is set.  Host-only: stores the pointer. */
+int gc_set_policy_stack(gc_env *env, const int32_t *table_of_env, int32_t n_tables);
 int gc_rollout(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, int8_t *state,
                int32_t *t, uint32_t *index, float *ret, int32_t *n_unsafe, int64_t *stats, void *stream);
 
@@ -318,6 +328,8 @@ typedef struct {
  *                     floor(word * A^C / 2^32) (cellular) or by the random policy's rule (grid world); otherwise
  *                     action = policy[obs].  G is the global step even under GC_F_RNG_EPISODIC (exploration is the
  *                     agent's, not the environment's).  epsilon = 0 draws nothing: gc_rollout's actions exactly.
+ *   GC_POLICY_TABLE_STACK  the same epsilon-greedy rule, with the same draws; env e's greedy action is that of its own
+ *                     table (gc_set_policy_stack), an exploring env takes the uniform joint action whatever its table.
  * No per-env return / unsafe count: the record holds the per-step values.  One kernel launch. */
 int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
                int8_t *state, int32_t *t, uint32_t *index, const gc_record *record, int64_t *stats, void *stream);
