@@ -23,7 +23,7 @@ EXPORTS = ["gc_abi_version", "gc_last_error", "gc_create", "gc_destroy", "gc_set
            "gc_bind_step", "gc_step_bound", "gc_step_many", "gc_prepare_step_many", "gc_step_host", "gc_rollout", "gc_collect", "gc_collect_counts", "gc_poll_status", "gc_encode",
            "gc_decode", "gc_encode_mixed", "gc_decode_mixed", "gc_reset_packed", "gc_step_packed", "gc_bind_step_packed",
            "gc_step_host_packed", "gc_pack_cells", "gc_unpack_cells", "gc_compressible_supported", "gc_alloc_compressible",
-           "gc_free_compressible", "gc_is_compressible", "gc_set_policy_stack"]
+           "gc_free_compressible", "gc_is_compressible", "gc_set_policy_stack", "gc_collect_counts_grouped"]
 FLAG_UNSAFE, FLAG_TRUNCATED, FLAG_COUNT_SHIFT = 1, 2, 2
 
 
@@ -94,6 +94,7 @@ def load():
     L.gc_rollout.argtypes = [vp, C.c_int32, C.c_int32] + [vp] * 8
     L.gc_collect.argtypes = [vp, C.c_int32, C.c_int32, vp, C.c_double, vp, vp, vp, C.POINTER(GcRecord), vp, vp]
     L.gc_collect_counts.argtypes = [vp, C.c_int32, C.c_int32, vp, C.c_double, vp, vp, vp, C.POINTER(GcCounts), vp, vp]
+    L.gc_collect_counts_grouped.argtypes = [vp, C.c_int32, vp, C.c_double, vp, vp, vp, C.POINTER(GcCounts), vp, vp]
     L.gc_poll_status.argtypes = [vp, vp]
     L.gc_encode.argtypes = [C.c_int, i64, i64, C.c_int32, C.c_int32, vp, vp, vp]
     L.gc_decode.argtypes = [C.c_int, i64, i64, C.c_int32, C.c_int32, vp, vp, vp]

@@ -1018,10 +1018,12 @@ int gc_collect(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t 
     return GC_OK;
 }
 
-int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
-                      int8_t *state, int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream)
+namespace {
+
+// gc_collect_counts and gc_collect_counts_grouped: every check before any CUDA call, then one COUNT launch
+int collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon, int8_t *state,
+                   int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream, bool grouped)
 {
-    GC_NVTX("gc_collect_counts");
     if (int rc = check_collect_args(env, n_steps, policy_kind, policy, epsilon, state, t, index, counts)) return rc;
     if (counts->struct_size != sizeof(gc_counts))
         return fail(GC_ERR_INVALID, "counts->struct_size %u != sizeof(gc_counts) %zu", counts->struct_size, sizeof(gc_counts));
@@ -1052,6 +1054,19 @@ int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const i
         return fail(GC_ERR_INVALID, "the joint (state, action) tables would have more than 2^31 entries: count cell_next only");
     if (counts->next && n_sas > kJointLimit)
         return fail(GC_ERR_INVALID, "the joint 'next' table would have more than 2^31 entries");
+    const unsigned long long n_groups = grouped ? static_cast<unsigned long long>(env->n_policy_tables) : 0;
+    const unsigned long long n_cell = cellular ? static_cast<unsigned long long>(env->cfg.n_cells) * env->cfg.n_states *
+                                                 env->cfg.n_actions * env->cfg.n_states : 0;
+    if (grouped) {
+        if ((counts->visits || counts->reward_q24 || counts->unsafe) && sat_mul(n_groups, n_sa) > kJointLimit)
+            return fail(GC_ERR_INVALID, "the grouped (state, action) tables would have more than 2^31 entries (%llu groups)",
+                        n_groups);
+        if (counts->next && sat_mul(n_groups, n_sas) > kJointLimit)
+            return fail(GC_ERR_INVALID, "the grouped 'next' table would have more than 2^31 entries (%llu groups)", n_groups);
+        if (counts->cell_next && sat_mul(n_groups, n_cell) > kJointLimit)
+            return fail(GC_ERR_INVALID, "the grouped 'cell_next' table would have more than 2^31 entries (%llu groups)",
+                        n_groups);
+    }
     GC_ON_DEVICE(env->cfg.device);
     RolloutIO io = make_collect_io(env, n_steps, policy_kind, policy, epsilon, state, t, index, stats);
     CountIO cnt;
@@ -1062,6 +1077,12 @@ int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const i
     cnt.cell_next = reinterpret_cast<unsigned long long *>(counts->cell_next);
     cnt.n_states = static_cast<uint32_t>(nS);          // used only when a joint table fits, i.e. nS, nA <= 2^31
     cnt.n_actions = static_cast<uint32_t>(nA);
+    cnt.n_groups = static_cast<uint32_t>(n_groups);
+    cnt.sa_stride = cnt.cell_stride = 0;
+    if (grouped) {                                      // each product with n_groups is <= 2^31 where the table is counted
+        if (counts->visits || counts->next || counts->reward_q24 || counts->unsafe) cnt.sa_stride = static_cast<uint32_t>(n_sa);
+        if (counts->cell_next) cnt.cell_stride = static_cast<uint32_t>(n_cell);
+    }
     cudaError_t e;
     if (cellular)
         e = gc_launch_cell_count(env->tab, io, cnt, env->d_pair_lut, (env->cfg.flags & GC_F_NOISE) != 0, env->n_sm,
@@ -1072,6 +1093,23 @@ int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const i
     env->launches += 1;
     env->global_step += n_steps;
     return GC_OK;
+}
+
+}  // namespace
+
+int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
+                      int8_t *state, int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream)
+{
+    GC_NVTX("gc_collect_counts");
+    return collect_counts(env, n_steps, policy_kind, policy, epsilon, state, t, index, counts, stats, stream, false);
+}
+
+int gc_collect_counts_grouped(gc_env *env, int32_t n_steps, const int32_t *policy, double epsilon, int8_t *state,
+                              int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream)
+{
+    GC_NVTX("gc_collect_counts_grouped");
+    return collect_counts(env, n_steps, GC_POLICY_TABLE_STACK, policy, epsilon, state, t, index, counts, stats, stream,
+                          true);
 }
 
 int gc_poll_status(gc_env *env, void *stream)

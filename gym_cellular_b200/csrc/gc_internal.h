@@ -117,6 +117,11 @@ struct CountIO {
     unsigned long long *unsafe;        // [nS][nA]
     unsigned long long *cell_next;     // [C][S][A][S], cellular only
     uint32_t n_states, n_actions;      // nS, nA of the joint tables
+    // gc_collect_counts_grouped (appended): every table has a leading [n_groups] dimension and env e adds into group
+    // g = min(table_of_env[e], n_groups - 1) of the policy stack's map (RolloutIO), at g times the table's size.
+    // n_groups = 0: ungrouped.  n_groups times each counted table's size is at most 2^31, so the offsets are 32-bit.
+    uint32_t n_groups;
+    uint32_t sa_stride, cell_stride;   // nS nA (the 'next' table's group size is sa_stride * nS), C S A S
 };
 
 // Constant tables of the cellular family, passed by value as a __grid_constant__ parameter and

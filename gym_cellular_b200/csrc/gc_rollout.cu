@@ -35,6 +35,9 @@
 //     The add that takes a bin across 2^31 moves 2^31 to global memory, so no shared bin wraps as long as fewer than
 //     2^31 further adds land on it before that subtraction does (each add is at most 4, and the subtraction is the
 //     next instruction of the thread that crossed).
+// Grouped counts (gc_collect_counts_grouped, policy stacks only): a runtime branch of the same COUNT instantiations.
+// Every table has a leading group dimension and env e adds into group min(table_of_env[e], n_tables - 1); the joint
+// tables match lanes on the group-offset bin, the per-cell table uses warp-aggregated global atomics on (group, cell, bin).
 #include "gc_device.cuh"
 
 namespace {
@@ -109,6 +112,13 @@ __device__ __forceinline__ const int32_t *stack_row(const RolloutIO &io, int32_t
     return io.policy + j * io.table_stride;
 }
 
+// count group of env e0 + e (gc_collect_counts_grouped): its table id clamped as stack_row clamps it, read at each use
+// (an L1 hit) so that no group is held in registers across the count adds
+__device__ __forceinline__ uint32_t count_group(const RolloutIO &io, int64_t e0, int e)
+{
+    return min(static_cast<uint32_t>(__ldg(io.table_of_env + e0 + e)), io.n_tables - 1u);
+}
+
 // lanes of this warp inside the env loop at this iteration (a prefix: lane l owns env e0 + 4 (l - lane))
 __device__ __forceinline__ unsigned live_lanes(int64_t e0, int64_t n)
 {
@@ -117,7 +127,8 @@ __device__ __forceinline__ unsigned live_lanes(int64_t e0, int64_t n)
 }
 
 // one env per lane of the joint tables: bin sa = s * nA + a, successor nx, reward term q24 (round(r * 2^24)),
-// 'unsafe' uns.  Lanes on the same bin add as one group; valid = false lanes (past the batch) count nothing.
+// 'unsafe' uns.  Lanes on the same bin add as one group; valid = false lanes (past the batch) count nothing.  Grouped
+// counts pass sa + g * nS nA: the 'next' bin (g nS nA + sa) nS + nx is then g * nS nA nS + sa * nS + nx as well.
 __device__ __forceinline__ void count_joint(const CountIO &cnt, unsigned lanes, bool valid, uint32_t sa, uint32_t nx,
                                             int32_t q24, uint32_t uns)
 {
@@ -141,6 +152,16 @@ __device__ __forceinline__ void count_joint(const CountIO &cnt, unsigned lanes, 
         if (valid && static_cast<uint32_t>(__ffs(p2) - 1) == lane)
             atomicAdd(cnt.next + sas, static_cast<unsigned long long>(__popc(p2)));
     }
+}
+
+// grouped per-cell counts: one env per lane, flat index `at` of the grouped [G][C][S][A][S] table.  The per-block shared
+// histogram holds one group only, so lanes on the same (group, cell, bin) add as one 64-bit global atomic instead.  Out
+// of line: inlined into the 128-register count kernels of 11 to 16 cells, this path made them spill more.
+__device__ __noinline__ void count_cell_grouped(unsigned long long *cell_next, unsigned lanes, bool valid, uint32_t at)
+{
+    const unsigned peers = __match_any_sync(lanes, valid ? at : 0xFFFFFFFFu);
+    if (valid && static_cast<uint32_t>(__ffs(peers) - 1) == (threadIdx.x & 31))
+        atomicAdd(cell_next + at, static_cast<unsigned long long>(__popc(peers)));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -362,7 +383,21 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                 }
             }
             if constexpr (MODE == kCount) {
-                if (cnt.cell_next) {
+                if (cnt.cell_next && cnt.n_groups) {
+                    const unsigned lanes = live_lanes(e0, io.n);
+#pragma unroll 2
+                    for (int e = 0; e < kEPT; ++e) {
+                        const uint32_t S = static_cast<uint32_t>(tab.n_states), A = static_cast<uint32_t>(tab.n_actions);
+                        uint32_t at = count_group(io, e0, e) * cnt.cell_stride;       // (group, cell 0) of env e
+                        const uint32_t SAS = S * A * S;
+#pragma unroll
+                        for (int c = 0; c < C; ++c) {
+                            count_cell_grouped(cnt.cell_next, lanes, e < rem,
+                                               at + (((sw[c] >> (8 * e)) & 3u) * A + ((aw[c] >> (8 * e)) & 3u)) * S + ((rows[c] >> (8 * e)) & 3u));
+                            at += SAS;
+                        }
+                    }
+                } else if (cnt.cell_next) {
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
                         const uint32_t b = (sw[c] << 4) | (aw[c] << 2) | rows[c];     // bytes s * 16 + a * 4 + s'
@@ -402,8 +437,9 @@ cell_rollout_kernel(const __grid_constant__ CellTables tab, const __grid_constan
                     const unsigned lanes = live_lanes(e0, io.n);
 #pragma unroll
                     for (int e = 0; e < kEPT; ++e)
-                        count_joint(cnt, lanes, e < rem, idx[e] * cnt.n_actions + ai[e], nx[e],
-                                    __float2int_rn(rlog[e] * 16777216.0f), byte_of(unsafe_w, e));
+                        count_joint(cnt, lanes, e < rem,
+                                    (cnt.n_groups ? count_group(io, e0, e) * cnt.sa_stride : 0u) + idx[e] * cnt.n_actions + ai[e],
+                                    nx[e], __float2int_rn(rlog[e] * 16777216.0f), byte_of(unsafe_w, e));
                 }
             }
 #pragma unroll
@@ -571,7 +607,8 @@ grid_rollout_kernel(const __grid_constant__ GridParams gp, const __grid_constant
                 const unsigned lanes = live_lanes(e0, io.n);
 #pragma unroll
                 for (int e = 0; e < kEPT; ++e)
-                    count_joint(cnt, lanes, e < rem, ob[e] * 25u + act[e], nx[e], static_cast<int32_t>(byte_of(rew_w, e) << 24), 0u);
+                    count_joint(cnt, lanes, e < rem, (cnt.n_groups ? count_group(io, e0, e) * cnt.sa_stride : 0u) + ob[e] * 25u + act[e],
+                                nx[e], static_cast<int32_t>(byte_of(rew_w, e) << 24), 0u);
             }
         }
         st_stream_u32(io.state + e0, c0[0] | (c0[1] << 8) | (c0[2] << 16) | (c0[3] << 24));

@@ -64,8 +64,13 @@ class Counts(namedtuple("Counts", "visits next reward_q24 unsafe cell_next")):
       reward_q24  [nS, nA]        sum of round(reward * 2**24), the term stats()['reward_sum'] is kept in
       unsafe      [nS, nA]        steps that reported 'unsafe'
       cell_next   [C, S, A, S]    per cell c: N_c(s_c, a_c, s'_c) (cellular family only)
-    P_hat(s' | s, a) = next / visits and R_hat(s, a) = reward_q24 * 2**-24 / visits."""
+    P_hat(s' | s, a) = next / visits and R_hat(s, a) = reward_q24 * 2**-24 / visits.
+    Grouped counts (`zero_counts(groups=P)`) have a leading [P] on every table: `group(g)` is group g's Counts."""
     __slots__ = ()
+
+    def group(self, g):
+        """Counts of group g of grouped counts: views of row g of every table (None stays None)."""
+        return Counts(*(None if t is None else t[g] for t in self))
 
 
 _JOINT_LIMIT = 2 ** 31              # entries of one joint count table (32-bit indices in the kernels)
@@ -741,16 +746,28 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             return 400, 25
         return self.n_states ** self.n_cells, self.n_actions ** self.n_cells
 
-    def zero_counts(self, joint=True, transitions=True):
+    def zero_counts(self, joint=True, transitions=True, groups=None):
         """Zeroed `Counts` tables for `collect_counts`.  joint=False leaves the four joint tables None (for envs too
         large for them, such as 16 cells x 4 levels, only the per-cell `cell_next` is kept); transitions=False leaves
-        `next` None.  `cell_next` is None for grid world."""
+        `next` None.  `cell_next` is None for grid world.  groups=P: grouped counts, one set per table of a policy stack
+        of P tables, with a leading [P] on every table (`collect_counts(..., policy_of_env=)`); each table then holds at
+        most 2**31 entries in all."""
         nS, nA = self._joint_sizes()
-        if joint and (nS * nA > _JOINT_LIMIT or (transitions and nS * nA * nS > _JOINT_LIMIT)):
-            raise ValueError(f"the joint count tables of {nS} states x {nA} actions exceed 2**31 entries: use joint=False"
-                             + ("" if nS * nA > _JOINT_LIMIT else " or transitions=False"))
-        z = lambda *shape: torch.zeros(*shape, dtype=torch.int64, device=self.device)      # noqa: E731
         S, A, Cn = self.n_states, self.n_actions, self.n_cells
+        lead = ()
+        if groups is not None:
+            if isinstance(groups, bool) or not isinstance(groups, (int, np.integer)) or groups < 1:
+                raise ValueError(f"groups must be an int >= 1 (got {groups!r})")
+            lead = (int(groups),)
+        G = lead[0] if lead else 1
+        what = f"{G} groups x " if lead else ""
+        if joint and (G * nS * nA > _JOINT_LIMIT or (transitions and G * nS * nA * nS > _JOINT_LIMIT)):
+            raise ValueError(f"the joint count tables of {what}{nS} states x {nA} actions exceed 2**31 entries: use "
+                             "joint=False" + ("" if G * nS * nA > _JOINT_LIMIT else " or transitions=False")
+                             + (" or fewer groups" if lead else ""))
+        if self.kind == "cellular" and G * Cn * S * A * S > _JOINT_LIMIT:
+            raise ValueError(f"the per-cell count table of {what}{Cn} cells exceeds 2**31 entries: use fewer groups")
+        z = lambda *shape: torch.zeros(*lead, *shape, dtype=torch.int64, device=self.device)      # noqa: E731
         return Counts(z(nS, nA) if joint else None, z(nS, nA, nS) if joint and transitions else None,
                       z(nS, nA) if joint else None, z(nS, nA) if joint else None,
                       z(Cn, S, A, S) if self.kind == "cellular" else None)
@@ -761,11 +778,13 @@ class CellularVectorEnv(gym.vector.VectorEnv):
         `zero_counts()`.  Returns `counts`; the counts equal the histogram of the record `collect()` would return, and
         state, time_step, tabular_state() and stats() advance exactly as `collect()` advances them.  The counts are
         integers, so they are exact, independent of the order of the adds and of how the envs are sharded.
-        policy_of_env: a stack of table policies, one per env, as for `rollout()`; all envs add to the one `counts`."""
+        policy_of_env: a stack of table policies, one per env, as for `rollout()`.  All envs add to the one `counts`,
+        unless `counts` are grouped (`zero_counts(groups=P)`, P = policy.shape[0]): env e then adds into group
+        policy_of_env[e] only, so `counts.group(g)` is the histogram of the record over the envs of table g and the sum
+        over the groups is what ungrouped counts would hold.  Still one launch."""
         return self._collect_counts(n_steps, policy, epsilon, counts, self._state, self._index, policy_of_env)
 
     def _collect_counts(self, n_steps, policy, epsilon, counts, state, index, policy_of_env=None):
-        kind, ptab = self._policy_table(policy, policy_of_env)
         if counts is None:
             counts = self.zero_counts()
         nS, nA = self._joint_sizes()
@@ -773,6 +792,17 @@ class CellularVectorEnv(gym.vector.VectorEnv):
                         (self.n_cells, self.n_states, self.n_actions, self.n_states) if self.kind == "cellular" else None)
         if not isinstance(counts, Counts) or all(t is None for t in counts):
             raise ValueError("counts must be a Counts with at least one table (see zero_counts())")
+        # grouped counts: one more leading dimension on every table, of the size of the policy stack
+        given = [(t, shape) for t, shape in zip(counts, shapes) if isinstance(t, torch.Tensor) and shape is not None]
+        grouped = bool(given) and given[0][0].dim() == len(given[0][1]) + 1
+        if grouped and policy_of_env is None:
+            raise ValueError("grouped counts (a leading group dimension) need policy_of_env: one group per table")
+        kind, ptab = self._policy_table(policy, policy_of_env)
+        if grouped:
+            if given[0][0].shape[0] != ptab.shape[0]:
+                raise ValueError(f"grouped counts have {given[0][0].shape[0]} groups; the policy stack has "
+                                 f"{ptab.shape[0]} tables (one group per table)")
+            shapes = Counts(*(None if sh is None else (ptab.shape[0],) + sh for sh in shapes))
         for name, t, shape in zip(Counts._fields, counts, shapes):
             if t is None:
                 continue
@@ -784,8 +814,14 @@ class CellularVectorEnv(gym.vector.VectorEnv):
             if t.dtype != torch.int64 or t.device != self.device or not t.is_contiguous():
                 raise ValueError("count tables must be contiguous int64 tensors on the env's device")
         cs = _lib.GcCounts(C.sizeof(_lib.GcCounts), *(None if t is None else t.data_ptr() for t in counts))
-        _lib.check(self._lib.gc_collect_counts(self._h, int(n_steps), kind, _ptr(ptab), float(epsilon), _ptr(state),
-                                               _ptr(self._t), _ptr(index), C.byref(cs), _ptr(self._stats), self._stream()))
+        if grouped:
+            _lib.check(self._lib.gc_collect_counts_grouped(self._h, int(n_steps), _ptr(ptab), float(epsilon), _ptr(state),
+                                                           _ptr(self._t), _ptr(index), C.byref(cs), _ptr(self._stats),
+                                                           self._stream()))
+        else:
+            _lib.check(self._lib.gc_collect_counts(self._h, int(n_steps), kind, _ptr(ptab), float(epsilon), _ptr(state),
+                                                   _ptr(self._t), _ptr(index), C.byref(cs), _ptr(self._stats),
+                                                   self._stream()))
         return counts
 
     def capture_steps(self, action_ring):

@@ -355,6 +355,17 @@ typedef struct {
 int gc_collect_counts(gc_env *env, int32_t n_steps, int32_t policy_kind, const int32_t *policy, double epsilon,
                       int8_t *state, int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream);
 
+/* Grouped experience counts: gc_collect_counts with kind GC_POLICY_TABLE_STACK (same policies, epsilon rule, draws and
+ * advance of state, t, index, global step, statistics and launch count; one launch), adding each env's transitions
+ * into a count set of its own table.  Every table of `counts` has a leading dimension of P = the n_tables of
+ * gc_set_policy_stack: visits, reward_q24 and unsafe [P][nS][nA], next [P][nS][nA][nS], cell_next [P][C][S][A][S].
+ * Env e adds into group min(table_of_env[e], P - 1) (a map id read as unsigned), the id that selects its table, so
+ * group g is the histogram of gc_collect's record over the envs of table g, and the sum over the groups is what
+ * gc_collect_counts adds.  Refused: GC_ERR_STATE without a map; GC_ERR_INVALID for the checks of gc_collect_counts and
+ * for a counted table of more than 2^31 entries in all (P times its size).  A refused call changes nothing. */
+int gc_collect_counts_grouped(gc_env *env, int32_t n_steps, const int32_t *policy, double epsilon, int8_t *state,
+                              int32_t *t, uint32_t *index, const gc_counts *counts, int64_t *stats, void *stream);
+
 /* Reads and clears the handle's device status word (synchronises `stream`).  Returns GC_OK or
  * GC_ERR_ACTION if some env received a grid-world action without any go-to position since the
  * last poll (the reference raises KeyError('position'), grid_world.py:143). */
