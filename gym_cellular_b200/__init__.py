@@ -8,6 +8,7 @@ from . import tables
 from .tables import right_polarizing, multiple_optima, nonlinear, nonlinear_right_polarizing
 from .vector_env import CellularVectorEnv, Counts, Transitions, make_vector_env
 from .packed_env import PackedCellularVectorEnv
+from .plan import Plan, value_iteration
 from .device_codec import encode_mixed, decode_mixed
 from .codec import (generalized_cellular2tabular, generalized_tabular2cellular, cellular2tabular,
                     tabular2cellular)
@@ -21,5 +22,6 @@ __all__ = ["CellularVectorEnv", "PackedCellularVectorEnv", "Transitions", "Count
            "nonlinear", "nonlinear_right_polarizing", "Cells3States3Actions3Env", "Cells2Rest3Env",
            "Cells3ResetVDeadlockEnv", "GridWorldEnv", "PriorKnowledge", "GridWorldPriorKnowledge",
            "generalized_cellular2tabular", "generalized_tabular2cellular", "cellular2tabular", "tabular2cellular",
-           "DebugEnv", "DeepPlanningDebugEnv", "DeepExplorationDebugEnv", "install_alias", "encode_mixed", "decode_mixed"]
+           "DebugEnv", "DeepPlanningDebugEnv", "DeepExplorationDebugEnv", "install_alias", "encode_mixed", "decode_mixed",
+           "Plan", "value_iteration"]
 __version__ = "0.1.0"
